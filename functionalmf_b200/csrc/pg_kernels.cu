@@ -52,6 +52,13 @@ __device__ __forceinline__ PgTilt pg_setup(double z) {
         const double x0 = log(fz) + fz * PG_TRUNC;
         qdivp = 4.0 / PG_PI * (exp(x0 - c.Z + log_phi(b)) + exp(x0 + c.Z + log_phi(a)));
     }
+    // q / p grows like exp(0.32 Z^2): it overflows to inf for |z| > ~97, and past 2^1022 its hardware reciprocal
+    // flushes to zero; (up - 1) * inv_qp would then be NaN (inf * 0) or 0 instead of a uniform, and the
+    // inverse-Gaussian proposal would never take its mu^2 / X root.  From 2^900 on the exponential tail's probability
+    // 1 / (1 + q/p) is below 2^-900, far under the 2^-53 resolution of u1, so every draw takes the inverse-Gaussian
+    // branch; with q/p capped at that power of two, up = u1 2^900 and (up - 1) 2^-900 round to exactly u1, the
+    // proper U(0,1) of the branch.
+    if (!(qdivp < 0x1p900)) qdivp = 0x1p900;
     c.inv_fz = pg_rcp_pos(fz);
     c.inv_p = 1.0 + qdivp;                               // 1 / P(exponential tail)
     c.inv_qp = qdivp > 1e-300 ? pg_rcp_pos(qdivp) : 0.0;  // (u1 / p - 1) / (q / p) is U(0,1) given the inverse-Gaussian branch
@@ -175,8 +182,10 @@ __device__ __forceinline__ double pg_mean(double b, double z) {
 __device__ __forceinline__ double pg_var(double b, double z) {
     z = fabs(z);
     if (z < 1e-3) return b * (1.0 / 24.0) * (1.0 - z * z * 0.2);
-    double ch = cosh(0.5 * z);
-    return b * (sinh(z) - z) / (4.0 * z * z * z * ch * ch);
+    // (sinh z - z) / cosh^2(z/2) = 2 tanh(z/2) - z sech^2(z/2): finite for every z, where the quotient is
+    // inf / inf = NaN past z = 710
+    const double sech = 1.0 / cosh(0.5 * z);
+    return b * (2.0 * tanh(0.5 * z) - z * sech * sech) / (4.0 * z * z * z);
 }
 
 __device__ double pg_draw(Rng& rng, double b, double z) {

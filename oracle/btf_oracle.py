@@ -309,9 +309,11 @@ def binomial_weights(Ysucc, Ntrials, omega):
 # ----------------------------------------------------------------------------
 # negative-binomial dispersion   (factor.py:513-554)
 # ----------------------------------------------------------------------------
-def step_R(R, W, V, data, rdims, zs, us, rpropstdev=0.1, rstdev=1.0):
+def step_R(R, W, V, data, rdims, zs, us, rpropstdev=0.1, rstdev=1.0, want_margin=False):
     """NegativeBinomialBTF._resample_R with explicit noise: ``zs`` [nmh, *R.shape]
-    standard normals, ``us`` [nmh, *R.shape] uniforms.  Returns (R, N)."""
+    standard normals, ``us`` [nmh, *R.shape] uniforms.  Returns (R, N), and with
+    ``want_margin`` also min |u - prob| / prob over the chain's decisions (inf for none):
+    how far the closest accept/reject decision was from a tie."""
     from scipy.special import gammaln
     data = np.asarray(data, dtype=float)
     if data.ndim == 3:
@@ -321,6 +323,7 @@ def step_R(R, W, V, data, rdims, zs, us, rpropstdev=0.1, rstdev=1.0):
     psi = np.einsum('nk,mtk->nmt', W, V).clip(-10, 10)
     P = (1.0 / (1.0 + np.exp(-psi)))[..., None]
     agg = [3] + sorted(rdims)[::-1]
+    margin = np.inf
     for s in range(zs.shape[0]):
         cand_log = logR + rpropstdev * zs[s][..., None]
         cand = np.exp(cand_log)
@@ -331,10 +334,14 @@ def step_R(R, W, V, data, rdims, zs, us, rpropstdev=0.1, rstdev=1.0):
             ll = np.nansum(ll, axis=dim)
         dprior = np.squeeze(dprior).reshape(ll.shape)
         prob = np.exp(np.clip(dprior + ll, -10, 1)).reshape(R.shape)
-        acc = (us[s][..., None] <= prob) & (cand > 1)
+        u = us[s][..., None]
+        acc = (u <= prob) & (cand > 1)
+        margin = min(margin, float(np.min(np.abs(u - prob) / prob)))
         logR[acc] = cand_log[acc]
         R[acc] = np.exp(cand_log[acc])
     Ncount = np.nansum(data + R, axis=-1)
+    if want_margin:
+        return R[..., 0], Ncount, margin
     return R[..., 0], Ncount
 
 

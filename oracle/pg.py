@@ -16,10 +16,11 @@ the published algorithms it is built from:
   b > 170: moment-matched normal approximation (the hybrid sampler's rule).
 
 Validated by moments (tests/test_pg_oracle.py):
-  E  = b/(2z) tanh(z/2),   Var = b/(4 z^3) (sinh z - z) sech^2(z/2).
+  E  = b/(2z) tanh(z/2),   Var = b/(4 z^3) (sinh z - z) sech^2(z/2)
+                                = b/(4 z^3) (2 tanh(z/2) - z sech^2(z/2)).
 """
 import numpy as np
-from scipy.special import ndtr, log_ndtr
+from scipy.special import expit, log_ndtr
 
 TRUNC = 0.64
 PI = np.pi
@@ -39,7 +40,10 @@ def pg_var(b, z):
     z = np.abs(np.asarray(z, dtype=float))
     small = z < 1e-3
     zs = np.where(small, 1.0, z)
-    v = (np.sinh(zs) - zs) / (4 * zs ** 3 * np.cosh(zs / 2) ** 2)
+    # (sinh z - z) sech^2(z/2) = 2 tanh(z/2) - z sech^2(z/2): no inf / inf past z = 710
+    with np.errstate(over='ignore'):
+        sech = 1.0 / np.cosh(zs / 2)
+    v = (2 * np.tanh(zs / 2) - zs * sech * sech) / (4 * zs ** 3)
     v0 = (1.0 / 24.0) * (1 - z * z * (1.0 / 4.0 - 1.0 / 20.0))   # series around 0
     return b * np.where(small, v0, v)
 
@@ -60,8 +64,9 @@ def _mass_texpon(Z):
     x0 = np.log(fz) + fz * TRUNC
     xb = x0 - Z + log_ndtr(b)
     xa = x0 + Z + log_ndtr(a)
-    qdivp = 4 / PI * (np.exp(xb) + np.exp(xa))
-    return 1.0 / (1.0 + qdivp)
+    # log(q/p) and p = 1 / (1 + q/p) = expit(-log(q/p)): q/p itself overflows for |z| > ~97, where p is 0
+    log_qdivp = np.log(4 / PI) + np.logaddexp(xb, xa)
+    return expit(-log_qdivp)
 
 
 def _rtigauss(Z, rng):

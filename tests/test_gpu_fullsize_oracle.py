@@ -136,3 +136,101 @@ def test_c5_slice_k32_sampled_rows_and_columns_vs_oracle():
     rs = np.random.RandomState(2)
     rows = [0, 31, 32] + sorted(rs.choice(np.arange(33, 2048), 5, replace=False).tolist())
     _run_case(2048, 1024, 128, 2, 32, 2, rows, [5, 1023], piece=128)
+
+
+def test_c3_shape_binomial_sampled_rows_and_columns_vs_oracle():
+    """BASELINE.json C3 (Binomial, 4096 x 1024 x 32, 4 trials, 1 % NaN, nembeds=8, tf_order=1): one W, V sweep with
+    injected Polya-Gamma weights through the f64-weight statistics kernels at full size; 16 rows, 2 columns.  The
+    weights are real, so the integer-tensor-core path must stay off."""
+    from oracle import btf_oracle as O
+    from functionalmf_b200.engine import Engine
+    N, M, T, K, order, trials = 4096, 1024, 32, 8, 1, 4
+    rs = np.random.RandomState(3)
+    rows_s = np.asarray([0, 7, 31, 32] + sorted(rs.choice(np.arange(33, N), 12, replace=False).tolist()))
+    cols_s = np.asarray([1, 1023])
+    W0 = rs.normal(size=(N, K))
+    W0[np.triu_indices(K, k=1)] = 0
+    V0 = rs.normal(size=(M, T, K)).cumsum(axis=1) * 0.2
+    # data, trials and weights in 256-row pieces (three 1 GB host arrays, no full-size temporaries)
+    Ys = np.empty((N, M, T))
+    Nt = np.empty((N, M, T))
+    omega = np.empty((N, M, T))
+    Vf = V0.reshape(M * T, K)
+    for a in range(0, N, 256):
+        b = min(N, a + 256)
+        mu = (W0[a:b] @ Vf.T).reshape(b - a, M, T) * 0.5
+        y = rs.binomial(trials, 1 / (1 + np.exp(-mu))).astype(float)
+        miss = rs.random_sample(y.shape) < 0.01
+        y[miss] = np.nan
+        Ys[a:b] = y
+        Nt[a:b] = np.where(miss, np.nan, float(trials))
+        omega[a:b] = np.where(miss, 0.0, rs.gamma(2.0, 0.2, size=y.shape) + 0.02)
+    eng = Engine(N, M, T, nembeds=K, tf_order=order, likelihood=1, seed=11)
+    Delta = eng.get('Delta')
+    RD = Delta.shape[0]
+    eng.set_data_binomial(Ys, Nt)
+    Wst = W0 + 0.05 * rs.normal(size=(N, K)) * (W0 != 0)
+    Vst = V0 + 0.05 * rs.normal(size=(M, T, K))
+    Tau2 = rs.gamma(2.0, 1.0, size=(M, RD)) + 0.05
+    sc = dict(lam2=0.7, lam2_a=1.3, sigma2=0.9)
+    zW, zV = rs.normal(size=(N, K)), rs.normal(size=(M, T, K))
+    eng.set('W', Wst); eng.set('V', Vst)
+    for nm in ('Tau2', 'Tau2_a', 'Tau2_b', 'Tau2_c'):
+        eng.set(nm, Tau2)
+    for k, v in sc.items():
+        eng.set(k, [v])
+    eng.set_sample_mask(16 | 32)
+    eng.enable_diag(True)
+    eng.inject('omega', omega)
+    eng.inject('z_W', zW); eng.inject('z_V', zV)
+    eng.sweep(1)
+    Lp = K * (K + 1) // 2
+    il = np.tril_indices(K)
+    dg = [k * (k + 1) // 2 + k for k in range(K)]
+
+    # ---- W step on the sampled rows
+    cw, sw = O.binomial_weights(Ys[rows_s], Nt[rows_s], omega[rows_s])
+    A, b_ = O.row_stats(Vst, cw, sw)
+    rstat = eng.diag('row_stats')[rows_s]
+    assert normerr(rstat[:, :Lp], A[:, il[0], il[1]]) < TOL
+    assert normerr(rstat[:, Lp:], b_) < TOL
+    assert np.max(np.abs(rstat[:, dg] / A[:, range(K), range(K)] - 1.0)) < TOL
+    Wn_s, dW = O.step_W(Wst[rows_s], Vst, cw, sw, sc['sigma2'], zW[rows_s], row_index=rows_s)
+    Wq = eng.diag('W_Q')[rows_s]
+    Wl = eng.diag('W_L')[rows_s]
+    Wg_all = eng.get('W')
+    for q, i in enumerate(rows_s):
+        d = min(i + 1, K)
+        assert normerr(Wq[q][:d, :d], dW['Q'][q][:d, :d]) < TOL, ('W_Q', i)
+        assert normerr(np.tril(Wl[q][:d, :d]), dW['L'][q][:d, :d]) < 1e-9, ('W_L', i)
+    assert normerr(Wg_all[rows_s], Wn_s) < 1e-9
+    assert np.all(Wg_all[np.triu_indices(K, k=1)] == 0)
+
+    # ---- V step on the sampled columns, given the engine's new W
+    cwc, swc = O.binomial_weights(Ys[:, cols_s], Nt[:, cols_s], omega[:, cols_s])
+    del Ys, Nt, omega
+    Ac, bc = O.col_stats(Wg_all, cwc, swc)
+    cstat = eng.diag('col_stats').reshape(M, T, Lp + K)[cols_s]
+    assert normerr(cstat[..., :Lp], Ac[..., il[0], il[1]]) < TOL
+    assert normerr(cstat[..., Lp:], bc) < TOL
+    assert np.max(np.abs(cstat[..., dg] / Ac[..., range(K), range(K)] - 1.0)) < TOL
+    Vn, dV = O.step_V(Wg_all, Vst[cols_s], cwc, swc, Delta, sc['lam2'], Tau2[cols_s], zV[cols_s], order, want_diag=True)
+    band = eng.diag('V_band')[cols_s]
+    mean = eng.diag('V_mean')[cols_s]
+    Vg = eng.get('V')
+    assert int(eng.diag('V_retries').sum()) == 0 and int(dV['retries'].sum()) == 0
+    for q, j in enumerate(cols_s):
+        assert normerr(band[q], band_rows_from_lower(dV['band'][q])) < TOL, ('band', j)
+        Qd = O.band_to_dense_lower(dV['band'][q])
+        Qd = Qd + np.tril(Qd, -1).T
+        kappa = np.linalg.cond(Qd)
+        tol = max(TOL, 50 * kappa * EPS)
+        assert normerr(mean[q], dV['mean'][q]) < tol, ('mean', j, kappa)
+        assert normerr(Vg[j], Vn[q]) < tol, ('draw', j, kappa)
+        rhs = dV['b'][q].ravel()
+        m = mean[q].ravel()
+        bwd = np.linalg.norm(Qd @ m - rhs) / (np.linalg.norm(Qd, 2) * np.linalg.norm(m) + np.linalg.norm(rhs))
+        assert bwd < 1e-13, (j, bwd)
+    ph = eng.time_phases(1)
+    assert ph.get('row_i8gemm', 0.0) == 0.0
+    eng.close()

@@ -37,8 +37,10 @@ def test_gamma_moments(shape):
 
 
 @pytest.mark.parametrize('b', [1.0, 2.0, 4.0, 2.5, 0.3, 30.0, 200.0])
-@pytest.mark.parametrize('z', [0.0, 0.5, 2.0, 5.0, -12.0])
+@pytest.mark.parametrize('z', [0.0, 0.5, 2.0, 5.0, -12.0, 30.0, -100.0, 300.0, 1000.0])
 def test_polya_gamma_moments(b, z):
+    # |z| >= 100: past the overflow of q/p in the Devroye set-up (exact sampler) and, with b = 200, past z = 710
+    # where the closed-form variance of the normal route is inf / inf
     from functionalmf_b200.engine import pg_sample
     from oracle import pg as OPG
     n = 60000 if b <= 4 else 20000
@@ -55,7 +57,7 @@ def test_polya_gamma_matches_cpu_oracle_distribution():
     from oracle import pg as OPG
     from scipy import stats
     rng = np.random.default_rng(3)
-    for b, z in [(1.0, 0.0), (1.0, 3.0), (4.0, 1.0), (2.5, 1.0)]:
+    for b, z in [(1.0, 0.0), (1.0, 3.0), (4.0, 1.0), (2.5, 1.0), (1.0, 100.0), (2.5, -150.0)]:
         n = 40000
         gpu = pg_sample(np.full(n, b), np.full(n, z), seed=77)
         cpu = OPG.pgdraw(np.full(n, b), np.full(n, z), rng)
