@@ -86,12 +86,8 @@ __global__ void __launch_bounds__(LaGeom<KB, Q>::NT, LaGeom<KB, Q>::MINB) band_l
     const int Kr = a.K;                                  // true embedding size (<= KB)
     const int L = Kr * (Kr + 1) / 2, nco = L + Kr, kd = Q * Kr, LS = kd + 1;
     const int T = a.T, n = T * Kr;
-    // Role rotation: warp 0 of the role map runs the serial pivot chain of every step.  The hardware puts warp w of a
-    // CTA on scheduler w mod 4, so without rotation the pivot warps of ALL co-resident CTAs share one scheduler (and its
-    // FP64 lanes) while the other three idle between tensor-pipe jobs.  CTAs that share an SM differ in blockIdx / #SMs
-    // (first wave), so rotating the role map by that quotient spreads the pivot chains over the four schedulers.
     const int lane = threadIdx.x & 31;
-    const int warp = ((int)(threadIdx.x >> 5) + (a.rotate_roles ? (int)(blockIdx.x / a.rotate_roles) : 0)) % NW;
+    const int warp = (int)(threadIdx.x >> 5);
     const int tid = warp * 32 + lane;
     const int jl = blockIdx.x, jg = a.col_begin + jl;
     const unsigned full = 0xffffffffu;
@@ -689,7 +685,7 @@ __global__ void __launch_bounds__(LaGeom<KB, Q>::NT, LaGeom<KB, Q>::MINB) band_l
             accum += wgt * (((p[0] + p[1]) + (p[2] + p[3])) + ((p[4] + p[5]) + (p[6] + p[7])));
         }
         double tot = block_sum(accum, red);
-        if (threadIdx.x == 0) a.resid_partials[jl] = tot;     // block_sum leaves the total in PHYSICAL thread 0 (roles are rotated)
+        if (threadIdx.x == 0) a.resid_partials[jl] = tot;
     }
     LAPROF(5);
 #ifdef BTF_BAND_PROFILE

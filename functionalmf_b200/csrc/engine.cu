@@ -39,6 +39,20 @@ struct DevBuf {
     size_t n = 0;
 };
 
+// Environment switches (INTEGRATION.md §1), read once per engine by read_env(); the kernel files get the values as arguments.
+struct EnvSwitches {
+    bool no_i8 = false, force_i8 = false;   // BTF_STATS_NO_I8, BTF_STATS_FORCE_I8
+    int i8_gemm2 = -1;                      // BTF_I8_GEMM2: 0 never / 1 always the 2-CTA product-block kernel, -1 by tile count
+    bool i8_guard = true;                   // BTF_I8_NO_GUARD
+    double i8_guard_tol = 1e-12;            // BTF_I8_GUARD_TOL
+    bool scol = true;                       // BTF_NO_SCOL
+    bool upload_bounce = true;              // BTF_UPLOAD_BOUNCE
+    int upload_threads = 0;                 // BTF_UPLOAD_THREADS (0: the cores this process may use, at most 16)
+    bool nvtx = false;                      // BTF_NVTX
+    bool band_scalar = false;               // BTF_BAND_SCALAR
+    bool nb_hist = true;                    // BTF_NB_NO_HIST
+};
+
 enum Phase { PH_NU2 = 0, PH_SIGMA2, PH_TAU2, PH_LAM2, PH_ROW_STATS, PH_ROW_SOLVE, PH_COL_STATS, PH_BAND_SOLVE, PH_COMM, PH_COUNT };
 
 // one held-out evaluator (eval_kernels.cu)
@@ -64,11 +78,8 @@ struct btf_engine {
     int sm_count;
     cudaStream_t stream = nullptr, copy_stream = nullptr;
     cudaStream_t side[2] = {nullptr, nullptr};   // forked inside a sweep: tensor-core product block | HBM-bound linear block
-    cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr}, ev_digits = nullptr;
-    bool sf_after_digits = false;   // BTF_SF_AFTER_DIGITS=1: the linear block starts with the GEMM (after the digit kernels), co-residency experiment
-    cudaEvent_t ev_chunk[2][16] = {{nullptr}};   // per column chunk of the V step: product block done | linear block done
-    int col_chunks = 1;          // BTF_COL_CHUNKS: the V step can run as a pipeline over column chunks (off by default: see DESIGN.md)
-    bool overlap = true;         // BTF_NO_OVERLAP=1: everything on one stream (A/B runs)
+    cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
+    EnvSwitches env;
     // state
     double *W = nullptr, *V = nullptr, *Tau2 = nullptr, *Tau2_a = nullptr, *Tau2_b = nullptr, *Tau2_c = nullptr;
     Scalars* scal = nullptr;
@@ -99,12 +110,12 @@ struct btf_engine {
     // K1 on the integer tensor cores (stats_i8.cu): decided per data set, buffers allocated on first use
     bool i8_on = false, i8_decided = false;
     StatsI8Buffers i8{};
+    int i8_route[2] = {0, 0};    // I8Route of the last row / column product block (0: none yet)
     unsigned *cnt_rowsum = nullptr, *cnt_colsum = nullptr;   // sum of the counts of every local row / owned (j,t): guard of the fixed-point block
     int* guard_n = nullptr;                                  // [2] rows / (j,t) recomputed in FP64 by the last W / V step
     unsigned char* guard_flags = nullptr;                    // [nloc + Ploc] flags set by the kernels that produce the block
-    bool guard_on = true;        // BTF_I8_NO_GUARD=1 switches the element-wise guard off
     double* Scol = nullptr;      // sharded engines, when it fits: S of this rank's (j,t) over ALL rows, [Nall_pad][Ploc_pad] -> the
-                                 // linear block of the V step needs no reduce-scatter (BTF_NO_SCOL=1 keeps the partial-sum route)
+                                 // linear block of the V step needs no reduce-scatter
     int Ploc_pad = 0;
     uint8_t* cntT = nullptr;     // [Ploc][Nall_pad] counts of this rank's columns over ALL rows (right operand of the column contraction)
     double *mu_mean = nullptr, *mu_m2 = nullptr; long long mu_count = 0; bool mu_track = false;   // posterior moments of Mu
@@ -219,6 +230,24 @@ static bool is_device_ptr(const void* p) {
     return at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
 }
 
+// The environment switches of INTEGRATION.md §1, read when an engine is created.
+static EnvSwitches read_env() {
+    auto on = [](const char* nm) { return getenv(nm) != nullptr; };
+    EnvSwitches s;
+    s.no_i8 = on("BTF_STATS_NO_I8");
+    s.force_i8 = on("BTF_STATS_FORCE_I8");
+    if (const char* g = getenv("BTF_I8_GEMM2")) s.i8_gemm2 = g[0] == '0' ? 0 : 1;
+    s.i8_guard = !on("BTF_I8_NO_GUARD");
+    if (const char* t = getenv("BTF_I8_GUARD_TOL")) s.i8_guard_tol = atof(t);
+    s.scol = !on("BTF_NO_SCOL");
+    if (const char* b = getenv("BTF_UPLOAD_BOUNCE")) s.upload_bounce = b[0] != '0';
+    if (const char* n = getenv("BTF_UPLOAD_THREADS")) s.upload_threads = std::max(1, atoi(n));
+    s.nvtx = on("BTF_NVTX");
+    s.band_scalar = on("BTF_BAND_SCALAR");
+    s.nb_hist = !on("BTF_NB_NO_HIST");
+    return s;
+}
+
 void btf_destroy(btf_engine* e);
 
 int btf_create(const btf_config* c, btf_engine** out) {
@@ -245,7 +274,7 @@ int btf_create(const btf_config* c, btf_engine** out) {
     if (e->nloc < 0 || e->Mloc < 0) { return set_err(BTF_EINVAL, "bad shard"); }
     e->Nall_pad = e->cfg.world_size > 1 ? round_up(e->N, 128) : e->nloc_pad;
     e->p0 = e->cfg.col_begin * e->T; e->Ploc = e->Mloc * e->T;
-    e->overlap = getenv("BTF_NO_OVERLAP") == nullptr;
+    e->env = read_env();
     CK(cudaSetDevice(c->device));
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, c->device));
@@ -255,7 +284,6 @@ int btf_create(const btf_config* c, btf_engine** out) {
         // are placed ahead of the queued tiles of the throughput kernels on the side streams
         int lo = 0, hi = 0;
         CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        if (getenv("BTF_NO_PRIO")) hi = lo;
         CK(cudaStreamCreateWithPriority(&e->stream, cudaStreamNonBlocking, hi));
     }
     CK(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
@@ -267,10 +295,6 @@ int btf_create(const btf_config* c, btf_engine** out) {
         CK(cudaEventCreateWithFlags(&e->ev_join[i], cudaEventDisableTiming));
     }
     CK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&e->ev_digits, cudaEventDisableTiming));
-    e->sf_after_digits = getenv("BTF_SF_AFTER_DIGITS") != nullptr;
-    for (int i = 0; i < 32; ++i) CK(cudaEventCreateWithFlags(&e->ev_chunk[i / 16][i % 16], cudaEventDisableTiming));
-    if (const char* cc = getenv("BTF_COL_CHUNKS")) e->col_chunks = std::min(16, std::max(1, atoi(cc)));
     CK(cudaEventCreateWithFlags(&e->ev_snap, cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&e->ev_copied, cudaEventDisableTiming));
     for (int i = 0; i <= PH_COUNT; ++i) CK(cudaEventCreate(&e->ph_ev[i]));
@@ -432,8 +456,6 @@ void btf_destroy(btf_engine* e) {
         if (e->ev_join[i]) cudaEventDestroy(e->ev_join[i]);
     }
     if (e->ev_fork) cudaEventDestroy(e->ev_fork);
-    if (e->ev_digits) cudaEventDestroy(e->ev_digits);
-    for (int i = 0; i < 32; ++i) if (e->ev_chunk[i / 16][i % 16]) cudaEventDestroy(e->ev_chunk[i / 16][i % 16]);
     if (e->stream) cudaStreamDestroy(e->stream);
     if (e->copy_stream) cudaStreamDestroy(e->copy_stream);
     delete e;
@@ -469,14 +491,14 @@ static bool is_pageable_host_ptr(const void* p) {
 
 // memcpy with several host threads: one thread copies ~10 GB/s, which is also all a cudaMemcpy from pageable memory
 // reaches (it goes through the driver's own single-threaded bounce buffer)
-static void parallel_memcpy(void* dst, const void* src, size_t bytes) {
+static void parallel_memcpy(void* dst, const void* src, size_t bytes, int threads) {
     // threads: the cores this process may run on, at most 16 (C2 on the bench box: 8 threads 36.6 GB/s, 16 threads 40.6 GB/s,
     // pinned source 55 GB/s), and at least 4 MB each
     unsigned hw = std::thread::hardware_concurrency();
     cpu_set_t cs;
     if (sched_getaffinity(0, sizeof(cs), &cs) == 0 && CPU_COUNT(&cs) > 0) hw = (unsigned)CPU_COUNT(&cs);
     int nt = (int)std::min<size_t>(std::min<unsigned>(hw ? hw : 4, 16), std::max<size_t>(1, bytes >> 22));
-    if (const char* s = getenv("BTF_UPLOAD_THREADS")) nt = std::max(1, atoi(s));
+    if (threads > 0) nt = threads;
     if (nt <= 1) { memcpy(dst, src, bytes); return; }
     std::vector<std::thread> th;
     const size_t per = ((bytes + nt - 1) / nt + 4095) & ~(size_t)4095;
@@ -507,7 +529,7 @@ int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int
     // Ordinary numpy memory: a cudaMemcpy from it runs at ~10 GB/s, and page-locking it in place for one upload costs
     // more than that copy (cudaHostRegister ~5-8 GB/s; tools/upload_timing.py) - so it is copied by several host threads
     // into two pinned bounce buffers, from which the asynchronous copies run at link speed.  BTF_UPLOAD_BOUNCE=0: plain copy.
-    const bool bounce = !on_dev && is_pageable_host_ptr(Y) && !(getenv("BTF_UPLOAD_BOUNCE") && getenv("BTF_UPLOAD_BOUNCE")[0] == '0');
+    const bool bounce = !on_dev && is_pageable_host_ptr(Y) && e->env.upload_bounce;
     int chunk = nrows;
     if (!on_dev) {
         // two staging buffers: the copy of piece i + 1 (copy stream) runs under the pre-reduction of piece i
@@ -541,7 +563,7 @@ int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int
             const double* hsrc = Y + (size_t)r0 * row_elems;
             if (bounce) {
                 if (piece >= 2) CK(cudaEventSynchronize(e->ev_h2d[b]));                    // the bounce buffer's previous copy has left it
-                parallel_memcpy(e->hstage[b], hsrc, (size_t)rows * row_elems * sizeof(double));
+                parallel_memcpy(e->hstage[b], hsrc, (size_t)rows * row_elems * sizeof(double), e->env.upload_threads);
                 hsrc = e->hstage[b];
             }
             if (piece >= 2) CK(cudaStreamWaitEvent(e->copy_stream, e->ev_k0[b], 0));       // the buffer's previous pre-reduction is done
@@ -634,7 +656,7 @@ int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps) {
         CK(cudaStreamSynchronize(e->stream));
         CK(cudaFree(scan));
         const size_t vstride = (size_t)h[0] + 1;
-        if (!h[1] && vstride * rsize <= ((size_t)1 << 24) && !getenv("BTF_NB_NO_HIST")) {
+        if (!h[1] && vstride * rsize <= ((size_t)1 << 24) && e->env.nb_hist) {
             CK(dev_alloc(&e->nb_hist, vstride * rsize));
             e->nb_hist_stride = (int)vstride;
             NbArgs nb;
@@ -830,6 +852,11 @@ int btf_get_diag(btf_engine* e, const char* name, double* host, size_t n) {
         if (e->guard_n) { int h[2]; CK(cudaMemcpy(h, e->guard_n, sizeof(h), cudaMemcpyDeviceToHost)); host[0] = h[0]; host[1] = h[1]; }
         return BTF_OK;
     }
+    if (nm == "i8_route") {
+        if (n != 2) return set_err(BTF_EINVAL, "i8_route: 2 values");
+        host[0] = e->i8_route[0]; host[1] = e->i8_route[1];
+        return BTF_OK;
+    }
     if (nm == "V_retries") {
         if (n != (size_t)e->Mloc) return set_err(BTF_EINVAL, "V_retries: expected %d values", e->Mloc);
         std::vector<int> tmp(e->Mloc);
@@ -851,8 +878,7 @@ static const char* const kPhaseNames[] = {"btf:nu2_or_pg", "btf:sigma2", "btf:ta
                                           "btf:col_stats", "btf:band_solve", "btf:comm"};
 static inline void phase_mark(btf_engine* e, int idx) {
     if (e->time_phases) cudaEventRecord(e->ph_ev[idx], e->stream);
-    static const bool nvtx = getenv("BTF_NVTX") != nullptr;
-    if (nvtx) {
+    if (e->env.nvtx) {
         if (idx > 0) nvtxRangePop();
         if (idx < PH_COUNT) nvtxRangePushA(kPhaseNames[idx]);
     }
@@ -882,12 +908,12 @@ static int begin_row_stats_i8(btf_engine* e, bool fork, int timer, I8Pending* pd
     cudaEvent_t* ev = (e->time_phases && timer >= 0) ? e->i8_ev[timer] : nullptr;
     fork_side(e, fork);
     stats_i8_digits(e->i8, e->K, e->V, e->P, e->Ppad, sa);
-    if (fork && e->sf_after_digits) { cudaEventRecord(e->ev_digits, sa); cudaStreamWaitEvent(sb, e->ev_digits, 0); }
     if (ev) cudaEventRecord(ev[0], sa);
-    const I8Guard gr{e->cnt_rowsum, e->guard_flags, e->guard_n, stats_i8_guard_tol()};
-    pd->product = stats_i8_product(e->i8, e->K, e->cnt, e->Ppad, e->Ppad, e->nloc, e->nloc_pad, 0, e->row_stats,
-                                   e->guard_on ? &gr : nullptr, sa);
-    if (pd->product != 0 && pd->product != 10) return set_err(BTF_ECUDA, "integer row statistics failed to launch");
+    const I8Guard gr{e->cnt_rowsum, e->guard_flags, e->guard_n, e->env.i8_guard_tol};
+    pd->product = stats_i8_product(e->i8, e->K, e->cnt, e->Ppad, e->Ppad, e->nloc, e->nloc_pad, e->row_stats,
+                                   e->env.i8_guard ? &gr : nullptr, e->env.i8_gemm2, sa);
+    if (!pd->product) return set_err(BTF_ECUDA, "integer row statistics failed to launch");
+    e->i8_route[0] = pd->product;
     if (ev) cudaEventRecord(ev[1], sa);
     pd->nsplit = stats_i8_linear(e->i8, false, e->K, e->S, e->Ppad, e->V, e->Ppad, e->nloc, e->i8.nsplit_b_row, e->i8.bpart, sb);
     if (ev) cudaEventRecord(ev[2], sb);
@@ -896,11 +922,11 @@ static int begin_row_stats_i8(btf_engine* e, bool fork, int timer, I8Pending* pd
 }
 static int finish_row_stats_i8(btf_engine* e, bool fork, const I8Pending& pd) {
     join_side(e, fork);
-    const I8Guard gr{e->cnt_rowsum, e->guard_flags, e->guard_n, stats_i8_guard_tol()};
-    stats_i8_combine(e->i8, e->K, e->nloc, e->nloc_pad, 0, pd.product == 10, e->i8.bpart, pd.nsplit, 0, e->nloc, e->row_stats,
-                     e->guard_on ? &gr : nullptr, e->stream);
+    const I8Guard gr{e->cnt_rowsum, e->guard_flags, e->guard_n, e->env.i8_guard_tol};
+    stats_i8_combine(e->i8, e->K, e->nloc, e->nloc_pad, pd.product == I8_ROUTE_FUSED, e->i8.bpart, pd.nsplit, 0, e->nloc,
+                     e->row_stats, e->env.i8_guard ? &gr : nullptr, e->stream);
     e->launches += 1;
-    if (e->guard_on) {
+    if (e->env.i8_guard) {
         stats_i8_fallback(e->K, e->cnt, e->Ppad, e->V, e->P, e->nloc, e->row_stats, gr, e->stream);
         e->launches += 1;
     }
@@ -909,105 +935,71 @@ static int finish_row_stats_i8(btf_engine* e, bool fork, const I8Pending& pd) {
 
 // Columns: every rank contracts ITS columns over ALL rows (column-sharded copy of the counts, digit planes of the
 // all-gathered W), so the product block needs no exchange; the linear block is a partial sum over the local rows
-// for all columns (S stays row-sharded: it is read once either way) and is reduce-scattered (M T K doubles).
-// The V step is a pipeline over column chunks: the statistics of chunk c + 1 (tensor cores / HBM, side streams) run
-// while the latency-bound band solve of chunk c holds a few warps per SM on the main stream.
-struct ColChunks { int n = 1, cols = 0; };
-static ColChunks plan_col_chunks(const btf_engine* e, bool fork) {
-    ColChunks cc;
-    cc.n = 1; cc.cols = e->Mloc;
-    if (!fork || e->diag || e->col_chunks <= 1 || e->Mloc < 2 * e->col_chunks) return cc;
-    // chunk boundaries on multiples of 256 (j, t) positions: whole GEMM tiles, 16-byte aligned int32 rows
-    int g = 256; { int a = 256, b = e->T; while (b) { int t = a % b; a = b; b = t; } g = 256 / a; }
-    int cols = round_up((e->Mloc + e->col_chunks - 1) / e->col_chunks, g);
-    if (cols >= e->Mloc) return cc;
-    cc.cols = cols; cc.n = (e->Mloc + cols - 1) / cols;
-    return cc;
-}
-
-// band: launches the band solve of local columns [j0, j0 + ncols) on the main stream
+// for all columns (S stays row-sharded: it is read once either way) and is reduce-scattered (M T K doubles), unless
+// the rank holds the column-sharded copy of S.  Then the recombination, the guard's fallback and the band solve.
+// band: launches the band solve of all local columns on the main stream
 template <typename BandFn>
 static int col_step_i8(btf_engine* e, bool fork, int timer, BandFn band) {
     cudaStream_t st = e->stream;
     cudaStream_t sa = fork ? e->side[0] : st, sb = fork ? e->side[1] : st;
     cudaEvent_t* ev = (e->time_phases && timer >= 0) ? e->i8_ev[timer] : nullptr;
-    const int nco = e->nco, T = e->T;
-    const ColChunks cc = plan_col_chunks(e, fork);
-    const int ldd = round_up(std::max(e->Ploc, 1), 256);
+    const int np = e->Ploc;
+    const int ldd = round_up(std::max(np, 1), 256);
     const double* Wloc = e->W + (size_t)e->cfg.row_begin * e->K;
     fork_side(e, fork);
     if (ev) cudaEventRecord(ev[0], sa);
-    if (e->Ploc > 0) { stats_i8_digits(e->i8, e->K, e->W, e->N, e->Nall_pad, sa); e->launches += 2; }
-    if (fork && e->sf_after_digits) { cudaEventRecord(e->ev_digits, sa); cudaStreamWaitEvent(sb, e->ev_digits, 0); }
+    if (np > 0) { stats_i8_digits(e->i8, e->K, e->W, e->N, e->Nall_pad, sa); e->launches += 2; }
     if (ev) cudaEventRecord(ev[0], sa);
     // linear block: sharded engines need the partial sums of ALL columns before the exchange -> one launch
     // (on the side stream when forked; in the serial mode it is issued after the product block, see below)
-    const bool lin_whole = e->shard != nullptr || cc.n == 1;
     const bool scol = e->shard != nullptr && e->Scol != nullptr;     // own columns over all rows: nothing to exchange
-    int whole_split = 1;
-    auto linear_whole = [&]() -> int {
+    int lin_split = 1;
+    auto linear = [&]() -> int {
         if (scol) {
             // (few row tiles per rank: split the contraction so that the launch still fills the GPU; the partials fit in the
             //  2 P K doubles of the buffer because P_loc <= P / world ... and at least P / 2 for two ranks)
-            const int max_split = std::max(1, std::min(8, (int)((2ll * e->P) / std::max(e->Ploc, 1))));
-            if (e->Ploc > 0) { whole_split = stats_i8_linear(e->i8, true, e->K, e->Scol, e->Ploc_pad, e->W, e->Nall_pad, e->Ploc, max_split, e->i8.bpart, sb); e->launches++; }
+            const int max_split = std::max(1, std::min(8, (int)((2ll * e->P) / std::max(np, 1))));
+            if (np > 0) { lin_split = stats_i8_linear(e->i8, true, e->K, e->Scol, e->Ploc_pad, e->W, e->Nall_pad, np, max_split, e->i8.bpart, sb); e->launches++; }
         } else if (e->nloc > 0) {
             // one GPU: the contraction may be split (the partial sums fit in the buffer that also serves the row step);
             // a row-sharded engine reduce-scatters ONE set of partial sums
             const size_t cap = std::max((size_t)e->i8.nsplit_b_row * e->nloc * e->K, (size_t)2 * e->P * e->K) / ((size_t)e->P * e->K);
             const int max_split = e->shard ? 1 : (int)std::min<size_t>(4, std::max<size_t>(cap, 1));
-            whole_split = stats_i8_linear(e->i8, true, e->K, e->S, e->Ppad, Wloc, e->nloc_pad, e->P, max_split, e->i8.bpart, sb); e->launches++;
+            lin_split = stats_i8_linear(e->i8, true, e->K, e->S, e->Ppad, Wloc, e->nloc_pad, e->P, max_split, e->i8.bpart, sb); e->launches++;
         } else {
             cudaMemsetAsync(e->i8.bpart, 0, (size_t)e->P * e->K * sizeof(double), sb);
         }
         if (fork) { cudaEventRecord(e->ev_join[1], sb); cudaStreamWaitEvent(st, e->ev_join[1], 0); }
-        if (e->shard && !scol && nccl_reduce_scatter_cols(e->shard, e->i8.bpart, (size_t)T * e->K, st))
+        if (e->shard && !scol && nccl_reduce_scatter_cols(e->shard, e->i8.bpart, (size_t)e->T * e->K, st))
             return set_err(BTF_ENCCL, "reduce-scatter(linear block) failed: %s", nccl_shard_error());
         return BTF_OK;
     };
-    if (lin_whole && fork) { int rc = linear_whole(); if (rc) return rc; }
-    int product = 0, lin_split = 1;
-    for (int c = 0; c < cc.n; ++c) {
-        const int j0 = c * cc.cols, ncols = std::min(cc.cols, e->Mloc - j0);
-        const long long q0 = (long long)j0 * T;            // first local (j, t) of the chunk
-        const int np = ncols * T;
-        double* out = e->col_stats + ((size_t)e->p0 + q0) * nco;
-        if (np > 0) {
-            const I8Guard gc{e->cnt_colsum + q0, e->guard_flags + std::max(e->nloc, 1) + q0, e->guard_n + 1, stats_i8_guard_tol()};
-            product = stats_i8_product(e->i8, e->K, e->cntT + (size_t)q0 * e->Nall_pad, e->Nall_pad, e->Nall_pad, np, ldd, q0, out,
-                                       e->guard_on ? &gc : nullptr, sa);
-            if (product != 0 && product != 10) return set_err(BTF_ECUDA, "integer column statistics failed to launch");
-            e->launches++;
-            if (!lin_whole) {
-                // a chunk's tiles alone are less than one wave: up to two splits, kept in the chunk's own region
-                lin_split = stats_i8_linear(e->i8, true, e->K, e->S + e->p0 + q0, e->Ppad, Wloc, e->nloc_pad, np, 2,
-                                            e->i8.bpart + (size_t)2 * q0 * e->K, sb);
-                e->launches++;
-            }
-        }
-        if (fork) {
-            cudaEventRecord(e->ev_chunk[0][c], sa); cudaStreamWaitEvent(st, e->ev_chunk[0][c], 0);
-            if (!lin_whole) { cudaEventRecord(e->ev_chunk[1][c], sb); cudaStreamWaitEvent(st, e->ev_chunk[1][c], 0); }
-        }
-        if (c == cc.n - 1 && ev) cudaEventRecord(ev[1], sa);
-        if (lin_whole && !fork) { int rc = linear_whole(); if (rc) return rc; }     // serial mode: one chunk
-        if (c == cc.n - 1 && ev) cudaEventRecord(ev[2], sb);
-        if (np > 0) {
-            const I8Guard gc{e->cnt_colsum + q0, e->guard_flags + std::max(e->nloc, 1) + q0, e->guard_n + 1, stats_i8_guard_tol()};
-            const I8Guard* gp = e->guard_on ? &gc : nullptr;
-            if (lin_whole && scol) stats_i8_combine(e->i8, e->K, np, ldd, q0, product == 10, e->i8.bpart, whole_split, q0, e->Ploc, out, gp, st);
-            else if (lin_whole) stats_i8_combine(e->i8, e->K, np, ldd, q0, product == 10, e->i8.bpart, whole_split, (long long)e->p0 + q0, e->P, out, gp, st);
-            else stats_i8_combine(e->i8, e->K, np, ldd, q0, product == 10, e->i8.bpart + (size_t)2 * q0 * e->K, lin_split, 0, np, out, gp, st);
-            e->launches++;
-            if (e->guard_on) {
-                stats_i8_fallback(e->K, e->cntT + (size_t)q0 * e->Nall_pad, e->Nall_pad, e->W, e->N, np, out, gc, st);
-                e->launches += 1;
-            }
-        }
-        if (c == 0) phase_mark(e, PH_BAND_SOLVE);
-        if (ncols > 0) band(j0, ncols);
+    if (fork) { int rc = linear(); if (rc) return rc; }
+    int product = 0;
+    double* out = e->col_stats + (size_t)e->p0 * e->nco;
+    const I8Guard gc{e->cnt_colsum, e->guard_flags + std::max(e->nloc, 1), e->guard_n + 1, e->env.i8_guard_tol};
+    const I8Guard* gp = e->env.i8_guard ? &gc : nullptr;
+    if (np > 0) {
+        product = stats_i8_product(e->i8, e->K, e->cntT, e->Nall_pad, e->Nall_pad, np, ldd, out, gp, e->env.i8_gemm2, sa);
+        if (!product) return set_err(BTF_ECUDA, "integer column statistics failed to launch");
+        e->i8_route[1] = product;
+        e->launches++;
     }
-    if (cc.n == 0 || e->Mloc == 0) phase_mark(e, PH_BAND_SOLVE);
+    if (fork) { cudaEventRecord(e->ev_join[0], sa); cudaStreamWaitEvent(st, e->ev_join[0], 0); }
+    if (ev) cudaEventRecord(ev[1], sa);
+    if (!fork) { int rc = linear(); if (rc) return rc; }
+    if (ev) cudaEventRecord(ev[2], sb);
+    if (np > 0) {
+        stats_i8_combine(e->i8, e->K, np, ldd, product == I8_ROUTE_FUSED, e->i8.bpart, lin_split, scol ? 0 : e->p0,
+                         scol ? np : e->P, out, gp, st);
+        e->launches++;
+        if (gp) {
+            stats_i8_fallback(e->K, e->cntT, e->Nall_pad, e->W, e->N, np, out, gc, st);
+            e->launches += 1;
+        }
+    }
+    phase_mark(e, PH_BAND_SOLVE);
+    if (e->Mloc > 0) band();
     return cudaGetLastError() == cudaSuccess ? BTF_OK : set_err(BTF_ECUDA, "integer column statistics failed");
 }
 
@@ -1019,12 +1011,11 @@ static int ensure_i8(btf_engine* e) {
     if (e->i8_decided) return BTF_OK;
     e->i8_decided = true;
     e->i8_on = false;
-    if (e->cfg.likelihood != BTF_GAUSSIAN || !e->has_data) return BTF_OK;
-    const bool force = getenv("BTF_STATS_FORCE_I8") != nullptr;
+    if (e->cfg.likelihood != BTF_GAUSSIAN || !e->has_data || e->env.no_i8) return BTF_OK;
     const long long cells = (long long)e->N * e->P / std::max(1, e->cfg.world_size);
     if (!stats_i8_supported(e->K, e->nreps, e->Ppad, e->Nall_pad)) return BTF_OK;
     if (e->cfg.world_size > 1 && !e->shard) return BTF_OK;       // a shard without a communicator cannot build its column copy
-    if (!force && cells < (1ll << 24)) return BTF_OK;
+    if (!e->env.force_i8 && cells < (1ll << 24)) return BTF_OK;
     cudaStream_t st = e->stream;
     if (!e->i8.planes) {
         StatsI8Sizes z;
@@ -1040,7 +1031,6 @@ static int ensure_i8(btf_engine* e) {
         CK(dev_alloc(&e->cnt_colsum, (size_t)std::max(e->Ploc, 1)));
         CK(dev_alloc(&e->guard_n, 2));
         CK(dev_alloc(&e->guard_flags, (size_t)std::max(e->nloc, 1) + std::max(e->Ploc, 1)));
-        e->guard_on = getenv("BTF_I8_NO_GUARD") == nullptr;
         e->i8.nsplit_b_row = z.nsplit_b_row;
     }
     if (!e->shard) {
@@ -1066,7 +1056,7 @@ static int ensure_i8(btf_engine* e) {
         // all rows and the M T K reduce-scatter disappears from the critical path (C2 on 8 GPUs: 0.06 of 0.77 ms).
         e->Ploc_pad = round_up(std::max(e->Ploc, 1), 256);
         if (e->Scol) { cudaFree(e->Scol); e->Scol = nullptr; }
-        if (!getenv("BTF_NO_SCOL")) {
+        if (e->env.scol) {
             const size_t max_rows = (size_t)std::max(nccl_shard_max_rows(e->shard), 1);
             const size_t max_pl = (size_t)round_up(std::max(nccl_shard_max_cols(e->shard), 1) * e->T, 256);
             const size_t need = ((size_t)e->Nall_pad + 32) * max_pl * 8 + 2 * max_rows * max_pl * 8;
@@ -1110,7 +1100,7 @@ static int ensure_i8(btf_engine* e) {
         int rc = begin_row_stats_i8(e, false, -1, &pd); if (rc) { e->i8_on = false; return rc; }
         rc = finish_row_stats_i8(e, false, pd); if (rc) { e->i8_on = false; return rc; }
     }
-    { int rc = col_step_i8(e, false, -1, [](int, int) {}); if (rc) { e->i8_on = false; return rc; } }
+    { int rc = col_step_i8(e, false, -1, []() {}); if (rc) { e->i8_on = false; return rc; } }
     CK(cudaStreamSynchronize(st));
     free_graph(e);
     return BTF_OK;
@@ -1139,7 +1129,7 @@ static int enqueue_sweep(btf_engine* e) {
     // Integer statistics path: the row statistics only read V and the data, so they start now on the side streams
     // (tensor-core product block | HBM-bound linear block) while the hyper-parameter steps run on the main stream.
     const bool doW = (mask & BTF_SAMPLE_W) && e->nloc > 0;
-    const bool fork = e->overlap && e->i8_on && !e->time_phases;
+    const bool fork = e->i8_on && !e->time_phases;
     I8Pending pend_row;
     if (fork && doW) { int rc = begin_row_stats_i8(e, true, 0, &pend_row); if (rc) return rc; }
 
@@ -1266,25 +1256,17 @@ static int enqueue_sweep(btf_engine* e) {
         ba.work_L = e->work_L; ba.work_y = e->work_y;
         ba.work_L_stride = e->wL_stride; ba.work_y_stride = e->wy_stride;
         ba.force_psd = c.force_psd; ba.attempts = c.force_psd_attempts; ba.eps = c.force_psd_eps;
-        ba.rotate_roles = getenv("BTF_BAND_ROT") ? e->sm_count : 0;     // (measured: no gain, off by default)
+        ba.force_scalar = e->env.band_scalar;
         const size_t bn = (size_t)e->Mloc * e->n * (e->kd + 1);
         ba.diag_band = diag_get(e, "V_band", bn);
         ba.diag_chol = diag_get(e, "V_chol", bn);
         ba.diag_mean = diag_get(e, "V_mean", (size_t)e->P * e->K);
         ba.diag_retries = e->diag_retries;
         ba.resid_partials = gauss ? e->resid_partials + c.col_begin : nullptr;
-        // the band solve of local columns [j0, j0 + ncols): every per-column array of the kernel is indexed from its base
-        auto band = [&](int j0, int ncols) {
-            BandSolveArgs b = ba;
-            b.col_begin = c.col_begin + j0; b.ncols_loc = ncols;
-            b.work_L = ba.work_L + (size_t)j0 * ba.work_L_stride; b.work_y = ba.work_y + (size_t)j0 * ba.work_y_stride;
-            if (b.resid_partials) b.resid_partials += j0;
-            if (b.diag_retries) b.diag_retries += j0;
-            launch_band_solve(b, st); e->launches++;
-        };
+        auto band = [&]() { launch_band_solve(ba, st); e->launches++; };
         if (e->i8_on) {
             e->col_collapsed = false;
-            int rc = col_step_i8(e, fork, 1, band);      // statistics and band solves, pipelined over column chunks
+            int rc = col_step_i8(e, fork, 1, band);
             if (rc) return rc;
         } else {
             int nsplit = e->plan_col.nsplit;
@@ -1310,7 +1292,7 @@ static int enqueue_sweep(btf_engine* e) {
             }
             ba.nsplit = nsplit;
             phase_mark(e, PH_BAND_SOLVE);
-            if (e->Mloc > 0) band(0, e->Mloc);
+            if (e->Mloc > 0) band();
         }
         phase_mark(e, PH_COMM);
         if (e->shard) {
@@ -1743,6 +1725,7 @@ int btf_init_state(btf_engine* e, int32_t init_mask) {
         ba.work_L = tmp ? wl : e->work_L; ba.work_y = tmp ? wy : e->work_y;
         ba.work_L_stride = e->wL_stride; ba.work_y_stride = e->wy_stride;
         ba.force_psd = c.force_psd; ba.attempts = c.force_psd_attempts; ba.eps = c.force_psd_eps;
+        ba.force_scalar = e->env.band_scalar;
         launch_band_solve(ba, st);
         launch_clip(e->V, (size_t)e->P * e->K, -10.0, 10.0, st);
         e->launches += 2;
@@ -1809,7 +1792,7 @@ int btf_nccl_init(btf_engine* e, const char* id128) {
                                  e->cfg.col_begin, e->cfg.col_end);
     if (!e->shard) return set_err(BTF_ENCCL, "NCCL init failed: %s", nccl_shard_error());
     // the lam2 step in its all-columns form needs every column's new Tau2: keep the chain replicated there
-    e->tau_sharded = e->cfg.ref_compat_lam2 != 0 && getenv("BTF_TAU_REPLICATED") == nullptr;
+    e->tau_sharded = e->cfg.ref_compat_lam2 != 0;
     e->i8_decided = false;
     return BTF_OK;
 }

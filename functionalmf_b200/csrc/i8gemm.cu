@@ -27,7 +27,6 @@ constexpr int I8_BM = 128, I8_BN = 256, I8_BK = 128, I8_STAGES = 4, I8_LAG = 2;
 constexpr int I8_A_BYTES = I8_BM * I8_BK, I8_B_BYTES = I8_BN * I8_BK, I8_STAGE_BYTES = I8_A_BYTES + I8_B_BYTES;
 constexpr int I8_SMEM = I8_STAGES * I8_STAGE_BYTES + 1024 /*alignment*/ + 256 /*barriers*/;
 constexpr int I8_SMEM2 = 2 * I8_STAGE_BYTES + 1024 + 256;     // two-stage variant: two CTAs per SM
-constexpr int I8_SMEM3 = 3 * I8_STAGE_BYTES + 1024 + 256;     // three stages, one CTA per SM, 78 KB left for a co-resident kernel
 constexpr int I8_TMEM_COLS = 256;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -224,7 +223,6 @@ int launch_i8gemm(const int8_t* A, long long lda, int M, const int8_t* B, long l
     if (attr_once.first()) {
         if (cudaFuncSetAttribute(i8gemm_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, I8_SMEM) != cudaSuccess) return 2;
         if (cudaFuncSetAttribute(i8gemm_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, I8_SMEM2) != cudaSuccess) return 2;
-        if (cudaFuncSetAttribute(i8gemm_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, I8_SMEM3) != cudaSuccess) return 2;
     }
     const int mt = (M + I8_BM - 1) / I8_BM, nt = (N + I8_BN - 1) / I8_BN, nchunks = K / I8_BK;
     // split-K when the tiles alone cannot fill the GPU (few rows: multi-GPU shards, small tensors)
@@ -243,11 +241,7 @@ int launch_i8gemm(const int8_t* A, long long lda, int M, const int8_t* B, long l
     I8Args p{A, lda, M, B, ldb, N, K, D, ldd, cps};
     dim3 grid(mt, nt, nsplit);
     // short contractions with many tiles: two CTAs per SM hide the per-CTA prologue and epilogue
-    // BTF_I8_STAGES = 2 | 3 | 4 forces a variant; 3 leaves room on every SM for one CTA of the linear-block kernel
-    const char* force = getenv("BTF_I8_STAGES");
-    const int stages = force ? (force[0] - '0') : ((cps <= 64 && mt * nt * nsplit >= 2 * 148) ? 2 : 4);
-    if (stages == 2) i8gemm_kernel<2><<<grid, 160, I8_SMEM2, st>>>(p);
-    else if (stages == 3) i8gemm_kernel<3><<<grid, 160, I8_SMEM3, st>>>(p);
+    if (cps <= 64 && mt * nt * nsplit >= 2 * 148) i8gemm_kernel<2><<<grid, 160, I8_SMEM2, st>>>(p);
     else i8gemm_kernel<4><<<grid, 160, I8_SMEM, st>>>(p);
     return cudaGetLastError() == cudaSuccess ? 0 : 3;
 }

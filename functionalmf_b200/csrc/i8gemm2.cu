@@ -32,10 +32,10 @@ namespace {
 
 constexpr int G2_ROWS = 128;                 // count rows / digit rows per CTA and stage
 constexpr int G2_BK = 128;                   // bytes of K per stage
-constexpr int G2_MAX_STAGES = 6;                          // 4 stages (130 KB) leave room for one CTA of the linear-block kernel per SM
+constexpr int G2_STAGES = 6;                              // operand stages (196 KB)
 constexpr int G2_TILE_BYTES = G2_ROWS * G2_BK;            // 16 KB
 constexpr int G2_STAGE_BYTES = 2 * G2_TILE_BYTES;         // counts + digits
-constexpr int g2_smem(int stages) { return stages * G2_STAGE_BYTES + 1024 /*alignment*/ + 256 /*barriers*/; }
+constexpr int G2_SMEM = G2_STAGES * G2_STAGE_BYTES + 1024 /*alignment*/ + 256 /*barriers*/;
 constexpr int G2_TMEM_COLS = 512;            // two accumulator stages of 256 columns
 constexpr int G2_THREADS = 192;              // warp 0: TMA, warp 1: MMA + tensor-memory allocation, warps 2-5: epilogue
 constexpr int G2_CPT = I8_COLS_PER_TILE;     // 36 product columns per tile
@@ -125,7 +125,6 @@ struct G2Args {
     int32_t* D; long long ldd;
 };
 
-template <int G2_STAGES>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G2_THREADS, 1)
 i8gemm2_kernel(const __grid_constant__ CUtensorMap tm_cnt, const __grid_constant__ CUtensorMap tm_dig, G2Args p) {
     const CUtensorMap* tm_cnt_p = &tm_cnt;     // counts
@@ -359,14 +358,11 @@ int launch_i8gemm2(const int8_t* Cn, long long ldc, int M, const int8_t* Pl, lon
     int sms = 148;
     { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); }
     static PerDeviceOnce attr_once;
-    if (attr_once.first()) {
-        if (cudaFuncSetAttribute(i8gemm2_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, g2_smem(6)) != cudaSuccess ||
-            cudaFuncSetAttribute(i8gemm2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, g2_smem(4)) != cudaSuccess) {
-            cudaGetLastError();
-            return 1;
-        }
+    if (attr_once.first() &&
+        cudaFuncSetAttribute(i8gemm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, G2_SMEM) != cudaSuccess) {
+        cudaGetLastError();
+        return 1;
     }
-    static const bool four = getenv("BTF_I8_G2_STAGES") != nullptr && getenv("BTF_I8_G2_STAGES")[0] == '4';
     if (nt > 16) return 1;
     // the descriptors travel as kernel parameters (a CUDA graph keeps its own copy of them)
     alignas(64) CUtensorMap tm_cnt, tm_dig;
@@ -383,12 +379,8 @@ int launch_i8gemm2(const int8_t* Cn, long long ldc, int M, const int8_t* Pl, lon
         p.cntsum = guard->cntsum; p.flags = guard->flags; p.tol = guard->tol;
         for (int k = 0; k * (k + 3) / 2 < L; ++k) { const int c = k * (k + 3) / 2; p.diag_mask[c / G2_CPT] |= 1ull << (c % G2_CPT); }
     }
-    // BTF_I8_G2_PAIRS=n: at most n CTA pairs, so that the rest of the SMs stay free for the linear block on the other stream
-    static const int pair_cap = getenv("BTF_I8_G2_PAIRS") ? atoi(getenv("BTF_I8_G2_PAIRS")) : 0;
-    int pairs = std::min(sms / 2, mt * nt * p.nsplit);
-    if (pair_cap > 0 && p.nsplit == 1) pairs = std::min(pairs, pair_cap);
-    if (four) i8gemm2_kernel<4><<<2 * pairs, G2_THREADS, g2_smem(4), st>>>(tm_cnt, tm_dig, p);
-    else i8gemm2_kernel<6><<<2 * pairs, G2_THREADS, g2_smem(6), st>>>(tm_cnt, tm_dig, p);
+    const int pairs = std::min(sms / 2, mt * nt * p.nsplit);
+    i8gemm2_kernel<<<2 * pairs, G2_THREADS, G2_SMEM, st>>>(tm_cnt, tm_dig, p);
     if (cudaGetLastError() != cudaSuccess) return 2;
     return p.nsplit > 1 ? 5 : 0;
 }

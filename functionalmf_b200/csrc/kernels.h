@@ -47,7 +47,7 @@ struct StatsPlan {
     int K, L, nct_z, nct_f, zw;
     int BM, KC;
     int mtiles, nchunks, nsplit, chunks_per_split;
-    int overlap;      // 1: Z generation overlapped with the DMMA loop (compile-time-K kernels), 2: + column parts
+    int overlap;      // 1: Z generation overlapped with the DMMA loop (K = 32, f64 weights)
     int zpre, zwg;    // 1: right operand pre-generated in global memory with row pitch zwg (stats_zpre.cu)
     size_t smem_bytes;
     size_t out_elems_per_split;   // m_valid * (L+K)
@@ -61,8 +61,8 @@ bool plan_stats(StatsPlan* plan, int K, bool trans, bool weights_f64, int mdim_p
 void launch_stats(const StatsPlan& plan, bool trans, bool weights_f64, const void* wt, const double* sv,
                   const double* F, long long frows, long long ld, int m_valid, double* out, double* zscratch,
                   cudaStream_t st);
-bool plan_stats_zpre(StatsPlan* p, bool trans, bool weights_f64, int mdim_pad, int kdim_pad, int nsplit_request,
-                     int sm_count);
+// count weights at K = 16 / 32
+bool plan_stats_zpre(StatsPlan* p, bool trans, int mdim_pad, int kdim_pad, int nsplit_request, int sm_count);
 void launch_stats_zpre(const StatsPlan& p, bool trans, const void* wt, const double* sv, const double* F,
                        long long frows, long long ld, int m_valid, double* out, double* Zg, cudaStream_t st);
 
@@ -82,7 +82,6 @@ struct StatsI8Buffers {
     int32_t* D;                     // [i8_plane_rows(L)][m_pad] exact digit-plane contractions (split-K route only)
     double* bpart;                  // [nsplit][m][K] partial sums of the linear block
     int nsplit_b_row;
-    cudaEvent_t ev[3];              // optional timers: before the GEMM, after the GEMM, after the linear block (null: off)
 };
 bool stats_i8_supported(int K, int nreps, long long kdim_row, long long kdim_col);
 // nall_pad: padded GLOBAL row count (contraction length of the column side), ploc: columns (j,t) owned by this rank
@@ -97,25 +96,24 @@ struct I8Guard {
 };
 // the four stages of the integer path (engine: tensor-core contraction and HBM-bound linear block on separate streams)
 void stats_i8_digits(const StatsI8Buffers& w, int K, const double* F, int f_rows, int kdim_pad, cudaStream_t st);
+// route of the product block: round-1 kernel / 2-CTA kernel in split-K mode (both leave int32 planes in w.D for
+// stats_i8_combine), or the 2-CTA kernel whose fused epilogue wrote `out`
+enum I8Route { I8_ROUTE_ROUND1 = 1, I8_ROUTE_FUSED = 2, I8_ROUTE_SPLITK = 3 };
+// gemm2 (BTF_I8_GEMM2): 0 never the 2-CTA kernel, 1 always, -1 when its 256 x 256 tiles fill most CTA pairs;
+// returns the I8Route taken, 0 when a launch failed
 int stats_i8_product(const StatsI8Buffers& w, int K, const uint8_t* B, long long ldb, int kdim_pad, int m_valid, int m_pad,
-                     long long d_off, double* out, const I8Guard* guard, cudaStream_t st);     // 0: int32 planes in w.D + d_off, 10: fused epilogue wrote out, else error
+                     double* out, const I8Guard* guard, int gemm2, cudaStream_t st);
 int stats_i8_linear(const StatsI8Buffers& w, bool trans, int K, const double* S, long long lds, const double* F,
                     int kdim_pad, int m_valid, int max_split, double* out, cudaStream_t st);     // returns the split count of `out`
-void stats_i8_combine(const StatsI8Buffers& w, int K, int m_valid, int m_pad, long long d_off, bool product_done,
+void stats_i8_combine(const StatsI8Buffers& w, int K, int m_valid, int m_pad, bool product_done,
                       const double* bpart, int nsplit_b, long long bpart_m0, long long bpart_rows, double* out,
                       const I8Guard* guard, cudaStream_t st);
 // element-wise guard of the fixed-point product block (see stats_i8.cu): the kernels that produce the block flag the rows
 // whose diagonal entries cannot be guaranteed to `tol` relative (2^(e_c - 55) sum_k cnt[m][k] > tol out[m][(k,k)]);
 // stats_i8_fallback recomputes the flagged rows in FP64, clears the flags and counts them in *nflag.
-
-double stats_i8_guard_tol();    // BTF_I8_GUARD_TOL, default 1e-12
 void stats_i8_count_rows(const uint8_t* B, long long ldb, int m_valid, int kdim_pad, unsigned* cntsum, cudaStream_t st);
 void stats_i8_fallback(int K, const uint8_t* B, long long ldb, const double* F, int f_rows, int m_valid, double* out,
                        const I8Guard& g, cudaStream_t st);
-// out[m][L+K] (one split) for count weights: exact product block + FP64 linear block, all stages on one stream
-int launch_stats_i8(const StatsI8Buffers& w, bool trans, int K, const uint8_t* B, long long ldb, const double* S,
-                    long long lds, const double* F, int f_rows, int kdim_pad, int m_valid, int m_pad, double* out,
-                    cudaStream_t st);
 
 // ---------------------------------------------------------------- residual (nu2)
 // resid_partials[b] = sum over the block's cells of cnt*Mu^2 - 2*Mu*S
@@ -182,7 +180,7 @@ struct BandSolveArgs {
     double* work_y;        // [ncols_loc][work_y_stride]  y | 1/diag(L)
     size_t work_L_stride, work_y_stride;   // per-column strides (sized for the padded block size)
     int force_psd, attempts; double eps;
-    int rotate_roles;      // look-ahead kernel: > 0 rotates the warp-role map by blockIdx / rotate_roles (= #SMs), 0 = off
+    int force_scalar;      // 1: the scalar kernel even where the look-ahead kernel applies (BTF_BAND_SCALAR)
     double *diag_band, *diag_chol, *diag_mean; int* diag_retries;
     double* resid_partials;   // [ncols_loc]: sum_t v^T A v - 2 v.b   (nu2 by-product)
 };

@@ -341,16 +341,9 @@ void launch_pg_draw(const PgArgs& a, cudaStream_t st) {
     }
     dim3 grid((a.P + 255) / 256, (a.nloc + 31) / 32);
     // 80 registers / three CTAs per SM instead of 126 / two (the sampler is a chain of dependent FP64 operations: more
-    // resident warps hide more of its latency, at the price of a few spilled values): 11.4 -> 10.4 ms at C3; BTF_PG_OCC=2 for the old build
-    static const bool occ3 = !(getenv("BTF_PG_OCC") != nullptr && getenv("BTF_PG_OCC")[0] == '2');
-    if (occ3) {
-        if (a.K <= 8) pg_draw_kernel<8, 3><<<grid, 256, 0, st>>>(a);
-        else if (a.K <= 16) pg_draw_kernel<16, 3><<<grid, 256, 0, st>>>(a);
-        else pg_draw_kernel<32, 2><<<grid, 256, 0, st>>>(a);
-        return;
-    }
-    if (a.K <= 8) pg_draw_kernel<8, 2><<<grid, 256, 0, st>>>(a);
-    else if (a.K <= 16) pg_draw_kernel<16, 2><<<grid, 256, 0, st>>>(a);
+    // resident warps hide more of its latency, at the price of a few spilled values): 11.4 -> 10.4 ms at C3
+    if (a.K <= 8) pg_draw_kernel<8, 3><<<grid, 256, 0, st>>>(a);
+    else if (a.K <= 16) pg_draw_kernel<16, 3><<<grid, 256, 0, st>>>(a);
     else pg_draw_kernel<32, 2><<<grid, 256, 0, st>>>(a);
 }
 

@@ -395,8 +395,7 @@ __global__ void band_solve_kernel(BandSolveArgs a) {
 }
 
 void launch_band_solve(const BandSolveArgs& a, cudaStream_t st) {
-    static const bool force_scalar = getenv("BTF_BAND_SCALAR") != nullptr;
-    if (!force_scalar && launch_band_solve_lookahead(a, st)) return;    // blocked look-ahead kernel (band_lookahead.cu): K <= 32, order <= 3
+    if (!a.force_scalar && launch_band_solve_lookahead(a, st)) return;    // blocked look-ahead kernel (band_lookahead.cu): K <= 32, order <= 3
     const int q = a.order + 1, kd = q * a.K, L = a.K * (a.K + 1) / 2, nco = L + a.K;
     int nt = ((kd + 2 + 31) / 32) * 32;
     int nt2 = (((nco + 3) / 4 + 31) / 32) * 32;

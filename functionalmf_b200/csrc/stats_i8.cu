@@ -126,9 +126,8 @@ __global__ void __launch_bounds__(256) zdigits_kernel(const double* __restrict__
 // out[split][m][j] = sum_k S[m,k] F[k,j] over the split's k range: FP64 tensor pipe, HBM bound.
 // 128 rows x KC contraction elements per stage, NST stages; a warp owns 16 rows x all columns = 2 CT independent
 // accumulator chains (the FP64 mma has a long latency: two chains left the pipe 40 % idle).
-// Work items (row tile, split) are dealt round-robin to the CTAs of the grid: one item per CTA in the classic
-// launch (KC = 32, two stages, two CTAs per SM), several in the co-resident launch (KC = 16, three stages, ONE CTA
-// per SM with < 77 KB of shared memory, so that it shares every SM with one CTA of the int8 GEMM).
+// Work items (row tile, split) are dealt round-robin to the CTAs of the grid; launch_sf_t gives every item its own
+// CTA (KC = 32, two stages, two CTAs per SM).
 template <int KB, bool TRANS, int KC, int NST, int MINB>
 __global__ void __launch_bounds__(256, MINB) sf_kernel(const double* __restrict__ S, long long lds, const double* __restrict__ F,
                                                        int K, int m_valid, int nchunks, int chunks_per_split, int m_tiles,
@@ -365,33 +364,23 @@ __global__ void __launch_bounds__(256) transpose_u8_kernel(const uint8_t* __rest
     }
 }
 
-template <int KB, bool TRANS, int KC, int NST, int MINB>
-void launch_sf_cfg(const double* S, long long lds, const double* F, int K, int m_valid, int m_tiles, int nchunks,
-                   int nsplit, int grid, double* out, cudaStream_t st) {
+// contraction chunks of 32 through a 2-stage ring, two CTAs per SM, one CTA per (tile, split) item
+template <int KB, bool TRANS>
+void launch_sf_t(const double* S, long long lds, const double* F, int K, int m_valid, int m_tiles, int nchunks, int nsplit,
+                 double* out, cudaStream_t st) {
+    constexpr int KC = 32, NST = 2;
     const size_t smem = (size_t)(NST * (TRANS ? KC * 132 : 128 * (KC + 4)) + NST * KC * (KB + 4)) * sizeof(double);
-    auto kern = sf_kernel<KB, TRANS, KC, NST, MINB>;
+    auto kern = sf_kernel<KB, TRANS, KC, NST, 2>;
     static PerDeviceOnce once;
     if (once.first()) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     const int cps = (nchunks + nsplit - 1) / nsplit;
     const int nitems = m_tiles * nsplit;
-    kern<<<grid > 0 ? std::min(grid, nitems) : nitems, 256, smem, st>>>(S, lds, F, K, m_valid, nchunks, cps, m_tiles, nitems, out);
-}
-
-// resident = true: the co-resident configuration (one 3-stage CTA per SM, contraction chunks of 16, `grid` CTAs)
-template <int KB, bool TRANS>
-void launch_sf_t(const double* S, long long lds, const double* F, int K, int m_valid, int m_tiles, int nchunks32,
-                 int nsplit, bool resident, int grid, double* out, cudaStream_t st) {
-    // BTF_SF_DEEP=1: chunks of 16 through a 4-stage ring, two CTAs per SM (more, smaller copies in flight)
-    static const bool deep = getenv("BTF_SF_DEEP") != nullptr && getenv("BTF_SF_DEEP")[0] != '0';
-    if (resident) launch_sf_cfg<KB, TRANS, 16, 3, 1>(S, lds, F, K, m_valid, m_tiles, nchunks32 * 2, nsplit, grid, out, st);
-    else if (deep) launch_sf_cfg<KB, TRANS, 16, 4, 2>(S, lds, F, K, m_valid, m_tiles, nchunks32 * 2, nsplit, 0, out, st);
-    else launch_sf_cfg<KB, TRANS, 32, 2, 2>(S, lds, F, K, m_valid, m_tiles, nchunks32, nsplit, 0, out, st);
+    kern<<<nitems, 256, smem, st>>>(S, lds, F, K, m_valid, nchunks, cps, m_tiles, nitems, out);
 }
 
 }  // namespace
 
 bool stats_i8_supported(int K, int nreps, long long kdim_row, long long kdim_col) {
-    if (getenv("BTF_STATS_NO_I8") != nullptr) return false;      // read per data set, so a process can switch
     if (!(K == 8 || K == 16 || K == 32)) return false;
     if (nreps < 1 || nreps > 127) return false;
     const long long kd = kdim_row > kdim_col ? kdim_row : kdim_col;
@@ -406,7 +395,7 @@ void stats_i8_sizes(int K, int nloc_pad, int Ppad, int nloc, int P, int nall_pad
     s->d_elems = (size_t)i8_plane_rows((int)L) * nd;
     s->cntT_bytes = (size_t)std::max(ploc, 1) * nall_pad;
     s->nsplit_b_row = 64;            // upper bound of the split count of the row-variant linear block (buffer size)
-    s->bpart_elems = std::max((size_t)s->nsplit_b_row * nloc * K, (size_t)2 * P * K);   // columns: up to two splits per chunk
+    s->bpart_elems = std::max((size_t)s->nsplit_b_row * nloc * K, (size_t)2 * P * K);   // columns: the split counts fit in 2 P K
     s->L = (int)L;
 }
 
@@ -432,24 +421,19 @@ void stats_i8_digits(const StatsI8Buffers& w, int K, const double* F, int f_rows
 }
 
 // 2. exact product block on the tensor cores: D[(8 c + s)][m] = sum_k d_s[k, c] B[m][k], m < m_valid (B = counts, K-major)
-//    returns 0 (int32 planes in w.D), 10 (fused epilogue wrote out[m][c] directly), else an error
 int stats_i8_product(const StatsI8Buffers& w, int K, const uint8_t* B, long long ldb, int kdim_pad, int m_valid, int m_pad,
-                     long long d_off, double* out, const I8Guard* guard, cudaStream_t st) {
+                     double* out, const I8Guard* guard, int gemm2, cudaStream_t st) {
     const int L = K * (K + 1) / 2;
-    // BTF_I8_GEMM2 = 0: never the 2-CTA kernel; = 1: always (tests); default: when its 256 x 256 tiles fill most CTA pairs
-    static const char* g2 = getenv("BTF_I8_GEMM2");
-    const int min_tiles = g2 ? (g2[0] == '0' ? (1 << 30) : 0) : 48;
-    // BTF_I8_G2_SPLITK=0: few-tile shapes take the round-1 kernel instead of the split-K mode of the 2-CTA kernel
-    static const bool g2split = !(getenv("BTF_I8_G2_SPLITK") != nullptr && getenv("BTF_I8_G2_SPLITK")[0] == '0');
+    const int min_tiles = gemm2 == 0 ? (1 << 30) : (gemm2 == 1 ? 0 : 48);
     const int rc = launch_i8gemm2(reinterpret_cast<const int8_t*>(B), ldb, m_valid, w.planes, kdim_pad, L, kdim_pad, w.expo, out,
-                                  L + K, min_tiles, guard, g2split ? w.D + d_off : nullptr, m_pad, st);
-    if (rc == 0) return 10;
-    if (rc == 5) return 0;          // exact int32 partial sums in w.D: the recombination kernel finishes (and applies the guard)
-    if (rc > 1) return 1;
+                                  L + K, min_tiles, guard, w.D, m_pad, st);
+    if (rc == 0) return I8_ROUTE_FUSED;
+    if (rc == 5) return I8_ROUTE_SPLITK;    // exact int32 partial sums in w.D: the recombination kernel finishes (and applies the guard)
+    if (rc > 1) return 0;
     // few tiles (small tensors, narrow shards): 128 x 256 tiles with split-K and integer atomics through the int32 planes
     // (the recombination kernel applies the guard on this route)
-    return launch_i8gemm(w.planes, kdim_pad, i8_plane_rows(L), reinterpret_cast<const int8_t*>(B), ldb, m_valid, kdim_pad, w.D + d_off,
-                         m_pad, st) ? 1 : 0;
+    return launch_i8gemm(w.planes, kdim_pad, i8_plane_rows(L), reinterpret_cast<const int8_t*>(B), ldb, m_valid, kdim_pad, w.D,
+                         m_pad, st) ? 0 : I8_ROUTE_ROUND1;
 }
 
 // 3. linear block in FP64: bpart[split][m][j] = sum_k S[m, k] F[k, j] over the split's k range; returns the split count
@@ -457,21 +441,16 @@ int stats_i8_linear(const StatsI8Buffers& w, bool trans, int K, const double* S,
                     int kdim_pad, int m_valid, int max_split, double* out, cudaStream_t st) {
     const int nchunks = kdim_pad / 32;
     const int m_tiles = (m_valid + 127) / 128;
-    // BTF_SF_RESIDENT=1: one CTA per SM with a small shared-memory footprint, dealt (tile, split) items round-robin,
-    // so that the linear block (HBM) and the int8 GEMM (tensor cores, L2) share every SM when they run on two streams
-    static const bool resident = getenv("BTF_SF_RESIDENT") != nullptr && getenv("BTF_SF_RESIDENT")[0] != '0';
     int sms = 148;
     { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); if (sms < 1) sms = 148; }
     // split-K partials are summed in split order by the recombination kernel
     int nsplit = 1;
-    // BTF_SF_WAVES=w: w times as many (smaller) items, for the block scheduler to balance when the GEMM holds part of the SMs
-    static const int waves = getenv("BTF_SF_WAVES") ? std::max(1, atoi(getenv("BTF_SF_WAVES"))) : 1;
-    const int target = resident ? 8 * sms : 2 * sms * waves;  // resident: 8 items per CTA; classic: one wave of two CTAs per SM
+    const int target = 2 * sms;      // one wave of two CTAs per SM
     if (m_tiles < target) {
         nsplit = target / m_tiles;       // never a partial last wave
         if (nsplit > nchunks / 8) nsplit = nchunks / 8 > 0 ? nchunks / 8 : 1;
         if (nsplit > max_split) nsplit = max_split;
-    } else if (max_split > 1 && !resident) {
+    } else if (max_split > 1) {
         // more tiles than CTA slots: the items run in ceil(items / slots) rounds, and a partial last round idles part of the
         // GPU (C2 columns: 512 tiles on 296 slots = 2 rounds for 1.73 rounds of work).  Splitting the contraction s ways
         // makes the rounds s times shorter: pick the s with the least rounds / s, 2 % per extra split for the partial sums.
@@ -484,34 +463,30 @@ int stats_i8_linear(const StatsI8Buffers& w, bool trans, int K, const double* S,
         }
     }
     { const int cps = (nchunks + nsplit - 1) / nsplit; nsplit = (nchunks + cps - 1) / cps; }
-    if (K <= 8) { if (trans) launch_sf_t<8, true>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, resident, sms, out, st); else launch_sf_t<8, false>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, resident, sms, out, st); }
-    else if (K <= 16) { if (trans) launch_sf_t<16, true>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, resident, sms, out, st); else launch_sf_t<16, false>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, resident, sms, out, st); }
-    else { if (trans) launch_sf_t<32, true>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, resident, sms, out, st); else launch_sf_t<32, false>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, resident, sms, out, st); }
+    if (K <= 8) { if (trans) launch_sf_t<8, true>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, out, st); else launch_sf_t<8, false>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, out, st); }
+    else if (K <= 16) { if (trans) launch_sf_t<16, true>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, out, st); else launch_sf_t<16, false>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, out, st); }
+    else { if (trans) launch_sf_t<32, true>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, out, st); else launch_sf_t<32, false>(S, lds, F, K, m_valid, m_tiles, nchunks, nsplit, out, st); }
     return nsplit;
 }
 
 // 4. recombination of the int32 planes (skipped when the fused epilogue already wrote them) and the sum of the
 //    linear-block partials: out[m][0..L) from D, out[m][L..L+K) from bpart[split][bpart_m0 + m][.] (row pitch of a
 //    split = bpart_rows)
-void stats_i8_combine(const StatsI8Buffers& w, int K, int m_valid, int m_pad, long long d_off, bool product_done,
+void stats_i8_combine(const StatsI8Buffers& w, int K, int m_valid, int m_pad, bool product_done,
                       const double* bpart, int nsplit_b, long long bpart_m0, long long bpart_rows, double* out,
                       const I8Guard* guard, cudaStream_t st) {
     const int L = K * (K + 1) / 2;
     const int ncy = (L + 31) / 32;
     const I8Guard g = guard ? *guard : I8Guard{nullptr, nullptr, nullptr, 0.0};
     if (product_done)
-        i8_combine_kernel<<<dim3((m_valid + 31) / 32, 1), 256, 0, st>>>(w.D + d_off, m_pad, w.expo, bpart, nsplit_b, m_valid, L, K, out, ncy,
+        i8_combine_kernel<<<dim3((m_valid + 31) / 32, 1), 256, 0, st>>>(w.D, m_pad, w.expo, bpart, nsplit_b, m_valid, L, K, out, ncy,
                                                                        bpart_m0, bpart_rows, g, guard != nullptr);
     else
-        i8_combine_kernel<<<dim3((m_valid + 31) / 32, ncy + 1), 256, 0, st>>>(w.D + d_off, m_pad, w.expo, bpart, nsplit_b, m_valid, L, K, out, 0,
+        i8_combine_kernel<<<dim3((m_valid + 31) / 32, ncy + 1), 256, 0, st>>>(w.D, m_pad, w.expo, bpart, nsplit_b, m_valid, L, K, out, 0,
                                                                              bpart_m0, bpart_rows, g, guard != nullptr);
 }
 
 // 5. FP64 recomputation of the rows flagged by the element-wise guard (see i8_fallback_kernel)
-double stats_i8_guard_tol() {
-    static const double tol = getenv("BTF_I8_GUARD_TOL") ? atof(getenv("BTF_I8_GUARD_TOL")) : 1e-12;
-    return tol;
-}
 void stats_i8_count_rows(const uint8_t* B, long long ldb, int m_valid, int kdim_pad, unsigned* cntsum, cudaStream_t st) {
     if (m_valid > 0) count_rows_kernel<<<(m_valid + 7) / 8, 256, 0, st>>>(B, ldb, m_valid, kdim_pad, cntsum);
 }
@@ -523,23 +498,6 @@ void stats_i8_fallback(int K, const uint8_t* B, long long ldb, const double* F, 
     const int grid = std::min((m_valid + 63) / 64, 592);
     if (L <= 256) i8_fallback_kernel<1><<<grid, 256, smem, st>>>(B, ldb, F, f_rows, K, L, m_valid, g.flags, g.nflag, out, nco);
     else i8_fallback_kernel<3><<<grid, 256, smem, st>>>(B, ldb, F, f_rows, K, L, m_valid, g.flags, g.nflag, out, nco);
-}
-
-// All four stages on one stream.
-// trans = false: m = local row, contraction over p (B = cnt [nloc][ldb = Ppad], F = V [P][K], S [nloc_pad][lds])
-// trans = true : m = p, contraction over local rows (B = cntT [P][ldb = nloc_pad], F = W local [nloc][K], S the same array)
-int launch_stats_i8(const StatsI8Buffers& w, bool trans, int K, const uint8_t* B, long long ldb, const double* S,
-                    long long lds, const double* F, int f_rows, int kdim_pad, int m_valid, int m_pad, double* out,
-                    cudaStream_t st) {
-    stats_i8_digits(w, K, F, f_rows, kdim_pad, st);
-    if (w.ev[0]) cudaEventRecord(w.ev[0], st);
-    const int pr = stats_i8_product(w, K, B, ldb, kdim_pad, m_valid, m_pad, 0, out, nullptr, st);
-    if (pr != 0 && pr != 10) return 1;
-    if (w.ev[1]) cudaEventRecord(w.ev[1], st);
-    const int nsplit = stats_i8_linear(w, trans, K, S, lds, F, kdim_pad, m_valid, trans ? 1 : w.nsplit_b_row, w.bpart, st);
-    if (w.ev[2]) cudaEventRecord(w.ev[2], st);
-    stats_i8_combine(w, K, m_valid, m_pad, 0, pr == 10, w.bpart, nsplit, 0, m_valid, out, nullptr, st);
-    return cudaGetLastError() == cudaSuccess ? 0 : 2;
 }
 
 }  // namespace btf

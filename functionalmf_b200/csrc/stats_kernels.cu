@@ -604,8 +604,6 @@ static void launch_stats_ovl_t(const StatsPlan& p, const void* wt, const double*
 #define BTF_CFG4 32, 1, 8, 10, 16
 #define BTF_CFG5 128, 8, 1, 6, 32
 #define BTF_CFG4U 32, 1, 8, 9, 16      // K == 32 with the unified tile list (overlapped kernel)
-#define BTF_CFG4H 64, 2, 4, 9, 32       // K == 32, two column parts per row tile (count weights)
-#define BTF_CFG3A 128, 8, 1, 19, 32    // K == 16 alternative: 8x1 warps, every warp owns all 19 tiles (no idle slot)
 
 static int cfg_wc(int cfg) { return (cfg == 1 || cfg == 4) ? 8 : (cfg == 3 ? 2 : 1); }
 
@@ -666,58 +664,33 @@ bool plan_stats(StatsPlan* p, int K, bool trans, bool weights_f64, int mdim_pad,
         default: p->smem_bytes = SMEM_OF(BTF_CFG5); break;
     }
 #undef SMEM_OF
-    // compile-time-K configurations: overlap Z generation with the DMMAs when the double
-    // buffers fit (BTF_STATS_NO_OVERLAP=1 keeps the three-phase kernel for A/B measurements)
+    // K = 32 with f64 weights: Z generation overlapped with the DMMAs (unified tile list, 185 KB).  K = 16 with f64
+    // weights keeps the three-phase kernel (its overlapped form would need 234 KB).
     p->overlap = 0;
-    static const bool no_ovl = getenv("BTF_STATS_NO_OVERLAP") != nullptr;
-    // (measured on B200: +6 % at K = 16, neutral at K = 32, slower at K = 8 where Z is tiny)
-    if ((p->cfg == 3 || p->cfg == 4) && !no_ovl) {
-#define SMEM_OVL(...) (trans ? (weights_f64 ? stats_smem_ovl<__VA_ARGS__, true, double>(K, p->zw)   \
-                                            : stats_smem_ovl<__VA_ARGS__, true, uint8_t>(K, p->zw)) \
-                             : (weights_f64 ? stats_smem_ovl<__VA_ARGS__, false, double>(K, p->zw)  \
-                                            : stats_smem_ovl<__VA_ARGS__, false, uint8_t>(K, p->zw)))
-        size_t so = p->cfg == 3 ? SMEM_OVL(BTF_CFG3) : (p->cfg == 4 ? SMEM_OVL(BTF_CFG4U) : SMEM_OVL(BTF_CFG5));
-#undef SMEM_OVL
-        if (so <= 220 * 1024) { p->overlap = 1; p->smem_bytes = so; }
-        static const bool no_halves = getenv("BTF_STATS_NO_HALVES") != nullptr;
-        if (p->cfg == 4 && !weights_f64 && !no_halves && mdim_pad % 64 == 0 && kdim_pad % 32 == 0) {
-            int zwh = 4 * 9 * 8;
-            while (!((zwh % 16) == 4 || (zwh % 16) == 12)) ++zwh;
-            size_t sh = trans ? stats_smem_ovl<BTF_CFG4H, true, uint8_t>(K, zwh) : stats_smem_ovl<BTF_CFG4H, false, uint8_t>(K, zwh);
-            if (sh <= 222 * 1024) {
-                p->overlap = 2; p->smem_bytes = sh; p->zw = zwh;
-                p->BM = 64; p->KC = 32;
-                p->mtiles = mdim_pad / p->BM;
-                p->nchunks = kdim_pad / p->KC;
-                int ns = nsplit_request;
-                if (ns <= 0) {
-                    ns = 1;
-                    double best = -1.0;
-                    int maxs = p->nchunks < 64 ? p->nchunks : 64;
-                    for (int s = 1; s <= maxs; ++s) {
-                        long long ctas = (long long)p->mtiles * s * 2;
-                        long long waves = (ctas + sm_count - 1) / sm_count;
-                        double eff = (double)ctas / (double)(waves * sm_count);
-                        if (eff > best + 0.03) { best = eff; ns = s; }
-                        if (best > 0.97) break;
-                    }
-                }
-                if (ns > p->nchunks) ns = p->nchunks;
-                if (ns < 1) ns = 1;
-                p->chunks_per_split = (p->nchunks + ns - 1) / ns;
-                p->nsplit = (p->nchunks + p->chunks_per_split - 1) / p->chunks_per_split;
-            }
-        }
+    if (p->cfg == 4 && weights_f64) {
+        p->overlap = 1;
+        p->smem_bytes = trans ? stats_smem_ovl<BTF_CFG4U, true, double>(K, p->zw) : stats_smem_ovl<BTF_CFG4U, false, double>(K, p->zw);
     }
     p->zpre = 0; p->zwg = 0;
-    if (plan_stats_zpre(p, trans, weights_f64, mdim_pad, kdim_pad, nsplit_request, sm_count)) return true;
+    // count weights at K = 16 / 32: the right operand is pre-generated in global memory (stats_zpre.cu)
+    if (!weights_f64 && (K == 16 || K == 32)) return plan_stats_zpre(p, trans, mdim_pad, kdim_pad, nsplit_request, sm_count);
     return p->smem_bytes <= 226 * 1024;
 }
 
 void launch_stats(const StatsPlan& p, bool trans, bool weights_f64, const void* wt, const double* sv,
                   const double* F, long long frows, long long ld, int m_valid, double* out, double* zscratch,
                   cudaStream_t st) {
-    if (p.zpre && zscratch) { launch_stats_zpre(p, trans, wt, sv, F, frows, ld, m_valid, out, zscratch, st); return; }
+    if (p.zpre) { launch_stats_zpre(p, trans, wt, sv, F, frows, ld, m_valid, out, zscratch, st); return; }
+    if (p.overlap) {
+        if (trans) launch_stats_ovl_t<BTF_CFG4U, true, double, 32, true, 1>(p, wt, sv, F, ld, m_valid, out, st);
+        else launch_stats_ovl_t<BTF_CFG4U, false, double, 32, true, 1>(p, wt, sv, F, ld, m_valid, out, st);
+        return;
+    }
+    if (p.cfg == 3) {   // K = 16 with count weights takes the zpre kernel
+        if (trans) launch_stats_t<BTF_CFG3, true, double, 16>(p, wt, sv, F, ld, m_valid, out, st);
+        else launch_stats_t<BTF_CFG3, false, double, 16>(p, wt, sv, F, ld, m_valid, out, st);
+        return;
+    }
 #define DISPATCH(KF, ...)                                                                                        \
     do {                                                                                                         \
         if (trans) {                                                                                             \
@@ -728,41 +701,11 @@ void launch_stats(const StatsPlan& p, bool trans, bool weights_f64, const void* 
             else launch_stats_t<__VA_ARGS__, false, uint8_t, KF>(p, wt, sv, F, ld, m_valid, out, st);            \
         }                                                                                                        \
     } while (0)
-#define DISPATCH_OVL(KF, UNI_, ...)                                                                                           \
-    do {                                                                                                                      \
-        if (trans) {                                                                                                          \
-            if (weights_f64) launch_stats_ovl_t<__VA_ARGS__, true, double, KF, UNI_, 1>(p, wt, sv, F, ld, m_valid, out, st);  \
-            else launch_stats_ovl_t<__VA_ARGS__, true, uint8_t, KF, UNI_, 1>(p, wt, sv, F, ld, m_valid, out, st);             \
-        } else {                                                                                                              \
-            if (weights_f64) launch_stats_ovl_t<__VA_ARGS__, false, double, KF, UNI_, 1>(p, wt, sv, F, ld, m_valid, out, st); \
-            else launch_stats_ovl_t<__VA_ARGS__, false, uint8_t, KF, UNI_, 1>(p, wt, sv, F, ld, m_valid, out, st);            \
-        }                                                                                                                     \
-    } while (0)
-    if (p.overlap == 2) {
-        // K = 32, count weights: two column parts per row tile (64 rows, KC 32)
-        if (trans) launch_stats_ovl_t<BTF_CFG4H, true, uint8_t, 32, true, 2>(p, wt, sv, F, ld, m_valid, out, st);
-        else launch_stats_ovl_t<BTF_CFG4H, false, uint8_t, 32, true, 2>(p, wt, sv, F, ld, m_valid, out, st);
-        return;
-    }
-    if (p.overlap) {
-        // K = 16: measured on B200 (C2): rows 2.85 ms with the 8x1 layout vs 2.92 ms with 4x2,
-        // columns 2.94 ms vs 2.89 ms -> 8x1 for the row contraction, 4x2 for the column contraction
-        static const bool k16_alt = getenv("BTF_STATS_K16_ALT") != nullptr;
-        if (p.cfg == 3 && (k16_alt || !trans)) { DISPATCH_OVL(16, false, BTF_CFG3A); return; }
-        switch (p.cfg) {
-            case 3: DISPATCH_OVL(16, false, BTF_CFG3); return;
-            case 4: DISPATCH_OVL(32, true, BTF_CFG4U); return;
-            default: DISPATCH_OVL(8, false, BTF_CFG5); return;
-        }
-    }
-#undef DISPATCH_OVL
     switch (p.cfg) {
         case 0: DISPATCH(0, BTF_CFG0); break;
         case 1: DISPATCH(0, BTF_CFG1); break;
         case 2: DISPATCH(0, BTF_CFG2); break;
-        case 3: DISPATCH(16, BTF_CFG3); break;
-        case 4: DISPATCH(32, BTF_CFG4); break;
-        default: DISPATCH(8, BTF_CFG5); break;
+        default: DISPATCH(8, BTF_CFG5); break;   // cfg 5 (cfg 4 is always overlapped or zpre)
     }
 #undef DISPATCH
 }

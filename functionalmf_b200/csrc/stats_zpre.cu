@@ -217,11 +217,9 @@ static int zpre_pitch(int ntiles) {
     return zw;
 }
 
-// Fill in the plan for the pre-generated-operand path; false when the shape has no such kernel.
-bool plan_stats_zpre(StatsPlan* p, bool trans, bool weights_f64, int mdim_pad, int kdim_pad, int nsplit_request,
-                     int sm_count) {
-    static const bool off = getenv("BTF_STATS_NO_ZPRE") != nullptr;
-    if (off || weights_f64 || (p->K != 16 && p->K != 32)) return false;
+// Fill in the plan for the pre-generated-operand path (count weights, K = 16 or 32); false when the shape has no such kernel.
+bool plan_stats_zpre(StatsPlan* p, bool trans, int mdim_pad, int kdim_pad, int nsplit_request, int sm_count) {
+    if (p->K != 16 && p->K != 32) return false;
     const int nct = p->nct_z + p->nct_f;
     int parts = 1;
     size_t smem;

@@ -225,7 +225,7 @@ class Engine(object):
             'W_Q': (N, K, K), 'W_L': (N, K, K), 'W_mean': (N, K), 'W_b': (N, K), 'V_mean': (M, T, K),
             'V_band': (self.Mloc, T * K, kd + 1), 'V_chol': (self.Mloc, T * K, kd + 1),
             'V_retries': (self.Mloc,), 'row_stats': (self.nloc, Lp + K), 'col_stats': (M * T, Lp + K),
-            'nu2_rate': (3,), 'lam2_rate': (2,), 'info': (3,), 'i8_guard': (2,),
+            'nu2_rate': (3,), 'lam2_rate': (2,), 'info': (3,), 'i8_guard': (2,), 'i8_route': (2,),
         }
         a = np.empty(shapes[name], dtype=np.float64)
         L.check(self.lib.btf_get_diag(self._h, name.encode(), _ptr(a), a.size))

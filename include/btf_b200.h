@@ -162,7 +162,10 @@ int btf_inject_noise(btf_engine* e, const char* name, const double* host, size_t
  * "W_Q","W_L" [N,K,K], "W_mean" [N,K], "W_b" [N,K], "V_mean" [M,T,K],
  * "V_band","V_chol" [Mloc,T*K,(p+1)K+1] (column j of the band / factor in row j),
  * "V_retries" [Mloc], "row_stats" [Nloc,L+K], "col_stats" [M*T,L+K],
- * "nu2_rate" [3] = (a_post,b_post,n_obs), "lam2_rate" [2]. */
+ * "nu2_rate" [3] = (a_post,b_post,n_obs), "lam2_rate" [2],
+ * "i8_route" [2] = route of the last row / column product block of the integer
+ * statistics path: 0 none yet, 1 round-1 kernel, 2 2-CTA kernel with the fused
+ * epilogue, 3 2-CTA kernel in split-K mode (recorded without btf_enable_diag). */
 int btf_enable_diag(btf_engine* e, int32_t on);
 int btf_get_diag(btf_engine* e, const char* name, double* host, size_t n);
 

@@ -37,17 +37,28 @@ def test_i8gemm_exact(shape):
     np.testing.assert_array_equal(_gemm(A, B), np.full((M, N), -64 * 127 * K, dtype=np.int32))
 
 
-GEMM_MODES = ('BTF_STATS_I8_FUSED', 'BTF_STATS_I8_NOFUSED')   # recombination in the GEMM epilogue / through the int32 planes
+# BTF_I8_GEMM2: '1' = the 2-CTA kernel with the recombination in its epilogue at every shape, '0' = the round-1 kernel
+# through the int32 planes; the engine reads it when it is created
+GEMM_MODES = ('1', '0')
+
+
+def _want_route(gemm_mode):
+    from functionalmf_b200 import _lib as L
+    return {'1': L.I8_ROUTE_FUSED, '0': L.I8_ROUTE_ROUND1}[gemm_mode]
 
 
 def _engine(N, M, T, R, K, env, gemm_mode=None):
     from functionalmf_b200.engine import Engine
-    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8') + GEMM_MODES:
+    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8', 'BTF_I8_GEMM2'):
         os.environ.pop(k, None)
     os.environ[env] = '1'
     if gemm_mode:
-        os.environ[gemm_mode] = '1'
-    return Engine(N, M, T, nembeds=K, tf_order=2, seed=5, use_graph=0)
+        os.environ['BTF_I8_GEMM2'] = gemm_mode
+    try:
+        return Engine(N, M, T, nembeds=K, tf_order=2, seed=5, use_graph=0)
+    finally:
+        for k in (env, 'BTF_I8_GEMM2'):
+            os.environ.pop(k, None)
 
 
 def _problem(N, M, T, R, K, seed):
@@ -71,7 +82,7 @@ def _load(eng, rs, W, V):
         eng.set(k, [v])
 
 
-@pytest.mark.parametrize('gemm_mode', GEMM_MODES)
+@pytest.mark.parametrize('gemm_mode', GEMM_MODES, ids=('two_cta_fused', 'round1'))
 @pytest.mark.parametrize('shape', [(150, 9, 21, 3, 8), (300, 7, 40, 2, 16), (129, 5, 33, 4, 32)])
 def test_product_block_is_the_exact_fixed_point_sum(shape, gemm_mode):
     N, M, T, R, K = shape
@@ -86,6 +97,7 @@ def test_product_block_is_the_exact_fixed_point_sum(shape, gemm_mode):
         z = np.zeros(N * K)
         eng.inject('z_W', z)                  # W stays at its conditional mean: the V statistics use a known W
         eng.sweep(1)
+        assert list(eng.diag('i8_route')) == [_want_route(gemm_mode)] * 2
         L = K * (K + 1) // 2
         cnt = (~np.isnan(Y)).sum(axis=-1).reshape(N, M * T)
         Ssum = np.nansum(Y, axis=-1).reshape(N, M * T)
@@ -105,11 +117,9 @@ def test_product_block_is_the_exact_fixed_point_sum(shape, gemm_mode):
         np.testing.assert_allclose(cols[:, L:], Ssum.T @ Wn, rtol=1e-12, atol=1e-12 * np.abs(Ssum.T @ Wn).max())
     finally:
         eng.close()
-        for k in ('BTF_STATS_FORCE_I8',) + GEMM_MODES:
-            os.environ.pop(k, None)
 
 
-@pytest.mark.parametrize('gemm_mode', GEMM_MODES)
+@pytest.mark.parametrize('gemm_mode', GEMM_MODES, ids=('two_cta_fused', 'round1'))
 @pytest.mark.parametrize('shape', [(260, 12, 24, 3, 16), (140, 6, 30, 2, 8), (200, 5, 20, 3, 32)])
 def test_sweep_matches_the_fp64_path(shape, gemm_mode):
     N, M, T, R, K = shape
@@ -122,12 +132,12 @@ def test_sweep_matches_the_fp64_path(shape, gemm_mode):
             _load(eng, rs, W, V)
             eng.enable_diag(True)
             eng.sweep(2)
+            if env == 'BTF_STATS_FORCE_I8':
+                assert list(eng.diag('i8_route')) == [_want_route(gemm_mode)] * 2
             res[env] = dict(W=eng.get('W'), V=eng.get('V'), Tau2=eng.get('Tau2'), nu2=eng.get_scalar('nu2'),
                             sigma2=eng.get_scalar('sigma2'), rows=eng.diag('row_stats'), cols=eng.diag('col_stats'))
         finally:
             eng.close()
-            for k in (env,) + GEMM_MODES:
-                os.environ.pop(k, None)
     a, b = res['BTF_STATS_FORCE_I8'], res['BTF_STATS_NO_I8']
     for k in ('rows', 'cols'):
         np.testing.assert_allclose(a[k], b[k], rtol=0, atol=1e-11 * np.abs(b[k]).max())
@@ -152,13 +162,13 @@ def test_two_cta_gemm_split_k_and_fused_modes_are_exact():
         eng.set_sample_mask(L.SAMPLE_W | L.SAMPLE_V)
         eng.inject('z_W', np.zeros(N * K))
         eng.sweep(1)
+        assert list(eng.diag('i8_route')) == [L.I8_ROUTE_SPLITK, L.I8_ROUTE_FUSED]
         Lp = K * (K + 1) // 2
         cnt = (~np.isnan(Y)).sum(axis=-1).reshape(N, M * T)
         np.testing.assert_array_equal(eng.diag('row_stats')[:, :Lp], product_block_fast((V * 1.1).reshape(M * T, K), cnt))
         np.testing.assert_array_equal(eng.diag('col_stats')[:, :Lp], product_block_fast(eng.get('W'), cnt.T))
     finally:
         eng.close()
-        os.environ.pop('BTF_STATS_FORCE_I8', None)
 
 
 def _exact_product_block(F, cnt):
@@ -182,7 +192,7 @@ def _guard_case(no_guard):
     Y[rs.random_sample(Y.shape) < 0.2] = np.nan
     Y[200:, :4] = np.nan                  # rows 200.. see only the small columns
     Y[:128, 6:] = np.nan                  # columns 6.. see only the small rows
-    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8', 'BTF_I8_NO_GUARD') + GEMM_MODES:
+    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8', 'BTF_I8_NO_GUARD', 'BTF_I8_GEMM2'):
         os.environ.pop(k, None)
     os.environ['BTF_STATS_FORCE_I8'] = '1'
     if no_guard:

@@ -3,7 +3,7 @@
 launch_nb_update (pg_kernels.cu) runs the random-walk Metropolis chain of R in one of two ways:
   * histogram route (nb_mh_hist_kernel): integer counts with (max count + 1) * groups <= 2^24; the sum of
     lgamma(y + r) over a group is taken from a per-group count histogram, the whole chain in one block;
-  * direct route (nb_mh_kernel + nb_lgamma_kernel): any other data, or BTF_NB_NO_HIST set when the data are set;
+  * direct route (nb_mh_kernel + nb_lgamma_kernel): any other data, or BTF_NB_NO_HIST set when the engine is created;
     per step a pass over the data with warp-aggregated atomics.
 The proposal normals and acceptance uniforms are injected, so device and oracle make the same decisions.  The
 oracle also reports how close its nearest decision came to a tie (|u - prob| / prob); noise with a margin below
