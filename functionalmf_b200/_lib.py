@@ -15,7 +15,7 @@ BTF_OK, BTF_EINVAL, BTF_ECUDA, BTF_ENOTPD, BTF_ESTATE, BTF_ENCCL = 0, -1, -2, -3
 GAUSSIAN, BINOMIAL, NEGBINOMIAL = 0, 1, 2
 SAMPLE_NU2, SAMPLE_SIGMA2, SAMPLE_TAU2, SAMPLE_LAM2, SAMPLE_W, SAMPLE_V, SAMPLE_R = 1, 2, 4, 8, 16, 32, 64
 SAMPLE_ALL = 127
-I8_ROUTE_ROUND1, I8_ROUTE_FUSED, I8_ROUTE_SPLITK = 1, 2, 3     # btf_get_diag("i8_route")
+I8_ROUTE_FUSED, I8_ROUTE_SPLITK = 2, 3     # btf_get_diag("i8_route")
 INIT_SIGMA2, INIT_LAM2, INIT_NU2, INIT_TAU2, INIT_W, INIT_V, INIT_R = 1, 2, 4, 8, 16, 32, 64
 PHASES = ['nu2_or_pg', 'sigma2', 'tau2', 'lam2', 'row_stats', 'row_solve', 'col_stats', 'band_solve', 'comm',
           # sub-phases of row_stats / col_stats on the integer-tensor-core path (0 when it is off)
@@ -99,7 +99,6 @@ SIGNATURES = {
     'btf_i8_peak': (C.c_double, [C.c_int32, C.c_int32]),
     'btf_pg_sample': (C.c_int, [C.c_int32, _P, _P, _P, C.c_int64, C.c_uint64]),
     'btf_rng_sample': (C.c_int, [C.c_int32, C.c_int32, C.c_double, _P, C.c_int64, C.c_uint64]),
-    'btf_i8gemm_test': (C.c_double, [C.c_int32, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     'btf_nccl_unique_id': (C.c_int, [C.c_char_p]),
     'btf_nccl_init': (C.c_int, [_P, C.c_char_p]),
 }

@@ -42,7 +42,6 @@ struct DevBuf {
 // Environment switches (INTEGRATION.md §1), read once per engine by read_env(); the kernel files get the values as arguments.
 struct EnvSwitches {
     bool no_i8 = false, force_i8 = false;   // BTF_STATS_NO_I8, BTF_STATS_FORCE_I8
-    int i8_gemm2 = -1;                      // BTF_I8_GEMM2: 0 never / 1 always the 2-CTA product-block kernel, -1 by tile count
     bool i8_guard = true;                   // BTF_I8_NO_GUARD
     double i8_guard_tol = 1e-12;            // BTF_I8_GUARD_TOL
     bool scol = true;                       // BTF_NO_SCOL
@@ -236,7 +235,6 @@ static EnvSwitches read_env() {
     EnvSwitches s;
     s.no_i8 = on("BTF_STATS_NO_I8");
     s.force_i8 = on("BTF_STATS_FORCE_I8");
-    if (const char* g = getenv("BTF_I8_GEMM2")) s.i8_gemm2 = g[0] == '0' ? 0 : 1;
     s.i8_guard = !on("BTF_I8_NO_GUARD");
     if (const char* t = getenv("BTF_I8_GUARD_TOL")) s.i8_guard_tol = atof(t);
     s.scol = !on("BTF_NO_SCOL");
@@ -911,7 +909,7 @@ static int begin_row_stats_i8(btf_engine* e, bool fork, int timer, I8Pending* pd
     if (ev) cudaEventRecord(ev[0], sa);
     const I8Guard gr{e->cnt_rowsum, e->guard_flags, e->guard_n, e->env.i8_guard_tol};
     pd->product = stats_i8_product(e->i8, e->K, e->cnt, e->Ppad, e->Ppad, e->nloc, e->nloc_pad, e->row_stats,
-                                   e->env.i8_guard ? &gr : nullptr, e->env.i8_gemm2, sa);
+                                   e->env.i8_guard ? &gr : nullptr, sa);
     if (!pd->product) return set_err(BTF_ECUDA, "integer row statistics failed to launch");
     e->i8_route[0] = pd->product;
     if (ev) cudaEventRecord(ev[1], sa);
@@ -947,7 +945,6 @@ static int col_step_i8(btf_engine* e, bool fork, int timer, BandFn band) {
     const int ldd = round_up(std::max(np, 1), 256);
     const double* Wloc = e->W + (size_t)e->cfg.row_begin * e->K;
     fork_side(e, fork);
-    if (ev) cudaEventRecord(ev[0], sa);
     if (np > 0) { stats_i8_digits(e->i8, e->K, e->W, e->N, e->Nall_pad, sa); e->launches += 2; }
     if (ev) cudaEventRecord(ev[0], sa);
     // linear block: sharded engines need the partial sums of ALL columns before the exchange -> one launch
@@ -980,7 +977,7 @@ static int col_step_i8(btf_engine* e, bool fork, int timer, BandFn band) {
     const I8Guard gc{e->cnt_colsum, e->guard_flags + std::max(e->nloc, 1), e->guard_n + 1, e->env.i8_guard_tol};
     const I8Guard* gp = e->env.i8_guard ? &gc : nullptr;
     if (np > 0) {
-        product = stats_i8_product(e->i8, e->K, e->cntT, e->Nall_pad, e->Nall_pad, np, ldd, out, gp, e->env.i8_gemm2, sa);
+        product = stats_i8_product(e->i8, e->K, e->cntT, e->Nall_pad, e->Nall_pad, np, ldd, out, gp, sa);
         if (!product) return set_err(BTF_ECUDA, "integer column statistics failed to launch");
         e->i8_route[1] = product;
         e->launches++;
@@ -1004,7 +1001,7 @@ static int col_step_i8(btf_engine* e, bool fork, int timer, BandFn band) {
 }
 
 // The integer-tensor-core statistics path: Gaussian data (count weights), K in {8, 16, 32}, accumulators
-// that cannot overflow, and a tensor large enough for the digit planes to pay (BTF_STATS_FORCE_I8=1
+// that cannot overflow, a device that runs the 2-CTA GEMM, and a tensor large enough for the digit planes to pay (BTF_STATS_FORCE_I8=1
 // forces it for any size, BTF_STATS_NO_I8=1 disables it).  The decision only uses global quantities, so
 // every rank of a sharded engine takes the same path (the two paths exchange different things).
 static int ensure_i8(btf_engine* e) {

@@ -6,7 +6,8 @@
 // (int8, K-major, stored tile-major: plane row (c / 36) * 252 + s * 36 + (c % 36), see stats_i8.cu).  Exact integer
 // contraction, recombined and rounded ONCE in the epilogue: no int32 intermediate in global memory.
 //
-// Shape of the kernel (what the round-1 kernel lacked - it was bound by operand traffic from L2 at 87 MAC/B):
+// Shape of the kernel (what the earlier single-CTA 128 x 256 kernel lacked - it was bound by operand traffic from L2 at
+// 87 MAC/B):
 //   * one CTA PAIR (cluster of 2, tcgen05 cta_group::2) owns a 256 x 256 tile: each CTA stages 128 count rows and 128
 //     digit rows per 128-byte K chunk (32 KB per stage, 6 stages) for 256 x 256 x 128 MACs of the pair
 //     = 128 MAC per byte read from L2, 1.5x the single-CTA 128 x 256 tile;
@@ -334,55 +335,55 @@ bool make_map(CUtensorMap* tm, const void* base, long long rows, long long ld, l
 
 }  // namespace
 
-// out[m][c] (c < L) for counts [M][ldc] and tile-major digit planes [n_tiles * 252][ldp], contraction length K (multiple
-// of 128).  Returns 0 on success, 1 when this kernel does not apply (too few tiles to fill the pairs, alignment, no TMA
-// entry point: the caller takes the split-K route through the int32 planes), > 1 on a launch error.
-// D / ldd (optional): int32 planes [i8_plane_rows(L)][ldd] for the split-K mode.  Returns 0: `out` written (fused epilogue);
-// 5: split-K, the exact partial sums are in D (the caller recombines); 1: not applicable; > 1 and != 5: launch error.
-int launch_i8gemm2(const int8_t* Cn, long long ldc, int M, const int8_t* Pl, long long ldp, int L, int K, const int* expo,
-                   double* out, long long ldo, int min_tiles, const I8Guard* guard, int32_t* D, long long ldd, cudaStream_t st) {
-    if (K % G2_BK != 0 || (ldc % 16) || (ldp % 16) || M < 1 || L < 1) return 1;
-    if ((reinterpret_cast<uintptr_t>(Cn) & 15) || (reinterpret_cast<uintptr_t>(Pl) & 15)) return 1;
-    const int mt = (M + 255) / 256, nt = (L + G2_CPT - 1) / G2_CPT;
-    int nsplit = 1;
-    if (mt * nt < min_tiles) {
-        // few tiles: split the contraction so that the jobs fill the CTA pairs (at least 8 chunks per job)
-        if (!D || min_tiles >= (1 << 29)) return 1;
-        const int kc = K / G2_BK;
-        int dev = 0, nsm = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-        nsplit = std::min(std::max(1, kc / 8), (nsm / 2) / (mt * nt));       // one wave of jobs on the CTA pairs
-        if (nsplit < 2) return 1;
-    }
-    int sms = 148;
-    { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); }
-    static PerDeviceOnce attr_once;
-    if (attr_once.first() &&
-        cudaFuncSetAttribute(i8gemm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, G2_SMEM) != cudaSuccess) {
+// The 2-CTA kernel runs on the current device: the driver exports the TMA descriptor encoder, and the kernel may use its
+// shared memory (the attribute is set here, before the first launch or graph capture on this device).
+bool i8gemm2_ready() {
+    if (!encode_fn()) return false;
+    if (cudaFuncSetAttribute(i8gemm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, G2_SMEM) != cudaSuccess) {
         cudaGetLastError();
-        return 1;
+        return false;
     }
-    if (nt > 16) return 1;
+    return true;
+}
+
+// out[m][c] (c < L) for counts [M][ldc] and tile-major digit planes [n_tiles * 252][ldp], contraction length K.
+// Fused route: the epilogue recombines the planes, writes `out` and applies the guard.  Split-K route, when the 256 x 256
+// tiles are too few to fill the CTA pairs (< 48) and the contraction is long enough to split: the exact int32 partial sums
+// go to the planes D [i8_plane_rows(L)][ldd], and stats_i8_combine recombines them (and applies the guard).
+// Needs i8gemm2_ready() on this device, K a multiple of 128, ldc and ldp multiples of 16, 16-byte aligned operands and at
+// most 16 column tiles (K <= 32): the engine's buffers always satisfy them.  Returns the I8Route taken, 0 when one of
+// these conditions fails or the launch does.
+int launch_i8gemm2(const int8_t* Cn, long long ldc, int M, const int8_t* Pl, long long ldp, int L, int K, const int* expo,
+                   double* out, long long ldo, const I8Guard* guard, int32_t* D, long long ldd, cudaStream_t st) {
+    const int mt = (M + 255) / 256, nt = (L + G2_CPT - 1) / G2_CPT;
+    if (K % G2_BK != 0 || (ldc % 16) || (ldp % 16) || M < 1 || L < 1 || nt > 16) return 0;
+    if ((reinterpret_cast<uintptr_t>(Cn) & 15) || (reinterpret_cast<uintptr_t>(Pl) & 15)) return 0;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // few tiles (narrow shards, small tensors): split the contraction so that one wave of jobs fills the CTA pairs, with
+    // at least 8 chunks per job
+    const int kc = K / G2_BK;
+    const int nsplit = mt * nt < 48 ? std::max(1, std::min(kc / 8, (sms / 2) / (mt * nt))) : 1;
     // the descriptors travel as kernel parameters (a CUDA graph keeps its own copy of them)
     alignas(64) CUtensorMap tm_cnt, tm_dig;
-    if (!make_map(&tm_cnt, Cn, M, ldc, K) || !make_map(&tm_dig, Pl, (long long)nt * G2_CPT * G2_NP, ldp, K)) return 1;
+    if (!make_map(&tm_cnt, Cn, M, ldc, K) || !make_map(&tm_dig, Pl, (long long)nt * G2_CPT * G2_NP, ldp, K)) return 0;
     G2Args p{};
-    p.M = M; p.L = L; p.k_chunks = K / G2_BK; p.m_tiles = mt; p.n_tiles = nt; p.expo = expo; p.out = out; p.ldo = ldo;
-    p.chunks_per_split = (p.k_chunks + nsplit - 1) / nsplit;
-    p.nsplit = (p.k_chunks + p.chunks_per_split - 1) / p.chunks_per_split;
+    p.M = M; p.L = L; p.k_chunks = kc; p.m_tiles = mt; p.n_tiles = nt; p.expo = expo; p.out = out; p.ldo = ldo;
+    p.chunks_per_split = (kc + nsplit - 1) / nsplit;
+    p.nsplit = (kc + p.chunks_per_split - 1) / p.chunks_per_split;
     p.D = D; p.ldd = ldd;
     if (p.nsplit > 1 &&
         cudaMemset2DAsync(D, (size_t)ldd * sizeof(int32_t), 0, (size_t)M * sizeof(int32_t), (size_t)nt * G2_CPT * G2_NP, st) != cudaSuccess)
-        return 2;
+        return 0;
     if (guard && p.nsplit == 1) {
         p.cntsum = guard->cntsum; p.flags = guard->flags; p.tol = guard->tol;
         for (int k = 0; k * (k + 3) / 2 < L; ++k) { const int c = k * (k + 3) / 2; p.diag_mask[c / G2_CPT] |= 1ull << (c % G2_CPT); }
     }
     const int pairs = std::min(sms / 2, mt * nt * p.nsplit);
     i8gemm2_kernel<<<2 * pairs, G2_THREADS, G2_SMEM, st>>>(tm_cnt, tm_dig, p);
-    if (cudaGetLastError() != cudaSuccess) return 2;
-    return p.nsplit > 1 ? 5 : 0;
+    if (cudaGetLastError() != cudaSuccess) return 0;
+    return p.nsplit > 1 ? I8_ROUTE_SPLITK : I8_ROUTE_FUSED;
 }
 
 }  // namespace btf

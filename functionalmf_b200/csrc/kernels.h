@@ -66,7 +66,7 @@ bool plan_stats_zpre(StatsPlan* p, bool trans, int mdim_pad, int kdim_pad, int n
 void launch_stats_zpre(const StatsPlan& p, bool trans, const void* wt, const double* sv, const double* F,
                        long long frows, long long ld, int m_valid, double* out, double* Zg, cudaStream_t st);
 
-// ---------------------------------------------------------------- K1 on the integer tensor cores (stats_i8.cu, i8gemm.cu, i8gemm2.cu)
+// ---------------------------------------------------------------- K1 on the integer tensor cores (stats_i8.cu, i8gemm2.cu)
 // Fixed-point form of a column of Z: q = rint(Z 2^(54 - e_c)), |q| <= 2^54, in 7 signed base-256 digits d_s in [-128, 127].
 // The digit planes are stored tile-major for the 2-CTA GEMM: a tile = 36 product columns x 7 planes = 252 rows, plane-major.
 constexpr int I8_NPLANES = 7, I8_FIXBITS = 54, I8_COLS_PER_TILE = 36;
@@ -83,6 +83,8 @@ struct StatsI8Buffers {
     double* bpart;                  // [nsplit][m][K] partial sums of the linear block
     int nsplit_b_row;
 };
+// K in {8, 16, 32}, int32 accumulators that cannot overflow, and the 2-CTA GEMM can run on the current device (its
+// shared-memory attribute is set there)
 bool stats_i8_supported(int K, int nreps, long long kdim_row, long long kdim_col);
 // nall_pad: padded GLOBAL row count (contraction length of the column side), ploc: columns (j,t) owned by this rank
 void stats_i8_sizes(int K, int nloc_pad, int Ppad, int nloc, int P, int nall_pad, int ploc, StatsI8Sizes* s);
@@ -96,13 +98,12 @@ struct I8Guard {
 };
 // the four stages of the integer path (engine: tensor-core contraction and HBM-bound linear block on separate streams)
 void stats_i8_digits(const StatsI8Buffers& w, int K, const double* F, int f_rows, int kdim_pad, cudaStream_t st);
-// route of the product block: round-1 kernel / 2-CTA kernel in split-K mode (both leave int32 planes in w.D for
-// stats_i8_combine), or the 2-CTA kernel whose fused epilogue wrote `out`
-enum I8Route { I8_ROUTE_ROUND1 = 1, I8_ROUTE_FUSED = 2, I8_ROUTE_SPLITK = 3 };
-// gemm2 (BTF_I8_GEMM2): 0 never the 2-CTA kernel, 1 always, -1 when its 256 x 256 tiles fill most CTA pairs;
-// returns the I8Route taken, 0 when a launch failed
+// route of the product block on the 2-CTA GEMM: its fused epilogue wrote `out` (>= 48 tiles of 256 x 256, or a contraction
+// too short to split), or split-K left int32 planes in w.D for stats_i8_combine
+enum I8Route { I8_ROUTE_FUSED = 2, I8_ROUTE_SPLITK = 3 };
+// returns the I8Route taken, 0 when the launch failed
 int stats_i8_product(const StatsI8Buffers& w, int K, const uint8_t* B, long long ldb, int kdim_pad, int m_valid, int m_pad,
-                     double* out, const I8Guard* guard, int gemm2, cudaStream_t st);
+                     double* out, const I8Guard* guard, cudaStream_t st);
 int stats_i8_linear(const StatsI8Buffers& w, bool trans, int K, const double* S, long long lds, const double* F,
                     int kdim_pad, int m_valid, int max_split, double* out, cudaStream_t st);     // returns the split count of `out`
 void stats_i8_combine(const StatsI8Buffers& w, int K, int m_valid, int m_pad, bool product_done,

@@ -6,8 +6,8 @@
 // column of Z is written as a fixed-point number against a power-of-two column scale,
 //   Z[k, c] ~ 2^(e_c - 54) q[k, c],   q = round(Z 2^(54 - e_c)),  |q| <= 2^54,   q = sum_{s<7} 256^s d_s,  d_s in [-128, 127],
 // and the seven digit planes are contracted with the counts by ONE exact int8 x int8 -> int32 GEMM on the
-// tcgen05 tensor cores (i8gemm2.cu: 2-CTA pairs, TMA, recombination in the epilogue; i8gemm.cu: split-K route for
-// shapes with few tiles):  D[(s, c), m] = sum_k d_s[k, c] cnt[m, k].  The planes are recombined in integer arithmetic
+// tcgen05 tensor cores (i8gemm2.cu: 2-CTA pairs, TMA, recombination in the epilogue, or split-K through int32 planes
+// for shapes with few tiles):  D[(s, c), m] = sum_k d_s[k, c] cnt[m, k].  The planes are recombined in integer arithmetic
 // (two int64 Horner sums re-split into parts that are exactly representable in a double) and rounded once.  The only error is the 2^-55 (relative to the column maximum) rounding of Z
 // itself - below the rounding noise of an FP64 accumulation over the same number of terms - and the result
 // does not depend on the order of summation at all.
@@ -21,11 +21,9 @@
 
 namespace btf {
 
-int launch_i8gemm(const int8_t* A, long long lda, int M, const int8_t* B, long long ldb, int N, int K, int32_t* D,
-                  long long ldd, cudaStream_t st);
+bool i8gemm2_ready();
 int launch_i8gemm2(const int8_t* Cn, long long ldc, int M, const int8_t* Pl, long long ldp, int L, int K, const int* expo,
-                   double* out, long long ldo, int min_tiles, const I8Guard* guard, int32_t* D, long long ldd,
-                   cudaStream_t st);
+                   double* out, long long ldo, const I8Guard* guard, int32_t* D, long long ldd, cudaStream_t st);
 
 namespace {
 
@@ -384,7 +382,8 @@ bool stats_i8_supported(int K, int nreps, long long kdim_row, long long kdim_col
     if (!(K == 8 || K == 16 || K == 32)) return false;
     if (nreps < 1 || nreps > 127) return false;
     const long long kd = kdim_row > kdim_col ? kdim_row : kdim_col;
-    return kd * nreps * 128 < (1ll << 31);          // the int32 accumulators cannot overflow
+    if (kd * nreps * 128 >= (1ll << 31)) return false;      // the int32 accumulators cannot overflow
+    return i8gemm2_ready();
 }
 
 void stats_i8_sizes(int K, int nloc_pad, int Ppad, int nloc, int P, int nall_pad, int ploc, StatsI8Sizes* s) {
@@ -420,20 +419,13 @@ void stats_i8_digits(const StatsI8Buffers& w, int K, const double* F, int f_rows
     zdigits_kernel<<<dim3(nbx, nby), 256, zs, st>>>(F, f_rows, kdim_pad, K, L, w.colmax, w.expo, w.planes, (long long)kdim_pad);
 }
 
-// 2. exact product block on the tensor cores: D[(8 c + s)][m] = sum_k d_s[k, c] B[m][k], m < m_valid (B = counts, K-major)
+// 2. exact product block on the tensor cores, D[(s, c)][m] = sum_k d_s[k, c] B[m][k], m < m_valid (B = counts, K-major):
+//    recombined into `out` by the GEMM's epilogue (fused route), or left as int32 planes in w.D (split-K route)
 int stats_i8_product(const StatsI8Buffers& w, int K, const uint8_t* B, long long ldb, int kdim_pad, int m_valid, int m_pad,
-                     double* out, const I8Guard* guard, int gemm2, cudaStream_t st) {
+                     double* out, const I8Guard* guard, cudaStream_t st) {
     const int L = K * (K + 1) / 2;
-    const int min_tiles = gemm2 == 0 ? (1 << 30) : (gemm2 == 1 ? 0 : 48);
-    const int rc = launch_i8gemm2(reinterpret_cast<const int8_t*>(B), ldb, m_valid, w.planes, kdim_pad, L, kdim_pad, w.expo, out,
-                                  L + K, min_tiles, guard, w.D, m_pad, st);
-    if (rc == 0) return I8_ROUTE_FUSED;
-    if (rc == 5) return I8_ROUTE_SPLITK;    // exact int32 partial sums in w.D: the recombination kernel finishes (and applies the guard)
-    if (rc > 1) return 0;
-    // few tiles (small tensors, narrow shards): 128 x 256 tiles with split-K and integer atomics through the int32 planes
-    // (the recombination kernel applies the guard on this route)
-    return launch_i8gemm(w.planes, kdim_pad, i8_plane_rows(L), reinterpret_cast<const int8_t*>(B), ldb, m_valid, kdim_pad, w.D,
-                         m_pad, st) ? 0 : I8_ROUTE_ROUND1;
+    return launch_i8gemm2(reinterpret_cast<const int8_t*>(B), ldb, m_valid, w.planes, kdim_pad, L, kdim_pad, w.expo, out, L + K,
+                          guard, w.D, m_pad, st);
 }
 
 // 3. linear block in FP64: bpart[split][m][j] = sum_k S[m, k] F[k, j] over the split's k range; returns the split count

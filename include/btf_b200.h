@@ -164,8 +164,8 @@ int btf_inject_noise(btf_engine* e, const char* name, const double* host, size_t
  * "V_retries" [Mloc], "row_stats" [Nloc,L+K], "col_stats" [M*T,L+K],
  * "nu2_rate" [3] = (a_post,b_post,n_obs), "lam2_rate" [2],
  * "i8_route" [2] = route of the last row / column product block of the integer
- * statistics path: 0 none yet, 1 round-1 kernel, 2 2-CTA kernel with the fused
- * epilogue, 3 2-CTA kernel in split-K mode (recorded without btf_enable_diag). */
+ * statistics path: 0 none yet, 2 2-CTA kernel with the fused epilogue, 3 2-CTA
+ * kernel in split-K mode (recorded without btf_enable_diag). */
 int btf_enable_diag(btf_engine* e, int32_t on);
 int btf_get_diag(btf_engine* e, const char* name, double* host, size_t n);
 
@@ -185,11 +185,6 @@ double btf_i8_peak(int32_t device, int32_t iters);
 int btf_pg_sample(int32_t device, const double* b, const double* z, double* out, int64_t n, uint64_t seed);
 int btf_rng_sample(int32_t device, int32_t kind, double param, double* out, int64_t n, uint64_t seed);
 
-/* Exact int8 x int8 -> int32 GEMM on the tcgen05 tensor cores (test / benchmark hook of the digit-plane
- * statistics path): D[M, N] = A[M, K] . B[N, K]^T, host buffers, K a multiple of 128.  Returns the time of
- * `reps` launches in ms, negative on failure. */
-double btf_i8gemm_test(int32_t device, const int8_t* A, const int8_t* B, int32_t* D, int32_t M, int32_t N, int32_t K,
-                       int32_t reps);
 /* ---- NCCL plumbing for the sharded sweep (SURVEY.md section 8e) */
 int btf_nccl_unique_id(char* id128);                    /* 128-byte ncclUniqueId */
 int btf_nccl_init(btf_engine* e, const char* id128);    /* uses cfg.world_size / cfg.rank */

@@ -1,6 +1,6 @@
 """CPU restatement of the exact fixed-point contraction of the integer statistics path.  TEST INFRASTRUCTURE.
 
-The engine (functionalmf_b200/csrc/stats_i8.cu + i8gemm2.cu / i8gemm.cu) computes the product block of the
+The engine (functionalmf_b200/csrc/stats_i8.cu + i8gemm2.cu) computes the product block of the
 sufficient statistics
 
     out[m, c] = sum_k cnt[m, k] * Z[k, c],      Z[k, (k1, k2)] = F[k, k1] * F[k, k2]   (k2 <= k1, packed)

@@ -1,11 +1,13 @@
-"""Integer-tensor-core statistics path (i8gemm.cu, stats_i8.cu).
+"""Integer-tensor-core statistics path (stats_i8.cu, i8gemm2.cu).
 
-* the tcgen05 int8 GEMM is bit-exact against numpy integer arithmetic (ragged shapes included);
 * the product block of the sufficient statistics equals, BIT FOR BIT, the correctly rounded value
-  of the fixed-point sum it is defined as (checked in Python big-integer arithmetic);
+  of the fixed-point sum it is defined as (checked in Python big-integer arithmetic), on the fused route and on the
+  split-K route through the int32 planes, for rows and for columns;
 * a sweep on the integer path equals the same sweep on the FP64 DMMA path to rounding.
+
+The route is the engine's own choice: the fused epilogue unless the 256 x 256 tiles are fewer than 48 and the
+contraction (rows: M T, columns: N, padded) is at least 2048 long, so that a split of 2 fits.
 """
-import ctypes as C
 import os
 import numpy as np
 import pytest
@@ -13,52 +15,21 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 
-def _gemm(A, B):
-    from functionalmf_b200 import _lib as L
-    lib = L.load()
-    M, K = A.shape
-    N = B.shape[0]
-    D = np.zeros((M, N), dtype=np.int32)
-    ms = lib.btf_i8gemm_test(0, C.c_void_p(A.ctypes.data), C.c_void_p(B.ctypes.data), C.c_void_p(D.ctypes.data), M, N, K, 1)
-    assert ms >= 0
-    return D
-
-
-@pytest.mark.parametrize('shape', [(128, 256, 128), (1, 1, 128), (130, 257, 384), (200, 300, 1024), (1088, 520, 2048), (128, 256, 8192), (300, 100, 16384)])
-def test_i8gemm_exact(shape):
-    M, N, K = shape
-    rs = np.random.RandomState(M + N + K)
-    A = rs.randint(-64, 64, size=(M, K)).astype(np.int8)
-    B = rs.randint(0, 4, size=(N, K)).astype(np.int8)
-    np.testing.assert_array_equal(_gemm(A, B), A.astype(np.int32) @ B.astype(np.int32).T)
-    # extreme digits and counts: the int32 accumulators hold them exactly
-    A[:] = -64
-    B[:] = 127
-    np.testing.assert_array_equal(_gemm(A, B), np.full((M, N), -64 * 127 * K, dtype=np.int32))
-
-
-# BTF_I8_GEMM2: '1' = the 2-CTA kernel with the recombination in its epilogue at every shape, '0' = the round-1 kernel
-# through the int32 planes; the engine reads it when it is created
-GEMM_MODES = ('1', '0')
-
-
-def _want_route(gemm_mode):
-    from functionalmf_b200 import _lib as L
-    return {'1': L.I8_ROUTE_FUSED, '0': L.I8_ROUTE_ROUND1}[gemm_mode]
-
-
-def _engine(N, M, T, R, K, env, gemm_mode=None):
+def _engine(N, M, T, R, K, env):
     from functionalmf_b200.engine import Engine
-    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8', 'BTF_I8_GEMM2'):
+    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8'):
         os.environ.pop(k, None)
     os.environ[env] = '1'
-    if gemm_mode:
-        os.environ['BTF_I8_GEMM2'] = gemm_mode
     try:
         return Engine(N, M, T, nembeds=K, tf_order=2, seed=5, use_graph=0)
     finally:
-        for k in (env, 'BTF_I8_GEMM2'):
-            os.environ.pop(k, None)
+        os.environ.pop(env, None)
+
+
+def _routes(*names):
+    """I8_ROUTE_* values of the row and the column product block, as btf_get_diag('i8_route') reports them"""
+    from functionalmf_b200 import _lib as L
+    return [getattr(L, 'I8_ROUTE_' + n) for n in names]
 
 
 def _problem(N, M, T, R, K, seed):
@@ -82,12 +53,15 @@ def _load(eng, rs, W, V):
         eng.set(k, [v])
 
 
-@pytest.mark.parametrize('gemm_mode', GEMM_MODES, ids=('two_cta_fused', 'round1'))
-@pytest.mark.parametrize('shape', [(150, 9, 21, 3, 8), (300, 7, 40, 2, 16), (129, 5, 33, 4, 32)])
-def test_product_block_is_the_exact_fixed_point_sum(shape, gemm_mode):
+# (N, M, T, R, K), routes of the row and the column product block
+@pytest.mark.parametrize('shape,routes', [
+    ((150, 9, 21, 3, 8), ('FUSED', 'FUSED')), ((300, 7, 40, 2, 16), ('FUSED', 'FUSED')), ((129, 5, 33, 4, 32), ('FUSED', 'FUSED')),
+    ((40, 8, 230, 2, 8), ('SPLITK', 'FUSED')), ((1930, 3, 8, 2, 16), ('FUSED', 'SPLITK')), ((1930, 2, 5, 2, 32), ('FUSED', 'SPLITK')),
+], ids=('K8', 'K16', 'K32', 'K8_rows_split_k', 'K16_cols_split_k', 'K32_cols_split_k'))
+def test_product_block_is_the_exact_fixed_point_sum(shape, routes):
     N, M, T, R, K = shape
     rs, W, V, Y = _problem(N, M, T, R, K, 11)
-    eng = _engine(N, M, T, R, K, 'BTF_STATS_FORCE_I8', gemm_mode)
+    eng = _engine(N, M, T, R, K, 'BTF_STATS_FORCE_I8')
     try:
         eng.set_data_gaussian(Y)
         _load(eng, rs, W, V)
@@ -97,7 +71,7 @@ def test_product_block_is_the_exact_fixed_point_sum(shape, gemm_mode):
         z = np.zeros(N * K)
         eng.inject('z_W', z)                  # W stays at its conditional mean: the V statistics use a known W
         eng.sweep(1)
-        assert list(eng.diag('i8_route')) == [_want_route(gemm_mode)] * 2
+        assert list(eng.diag('i8_route')) == _routes(*routes)
         L = K * (K + 1) // 2
         cnt = (~np.isnan(Y)).sum(axis=-1).reshape(N, M * T)
         Ssum = np.nansum(Y, axis=-1).reshape(N, M * T)
@@ -119,21 +93,23 @@ def test_product_block_is_the_exact_fixed_point_sum(shape, gemm_mode):
         eng.close()
 
 
-@pytest.mark.parametrize('gemm_mode', GEMM_MODES, ids=('two_cta_fused', 'round1'))
-@pytest.mark.parametrize('shape', [(260, 12, 24, 3, 16), (140, 6, 30, 2, 8), (200, 5, 20, 3, 32)])
-def test_sweep_matches_the_fp64_path(shape, gemm_mode):
+@pytest.mark.parametrize('shape,routes', [
+    ((260, 12, 24, 3, 16), ('FUSED', 'FUSED')), ((140, 6, 30, 2, 8), ('FUSED', 'FUSED')), ((200, 5, 20, 3, 32), ('FUSED', 'FUSED')),
+    ((1930, 3, 8, 2, 8), ('FUSED', 'SPLITK')), ((60, 8, 230, 3, 16), ('SPLITK', 'FUSED')), ((40, 4, 450, 2, 32), ('SPLITK', 'FUSED')),
+], ids=('K16', 'K8', 'K32', 'K8_cols_split_k', 'K16_rows_split_k', 'K32_rows_split_k'))
+def test_sweep_matches_the_fp64_path(shape, routes):
     N, M, T, R, K = shape
     rs, W, V, Y = _problem(N, M, T, R, K, 21)
     res = {}
     for env in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8'):
-        eng = _engine(N, M, T, R, K, env, gemm_mode)
+        eng = _engine(N, M, T, R, K, env)
         try:
             eng.set_data_gaussian(Y)
             _load(eng, rs, W, V)
             eng.enable_diag(True)
             eng.sweep(2)
             if env == 'BTF_STATS_FORCE_I8':
-                assert list(eng.diag('i8_route')) == [_want_route(gemm_mode)] * 2
+                assert list(eng.diag('i8_route')) == _routes(*routes)
             res[env] = dict(W=eng.get('W'), V=eng.get('V'), Tau2=eng.get('Tau2'), nu2=eng.get_scalar('nu2'),
                             sigma2=eng.get_scalar('sigma2'), rows=eng.diag('row_stats'), cols=eng.diag('col_stats'))
         finally:
@@ -147,28 +123,30 @@ def test_sweep_matches_the_fp64_path(shape, gemm_mode):
 
 
 def test_two_cta_gemm_split_k_and_fused_modes_are_exact():
-    """300 rows x (64 x 128) columns at K = 16: the row contraction has 2 x 4 tiles of the 2-CTA GEMM, so it runs in its
-    split-K mode (int32 atomics + recombination kernel); the column contraction has 128 tiles and runs with the fused
-    epilogue.  Both must equal the fixed-point definition bit for bit (oracle.fixed_point.product_block_fast)."""
+    """Both routes on both sides, at K = 16.  300 rows x (64 x 128) columns: the row contraction has 2 x 4 tiles of the
+    2-CTA GEMM and is 8192 long, so it runs in split-K mode (int32 atomics + recombination kernel), and the column
+    contraction has 128 tiles and runs with the fused epilogue.  2048 rows x (8 x 16) columns, the transposed case: the
+    column contraction has 4 tiles and is 2048 long (split-K), the row contraction has 32 tiles but is only 256 long
+    (fused).  Every block must equal the fixed-point definition bit for bit (oracle.fixed_point.product_block_fast)."""
     from oracle.fixed_point import product_block_fast
     from functionalmf_b200 import _lib as L
-    N, M, T, R, K = 300, 64, 128, 2, 16
-    rs, W, V, Y = _problem(N, M, T, R, K, 31)
-    eng = _engine(N, M, T, R, K, 'BTF_STATS_FORCE_I8')
-    try:
-        eng.set_data_gaussian(Y)
-        _load(eng, rs, W, V)
-        eng.enable_diag(True)
-        eng.set_sample_mask(L.SAMPLE_W | L.SAMPLE_V)
-        eng.inject('z_W', np.zeros(N * K))
-        eng.sweep(1)
-        assert list(eng.diag('i8_route')) == [L.I8_ROUTE_SPLITK, L.I8_ROUTE_FUSED]
-        Lp = K * (K + 1) // 2
-        cnt = (~np.isnan(Y)).sum(axis=-1).reshape(N, M * T)
-        np.testing.assert_array_equal(eng.diag('row_stats')[:, :Lp], product_block_fast((V * 1.1).reshape(M * T, K), cnt))
-        np.testing.assert_array_equal(eng.diag('col_stats')[:, :Lp], product_block_fast(eng.get('W'), cnt.T))
-    finally:
-        eng.close()
+    for (N, M, T, R, K), routes in (((300, 64, 128, 2, 16), ('SPLITK', 'FUSED')), ((2048, 8, 16, 2, 16), ('FUSED', 'SPLITK'))):
+        rs, W, V, Y = _problem(N, M, T, R, K, 31)
+        eng = _engine(N, M, T, R, K, 'BTF_STATS_FORCE_I8')
+        try:
+            eng.set_data_gaussian(Y)
+            _load(eng, rs, W, V)
+            eng.enable_diag(True)
+            eng.set_sample_mask(L.SAMPLE_W | L.SAMPLE_V)
+            eng.inject('z_W', np.zeros(N * K))
+            eng.sweep(1)
+            assert list(eng.diag('i8_route')) == _routes(*routes), (N, M, T)
+            Lp = K * (K + 1) // 2
+            cnt = (~np.isnan(Y)).sum(axis=-1).reshape(N, M * T)
+            np.testing.assert_array_equal(eng.diag('row_stats')[:, :Lp], product_block_fast((V * 1.1).reshape(M * T, K), cnt))
+            np.testing.assert_array_equal(eng.diag('col_stats')[:, :Lp], product_block_fast(eng.get('W'), cnt.T))
+        finally:
+            eng.close()
 
 
 def _exact_product_block(F, cnt):
@@ -179,20 +157,21 @@ def _exact_product_block(F, cnt):
     return (cnt.astype(np.longdouble) @ Z).astype(np.float64)
 
 
-def _guard_case(no_guard):
-    """Block-structured missingness + factor scales spanning 1e6 (VERDICT r1, weak #1): rows >= 200 observe only the
-    columns whose V is 1e-6 times smaller, so their statistics sit 1e-12 below the column maxima that fix the
-    fixed-point scale; same construction transposed for the column statistics."""
+def _guard_case(no_guard, N, T):
+    """Block-structured missingness + factor scales spanning 1e6 (VERDICT r1, weak #1): the last 56 rows observe only
+    the columns j >= 4, whose V is 1e-6 times smaller, so their statistics sit 1e-12 below the column maxima that fix the
+    fixed-point scale; same construction transposed for the column statistics: the columns j = 6, 7 (2 T of the (j, t))
+    observe only the rows >= N / 2, whose W is 1e-6 times smaller."""
     from functionalmf_b200 import _lib as L
-    N, M, T, R, K = 256, 8, 16, 2, 16
+    M, R, K = 8, 2, 16
     rs = np.random.RandomState(4)
     V = rs.normal(size=(M, T, K)); V[4:] *= 1e-6
-    W = rs.normal(size=(N, K)); W[128:] *= 1e-6
+    W = rs.normal(size=(N, K)); W[N // 2:] *= 1e-6
     Y = rs.normal(size=(N, M, T, R))
     Y[rs.random_sample(Y.shape) < 0.2] = np.nan
-    Y[200:, :4] = np.nan                  # rows 200.. see only the small columns
-    Y[:128, 6:] = np.nan                  # columns 6.. see only the small rows
-    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8', 'BTF_I8_NO_GUARD', 'BTF_I8_GEMM2'):
+    Y[N - 56:, :4] = np.nan               # the last 56 rows see only the small columns
+    Y[:N // 2, 6:] = np.nan               # columns 6.. see only the small rows
+    for k in ('BTF_STATS_FORCE_I8', 'BTF_STATS_NO_I8', 'BTF_I8_NO_GUARD'):
         os.environ.pop(k, None)
     os.environ['BTF_STATS_FORCE_I8'] = '1'
     if no_guard:
@@ -229,6 +208,7 @@ def _guard_case(no_guard):
         out['row_rel'] = np.abs(rows[:, dg] / want[:, dg] - 1.0)
         sc = np.sqrt(want[:, dg][:, il[0]] * want[:, dg][:, il[1]])
         out['row_off'] = np.abs(rows - want) / sc
+        out['routes'] = list(eng.diag('i8_route'))
         return out
     finally:
         eng.close()
@@ -240,11 +220,16 @@ def test_elementwise_guard_keeps_badly_scaled_rows_accurate():
     """Element-wise (not normwise) accuracy of the integer path: every diagonal entry of every row / (j,t) statistic to
     1e-10 relative, every off-diagonal entry to 1e-10 of sqrt(d1 d2), although the fixed-point scale is set by column
     maxima 1e12 times larger.  The guard must list exactly the rows / columns that only see the small factors, and
-    without it (BTF_I8_NO_GUARD=1) the same data must miss the bound - the test has teeth."""
-    g = _guard_case(no_guard=False)
-    assert g['row_flagged'] == 56 and g['col_flagged'] == 2 * 16          # rows 200..255; columns j = 6, 7 at every t
-    assert g['row_rel'].max() < 1e-10 and g['col_rel'].max() < 1e-10
-    assert g['row_off'].max() < 1e-10 and g['col_off'].max() < 1e-10
-    bad = _guard_case(no_guard=True)
-    assert bad['row_flagged'] == 0 and bad['col_flagged'] == 0
-    assert bad['row_rel'].max() > 1e-8 and bad['col_rel'].max() > 1e-8
+    without it (BTF_I8_NO_GUARD=1) the same data must miss the bound - the test has teeth.  The GEMM epilogue applies
+    the guard on the fused route and the recombination kernel on the split-K route: N = 256, T = 16 runs both sides
+    fused; T = 256 makes the row contraction 2048 long over 4 tiles (split-K), N = 2048 does the same for the columns."""
+    for N, T, routes in ((256, 16, ('FUSED', 'FUSED')), (256, 256, ('SPLITK', 'FUSED')), (2048, 16, ('FUSED', 'SPLITK'))):
+        g = _guard_case(False, N, T)
+        assert g['routes'] == _routes(*routes), (N, T)
+        assert g['row_flagged'] == 56 and g['col_flagged'] == 2 * T, (N, T)        # the last 56 rows; columns j = 6, 7 at every t
+        assert g['row_rel'].max() < 1e-10 and g['col_rel'].max() < 1e-10, (N, T)
+        assert g['row_off'].max() < 1e-10 and g['col_off'].max() < 1e-10, (N, T)
+        bad = _guard_case(True, N, T)
+        assert bad['routes'] == _routes(*routes), (N, T)
+        assert bad['row_flagged'] == 0 and bad['col_flagged'] == 0, (N, T)
+        assert bad['row_rel'].max() > 1e-8 and bad['col_rel'].max() > 1e-8, (N, T)
