@@ -68,6 +68,7 @@ SIGNATURES = {
     'btf_set_data_gaussian_rows': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     'btf_set_data_binomial': (C.c_int, [_P, _P, _P]),
     'btf_set_data_negbin': (C.c_int, [_P, _P, C.c_int32]),
+    'btf_set_nu2_cells': (C.c_int, [_P, _P]),
     'btf_set_state': (C.c_int, [_P, C.c_char_p, _P, C.c_size_t]),
     'btf_get_state': (C.c_int, [_P, C.c_char_p, _P, C.c_size_t]),
     'btf_delta_rows': (C.c_int, [_P]),
@@ -80,6 +81,7 @@ SIGNATURES = {
     'btf_mu_stats_track': (C.c_int, [_P, C.c_int32]),
     'btf_mu_stats_get': (C.c_int, [_P, _P, _P, C.POINTER(C.c_int64)]),
     'btf_eval_set': (C.c_int, [_P, C.c_int32, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int64]),
+    'btf_eval_set_nu2': (C.c_int, [_P, C.c_int32, _P]),
     'btf_eval_clear': (C.c_int, [_P, C.c_int32]),
     'btf_eval_update': (C.c_int, [_P, C.c_int32]),
     'btf_eval_samples': (C.c_int, [_P, C.c_int32, _P, C.POINTER(C.c_int64)]),

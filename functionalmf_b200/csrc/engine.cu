@@ -62,6 +62,7 @@ struct EvalSlot {
     double *mean = nullptr, *below = nullptr, *above = nullptr, *cdf = nullptr;
     unsigned *c_lt = nullptr, *c_le = nullptr;
     double *partial = nullptr, *samples = nullptr, *summary = nullptr;
+    double* nu2 = nullptr;       // [nloc][P] known per-cell variances of the scored cells (btf_eval_set_nu2)
     long long count = 0, max_samples = 0;
 };
 constexpr int EVAL_SLOTS = 4;
@@ -88,6 +89,13 @@ struct btf_engine {
     double* ntr = nullptr;       // PG paths: number of trials b
     double* omega = nullptr;     // PG paths: Polya-Gamma draws
     double* Yraw = nullptr;      // NB: raw counts [nloc][P][R]
+    // Gaussian with known per-cell noise variances (btf_set_nu2_cells; single GPU): the statistics take the f64 weights
+    // wc = cnt / nu2 and sc = S / nu2, formed from the kept variances nu2c whenever data or variances change
+    bool nu2_cells = false, nu2_dirty = false;
+    unsigned long long nu2_bad = 0;                            // observed cells whose variance is NaN or <= 0
+    double *nu2c = nullptr, *wc = nullptr, *sc = nullptr;      // [nloc_pad][Ppad], allocated on first use
+    unsigned long long* nu2_nbad = nullptr;
+    StatsPlan plan_row_w{}, plan_col_w{};                      // statistics plans for those f64 weights
     int nreps = 1;
     bool has_data = false, data_reduced = false;
     double* staging[2] = {nullptr, nullptr};   // upload staging (kept for the engine's lifetime: no malloc/free per call, no leak on error paths)
@@ -412,12 +420,18 @@ int btf_create(const btf_config* c, btf_engine** out) {
     return BTF_OK;
 }
 
+// the statistics plan of the rows (col = false) or columns: count weights, or f64 weights with per-cell variances
+static const StatsPlan& stats_plan(const btf_engine* e, bool col) {
+    if (e->nu2_cells) return col ? e->plan_col_w : e->plan_row_w;
+    return col ? e->plan_col : e->plan_row;
+}
+
 static void free_graph(btf_engine* e) {
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
 }
 
 static void eval_free(EvalSlot& s) {
-    void* ptrs[] = {s.target, s.cls, s.mean, s.below, s.above, s.cdf, s.c_lt, s.c_le, s.partial, s.samples, s.summary};
+    void* ptrs[] = {s.target, s.cls, s.mean, s.below, s.above, s.cdf, s.c_lt, s.c_le, s.partial, s.samples, s.summary, s.nu2};
     for (void* p : ptrs) if (p) cudaFree(p);
     s = EvalSlot();
 }
@@ -431,7 +445,7 @@ void btf_destroy(btf_engine* e) {
     void* ptrs[] = {e->W, e->V, e->Tau2, e->Tau2_a, e->Tau2_b, e->Tau2_c, e->scal, e->cnt, e->S, e->ntr, e->omega,
                     e->Yraw, e->Rdisp, e->nb_work, e->nb_hist, e->d_start, e->d_width, e->d_coef, e->pm_ptr, e->pm_row, e->pm_coef,
                     e->row_stats, e->col_stats, e->zbuf, e->mu_mean, e->mu_m2, e->work_L, e->work_y, e->partials, e->lam_partials, e->resid_partials,
-                    e->snapW, e->snapV, e->snapTau2, e->snapScal, e->snapR, e->diag_retries};
+                    e->snapW, e->snapV, e->snapTau2, e->snapScal, e->snapR, e->diag_retries, e->nu2c, e->wc, e->sc, e->nu2_nbad};
     for (void* p : ptrs) if (p) cudaFree(p);
     {
         void* i8p[] = {e->i8.planes, e->i8.colmax, e->i8.expo, e->i8.D, e->i8.bpart, e->cntT, e->cnt_rowsum, e->cnt_colsum, e->guard_n, e->guard_flags, e->Scol};
@@ -581,6 +595,7 @@ int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int
     CK(cudaStreamSynchronize(e->stream));
     CK(cudaGetLastError());
     e->has_data = true; e->data_reduced = false; e->resid_valid = false; e->i8_decided = false;
+    e->nu2_dirty = true;
     return BTF_OK;
 }
 
@@ -670,6 +685,91 @@ int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps) {
     return BTF_OK;
 }
 
+// Known per-cell noise variances (the reference's heteroskedastic Gaussian branch: nu2 an [N, M, T] array).
+// First use: the statistics plans for f64 weights (their split buffers may be larger) and the cell buffers.
+static int ensure_nu2_buffers(btf_engine* e) {
+    if (e->wc) return BTF_OK;
+    if (!plan_stats(&e->plan_row_w, e->K, false, true, e->nloc_pad, e->Ppad, e->nloc, e->cfg.stats_splits_row, e->sm_count) ||
+        !plan_stats(&e->plan_col_w, e->K, true, true, e->Ppad, e->nloc_pad, e->P, e->cfg.stats_splits_col, e->sm_count))
+        return set_err(BTF_EINVAL, "no statistics plan for per-cell weights at K=%d", e->K);
+    auto grow = [](double** buf, const StatsPlan& have, const StatsPlan& want) -> cudaError_t {
+        const size_t nh = have.nsplit * have.out_elems_per_split, nw = want.nsplit * want.out_elems_per_split;
+        if (nw <= nh) return cudaSuccess;
+        cudaFree(*buf); *buf = nullptr;
+        return dev_alloc(buf, nw);
+    };
+    CK(grow(&e->row_stats, e->plan_row, e->plan_row_w));
+    CK(grow(&e->col_stats, e->plan_col, e->plan_col_w));
+    const size_t cells = (size_t)e->nloc_pad * e->Ppad;
+    CK(dev_alloc(&e->nu2_nbad, 1));
+    CK(dev_alloc(&e->nu2c, cells));
+    CK(dev_alloc(&e->sc, cells));
+    CK(dev_alloc(&e->wc, cells));
+    return BTF_OK;
+}
+
+// Weights from `rows` rows of variances at pitch lds (starting at local row row0); keep != 0: store the variances too.
+static void enqueue_nu2_weights(btf_engine* e, const double* nu2, long long lds, int row0, int rows, bool keep) {
+    const size_t o = (size_t)row0 * e->Ppad;
+    launch_nu2_weights(nu2, lds, rows, e->P, e->cnt + o, e->S + o, e->Ppad, keep ? e->nu2c + o : nullptr, e->wc + o,
+                       e->sc + o, e->nu2_nbad, e->stream);
+    e->launches++;
+}
+
+static int read_nu2_bad(btf_engine* e) {
+    CK(cudaMemcpyAsync(e->pinned_scal, e->nu2_nbad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    CK(cudaGetLastError());
+    memcpy(&e->nu2_bad, e->pinned_scal, sizeof(unsigned long long));
+    return BTF_OK;
+}
+
+static int nu2_bad_error(btf_engine* e) {
+    return set_err(BTF_EINVAL, "%llu observed cell(s) have a noise variance that is NaN or <= 0 (+inf marks a cell as missing)",
+                   e->nu2_bad);
+}
+
+int btf_set_nu2_cells(btf_engine* e, const double* nu2) {
+    if (!e) return set_err(BTF_EINVAL, "null engine");
+    if (e->cfg.likelihood != BTF_GAUSSIAN) return set_err(BTF_ESTATE, "per-cell noise variances need a Gaussian engine");
+    if (e->cfg.world_size > 1) return set_err(BTF_EINVAL, "per-cell noise variances are single-GPU");
+    CK(cudaSetDevice(e->cfg.device));
+    CK(cudaStreamSynchronize(e->stream));
+    // the sweep changes route (and the integer statistics path is decided again): drop the captured graph
+    free_graph(e);
+    e->i8_decided = false;
+    e->resid_valid = false;
+    e->nu2_cells = false;         // scalar mode until the variances are accepted
+    if (!nu2) return BTF_OK;
+    { int rc = ensure_nu2_buffers(e); if (rc) return rc; }
+    CK(cudaMemsetAsync(e->nu2_nbad, 0, sizeof(unsigned long long), e->stream));
+    const size_t row_elems = (size_t)e->P;
+    if (is_device_ptr(nu2)) {
+        enqueue_nu2_weights(e, nu2, e->P, 0, e->nloc, true);
+    } else {
+        const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)std::max(e->nloc, 1), ((size_t)128 << 20) / (row_elems * 8)));
+        const size_t need = (size_t)chunk * row_elems * sizeof(double);
+        if (need > e->staging_bytes) {                 // engine-lifetime staging buffers (freed by btf_destroy)
+            for (int b = 0; b < 2; ++b) { if (e->staging[b]) cudaFree(e->staging[b]); e->staging[b] = nullptr; }
+            e->staging_bytes = 0;
+            for (int b = 0; b < 2; ++b) CK(cudaMalloc((void**)&e->staging[b], need));
+            e->staging_bytes = need;
+        }
+        int piece = 0;
+        for (int r0 = 0; r0 < e->nloc; r0 += chunk, ++piece) {
+            const int rows = std::min(chunk, e->nloc - r0);
+            double* buf = e->staging[piece & 1];
+            int rc = upload_rows(e, nu2, row_elems, r0, rows, buf); if (rc) return rc;
+            enqueue_nu2_weights(e, buf, e->P, r0, rows, true);
+        }
+    }
+    { int rc = read_nu2_bad(e); if (rc) return rc; }
+    e->nu2_dirty = false;
+    if (e->nu2_bad) return nu2_bad_error(e);
+    e->nu2_cells = true;
+    return BTF_OK;
+}
+
 // ------------------------------------------------------------------ state
 struct StateRef { double* p; size_t n; bool scalar_field; };
 
@@ -728,7 +828,7 @@ int btf_set_state(btf_engine* e, const char* name, const double* host, size_t n)
     if (nm == "W" || nm == "V") e->resid_valid = false;
     // restoring a checkpoint: the residual sum that belongs to the (W, V) just set, so that the next nu2 step uses the same
     // number the interrupted chain would have used (set it AFTER W and V)
-    if (nm == "resid" && e->cfg.likelihood == BTF_GAUSSIAN && e->has_data) e->resid_valid = true;
+    if (nm == "resid" && e->cfg.likelihood == BTF_GAUSSIAN && e->has_data && !e->nu2_cells) e->resid_valid = true;
     return BTF_OK;
 }
 
@@ -832,7 +932,7 @@ int btf_get_diag(btf_engine* e, const char* name, double* host, size_t n) {
     }
     if (nm == "row_stats" || nm == "col_stats") {
         // sum of the split partials, in split order
-        const StatsPlan& pl = nm == "row_stats" ? e->plan_row : e->plan_col;
+        const StatsPlan& pl = stats_plan(e, nm == "col_stats");
         const double* src = nm == "row_stats" ? e->row_stats : e->col_stats;
         if (n != pl.out_elems_per_split) return set_err(BTF_EINVAL, "%s: expected %zu values", name, pl.out_elems_per_split);
         std::vector<double> tmp(n);
@@ -1008,7 +1108,8 @@ static int ensure_i8(btf_engine* e) {
     if (e->i8_decided) return BTF_OK;
     e->i8_decided = true;
     e->i8_on = false;
-    if (e->cfg.likelihood != BTF_GAUSSIAN || !e->has_data || e->env.no_i8) return BTF_OK;
+    // (per-cell variances make the weights cnt / nu2 non-integer)
+    if (e->cfg.likelihood != BTF_GAUSSIAN || !e->has_data || e->env.no_i8 || e->nu2_cells) return BTF_OK;
     const long long cells = (long long)e->N * e->P / std::max(1, e->cfg.world_size);
     if (!stats_i8_supported(e->K, e->nreps, e->Ppad, e->Nall_pad)) return BTF_OK;
     if (e->cfg.world_size > 1 && !e->shard) return BTF_OK;       // a shard without a communicator cannot build its column copy
@@ -1120,6 +1221,9 @@ static int enqueue_sweep(btf_engine* e) {
     const btf_config& c = e->cfg;
     cudaStream_t st = e->stream;
     const bool gauss = c.likelihood == BTF_GAUSSIAN;
+    // known per-cell variances: the PG models' f64-weight route, with weights cnt / nu2 and right-hand side S / nu2
+    const bool percell = gauss && e->nu2_cells;
+    const bool homo = gauss && !percell;      // one scalar nu2 scales the statistics
     const int mask = c.sample_mask;
     launch_bump_sweep(e->scal, st); e->launches++;
     phase_mark(e, PH_NU2);
@@ -1213,20 +1317,24 @@ static int enqueue_sweep(btf_engine* e) {
     }
     // ---- W | rest
     phase_mark(e, PH_ROW_STATS);
-    const void* wt = gauss ? (const void*)e->cnt : (const void*)e->omega;
+    const void* wt = percell ? (const void*)e->wc : gauss ? (const void*)e->cnt : (const void*)e->omega;
+    const double* sv = percell ? e->sc : e->S;
+    const bool wf64 = !homo;
+    const StatsPlan& prow = stats_plan(e, false);
+    const StatsPlan& pcol = stats_plan(e, true);
     if (doW) {
         if (e->i8_on) {
             if (!fork) { int rc = begin_row_stats_i8(e, false, 0, &pend_row); if (rc) return rc; }
             { int rc = finish_row_stats_i8(e, fork, pend_row); if (rc) return rc; }
         } else {
-            launch_stats(e->plan_row, false, !gauss, wt, e->S, e->V, e->Ppad, e->Ppad, e->nloc, e->row_stats, e->zbuf, st);
-            e->launches += e->plan_row.zpre ? 2 : 1;
+            launch_stats(prow, false, wf64, wt, sv, e->V, e->Ppad, e->Ppad, e->nloc, e->row_stats, e->zbuf, st);
+            e->launches += prow.zpre ? 2 : 1;
         }
         phase_mark(e, PH_ROW_SOLVE);
         RowSolveArgs ra;
-        ra.stats = e->row_stats; ra.nsplit = e->i8_on ? 1 : e->plan_row.nsplit; ra.split_stride = e->plan_row.out_elems_per_split;
+        ra.stats = e->row_stats; ra.nsplit = e->i8_on ? 1 : prow.nsplit; ra.split_stride = prow.out_elems_per_split;
         ra.nloc = e->nloc; ra.row_begin = c.row_begin; ra.K = e->K;
-        ra.scale_from_nu2 = gauss ? &e->scal->nu2 : nullptr; ra.scal = e->scal; ra.W = e->W;
+        ra.scale_from_nu2 = homo ? &e->scal->nu2 : nullptr; ra.scal = e->scal; ra.W = e->W;
         ra.z_inject = inj(e, "z_W"); ra.seed = c.seed;
         ra.diag_Q = diag_get(e, "W_Q", (size_t)e->N * e->K * e->K);
         ra.diag_L = diag_get(e, "W_L", (size_t)e->N * e->K * e->K);
@@ -1244,9 +1352,9 @@ static int enqueue_sweep(btf_engine* e) {
     // ---- V | rest
     if (mask & BTF_SAMPLE_V) {
         BandSolveArgs ba;
-        ba.stats = e->col_stats; ba.nsplit = 1; ba.split_stride = e->plan_col.out_elems_per_split;
+        ba.stats = e->col_stats; ba.nsplit = 1; ba.split_stride = pcol.out_elems_per_split;
         ba.col_begin = c.col_begin; ba.ncols_loc = e->Mloc; ba.T = e->T; ba.K = e->K; ba.order = e->order; ba.RD = e->RD;
-        ba.homoskedastic = gauss ? 1 : 0; ba.scal = e->scal; ba.Tau2 = e->Tau2;
+        ba.homoskedastic = homo ? 1 : 0; ba.scal = e->scal; ba.Tau2 = e->Tau2;
         ba.prior_clip = c.clip_prior_precision ? c.stability : 0.0;
         ba.pm_ptr = e->pm_ptr; ba.pm_row = e->pm_row; ba.pm_coef = e->pm_coef;
         ba.V = e->V; ba.z_inject = inj(e, "z_V"); ba.seed = c.seed;
@@ -1259,28 +1367,28 @@ static int enqueue_sweep(btf_engine* e) {
         ba.diag_chol = diag_get(e, "V_chol", bn);
         ba.diag_mean = diag_get(e, "V_mean", (size_t)e->P * e->K);
         ba.diag_retries = e->diag_retries;
-        ba.resid_partials = gauss ? e->resid_partials + c.col_begin : nullptr;
+        ba.resid_partials = homo ? e->resid_partials + c.col_begin : nullptr;
         auto band = [&]() { launch_band_solve(ba, st); e->launches++; };
         if (e->i8_on) {
             e->col_collapsed = false;
             int rc = col_step_i8(e, fork, 1, band);
             if (rc) return rc;
         } else {
-            int nsplit = e->plan_col.nsplit;
-            launch_stats(e->plan_col, true, !gauss, wt, e->S, e->W + (size_t)c.row_begin * e->K, e->nloc_pad, e->Ppad, e->P,
+            int nsplit = pcol.nsplit;
+            launch_stats(pcol, true, wf64, wt, sv, e->W + (size_t)c.row_begin * e->K, e->nloc_pad, e->Ppad, e->P,
                          e->col_stats, e->zbuf, st);
-            e->launches += e->plan_col.zpre ? 2 : 1;
+            e->launches += pcol.zpre ? 2 : 1;
             if (e->shard) {
                 // FP64 statistics path across GPUs: partial statistics over the local rows for all columns, collapsed
                 // over the splits, then reduce-scattered by column block
-                if (nccl_reduce_col_stats(e->shard, e->col_stats, nsplit, e->plan_col.out_elems_per_split, e->T * e->nco, st))
+                if (nccl_reduce_col_stats(e->shard, e->col_stats, nsplit, pcol.out_elems_per_split, e->T * e->nco, st))
                     return set_err(BTF_ENCCL, "reduce-scatter(col stats) failed");
                 nsplit = 1;
                 e->col_collapsed = true;
             } else if (nsplit > 2) {
                 // deep split-K (few columns): one pass that sums the partials in split order, instead of
                 // nsplit dependent loads per statistic inside the latency-bound band kernel
-                launch_collapse_splits(e->col_stats, nsplit, e->plan_col.out_elems_per_split, st);
+                launch_collapse_splits(e->col_stats, nsplit, pcol.out_elems_per_split, st);
                 e->launches++;
                 nsplit = 1;
                 e->col_collapsed = true;
@@ -1295,7 +1403,7 @@ static int enqueue_sweep(btf_engine* e) {
         if (e->shard) {
             if (nccl_allgather_cols(e->shard, e->V, e->n, st)) return set_err(BTF_ENCCL, "all-gather(V) failed");
         }
-        if (gauss && !c.resid_direct) {
+        if (homo && !c.resid_direct) {
             // nu2 by-product: resid = ss_total + sum_j [v^T A v - 2 v.b]
             if (e->shard) {
                 if (nccl_allgather_doubles(e->shard, e->resid_partials, st)) return set_err(BTF_ENCCL, "all-gather(resid) failed");
@@ -1307,6 +1415,7 @@ static int enqueue_sweep(btf_engine* e) {
         phase_mark(e, PH_BAND_SOLVE);
         phase_mark(e, PH_COMM);
     }
+    if (percell) e->resid_valid = false;   // no residual by-product: a later nu2 step takes the direct pass
     phase_mark(e, PH_COUNT);
     return BTF_OK;
 }
@@ -1382,6 +1491,20 @@ static int pre_run(btf_engine* e) {
     if (!e->has_data && ((e->cfg.sample_mask & needs_data) || e->cfg.likelihood != BTF_GAUSSIAN))
         return set_err(BTF_ESTATE, "no data: call btf_set_data_* first");
     CK(cudaSetDevice(e->cfg.device));
+    if (e->nu2_cells) {
+        if (e->cfg.sample_mask & BTF_SAMPLE_NU2)
+            return set_err(BTF_ESTATE, "the nu2 step does not run with per-cell noise variances: clear BTF_SAMPLE_NU2 or "
+                                       "return to a scalar nu2 with btf_set_nu2_cells(e, NULL)");
+        if (e->nu2_dirty && e->has_data) {
+            // the data changed since the weights were formed
+            CK(cudaMemsetAsync(e->nu2_nbad, 0, sizeof(unsigned long long), e->stream));
+            enqueue_nu2_weights(e, e->nu2c, e->Ppad, 0, e->nloc, false);
+            int rc = read_nu2_bad(e);
+            if (rc) return rc;
+            e->nu2_dirty = false;
+        }
+        if (e->nu2_bad) return nu2_bad_error(e);
+    }
     int rc = ensure_data_reduced(e);
     if (rc) return rc;
     launch_clear_info(e->scal, e->stream); e->launches++;
@@ -1575,6 +1698,7 @@ static EvalArgs eval_args(btf_engine* e, EvalSlot& s) {
     a.scal = e->scal; a.count = (double)s.count;
     a.mean = s.mean; a.below = s.below; a.above = s.above; a.cdf = s.cdf; a.c_lt = s.c_lt; a.c_le = s.c_le;
     a.partial = s.partial;
+    a.nu2c = s.nu2;
     return a;
 }
 static int eval_enqueue(btf_engine* e, int slot) {
@@ -1622,6 +1746,24 @@ int btf_eval_set(btf_engine* e, int32_t slot, const double* target, const uint8_
     CK(dev_alloc(&s.summary, (size_t)nclasses * 6));
     CK(cudaStreamSynchronize(e->stream));
     s.active = true;
+    return BTF_OK;
+}
+
+// known per-cell variances of the slot's cells [Nloc, M, T] (host or device memory) for the Gaussian log-likelihood and
+// the predictive band; NULL: the sample's scalar nu2 again
+int btf_eval_set_nu2(btf_engine* e, int32_t slot, const double* nu2) {
+    if (!e) return set_err(BTF_EINVAL, "null engine");
+    if (slot < 0 || slot >= EVAL_SLOTS || !e->eval[slot].active)
+        return set_err(BTF_ESTATE, "no evaluator in this slot (btf_eval_set first)");
+    CK(cudaSetDevice(e->cfg.device));
+    CK(cudaStreamSynchronize(e->stream));
+    EvalSlot& s = e->eval[slot];
+    if (s.nu2) { CK(cudaFree(s.nu2)); s.nu2 = nullptr; }
+    if (!nu2) return BTF_OK;
+    const size_t n = (size_t)e->nloc * e->P;
+    CK(dev_alloc(&s.nu2, n, false));
+    CK(cudaMemcpy(s.nu2, nu2, n * 8, cudaMemcpyDefault));
+    CK(cudaStreamSynchronize(cudaStreamLegacy));
     return BTF_OK;
 }
 

@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(256, KMAX <= 16 ? 2 : 1) eval_update_kernel(Ev
         for (int m = 0; m < 4; ++m) acc[c][m] = 0.0;
     }
     for (int r0 = 0; r0 < nr; r0 += B) {
-        double yv[B];
+        double yv[B], nv[B];
         int cv[B];
         double mv[B], bv[B], av[B], fv[B];
         unsigned ltv[B], lev[B];
@@ -96,6 +96,7 @@ __global__ void __launch_bounds__(256, KMAX <= 16 ? 2 : 1) eval_update_kernel(Ev
             const long long o = (long long)(i0 + r0 + u) * a.P + p;
             yv[u] = ok ? a.target[o] : NAN;
             cv[u] = ok ? (a.cls ? (int)a.cls[o] : 0) : 255;
+            nv[u] = (ok && a.nu2c) ? a.nu2c[o] : nu2;
         }
         if (STATE) {
 #pragma unroll
@@ -123,8 +124,10 @@ __global__ void __launch_bounds__(256, KMAX <= 16 ? 2 : 1) eval_update_kernel(Ev
                 if (k < K) psi += ws[r * K + k] * v[k];
             const double mu = eval_transform(a, psi, i0 + r, p);
             const double d = y - mu;
+            double ln = lognorm, inu = inv_nu2, isd = inv_sd;
+            if (a.nu2c) { ln = log(6.283185307179586477 * nv[u]); inu = 1.0 / nv[u]; isd = rsqrt(nv[u]); }
             double ll = 0.0;
-            if (a.loglik == EVAL_LL_GAUSSIAN) ll = -0.5 * (lognorm + d * d * inv_nu2);
+            if (a.loglik == EVAL_LL_GAUSSIAN) ll = -0.5 * (ln + d * d * inu);
             else if (a.loglik == EVAL_LL_POISSON) ll = eval_loglik(EVAL_LL_POISSON, y, mu, nu2);
 #pragma unroll
             for (int c = 0; c < EVAL_MAX_CLASSES; ++c) {
@@ -141,7 +144,7 @@ __global__ void __launch_bounds__(256, KMAX <= 16 ? 2 : 1) eval_update_kernel(Ev
                     if (mu > bv[u]) a.below[o] = mu;
                 } else if (mu == y) a.c_le[o] = lev[u] + 1;
                 else if (mu < av[u]) a.above[o] = mu;
-                if (a.cdf) a.cdf[o] = fv[u] + 0.5 * erfc(-(d * inv_sd) * 0.70710678118654752440);
+                if (a.cdf) a.cdf[o] = fv[u] + 0.5 * erfc(-(d * isd) * 0.70710678118654752440);
             }
         }
     }
@@ -223,7 +226,7 @@ __global__ void __launch_bounds__(256) eval_summary_kernel(EvalArgs a, double lo
         if (cl >= a.ncls) continue;
         const double mean = a.mean[o];
         const double d = y - mean;
-        const double ll = eval_loglik(a.loglik, y, mean, nu2);
+        const double ll = eval_loglik(a.loglik, y, mean, a.nu2c ? a.nu2c[o] : nu2);
         const double c_lt = (double)a.c_lt[o], c_le = (double)a.c_le[o];
         const bool tie = c_le > c_lt;
         // lower end: y >= Q(lo)

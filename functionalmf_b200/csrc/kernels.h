@@ -38,6 +38,11 @@ void launch_prereduce_gaussian(const double* Y, int rows, int P, int R, uint8_t*
 // Binomial: (Ysucc, Ntrials) [rows][P] -> obs u8, kappa = y - n/2, ntr = n (0 where missing)
 void launch_prereduce_binomial(const double* Y, const double* Nt, int rows, int P, uint8_t* obs,
                                double* kappa, double* ntr, long long ld, cudaStream_t st);
+// Known per-cell noise variances nu2 [rows][P] at pitch `lds` -> f64 weights w = cnt / nu2 and s = S / nu2 at pitch `ld`
+// (0 where cnt = 0 or nu2 = +inf); `keep` (optional) receives nu2 at pitch `ld`; *nbad += # observed cells whose
+// variance is NaN or <= 0.
+void launch_nu2_weights(const double* nu2, long long lds, int rows, int P, const uint8_t* cnt, const double* S,
+                        long long ld, double* keep, double* w, double* s, unsigned long long* nbad, cudaStream_t st);
 // dst[0] += sum(src[0..n) step stride) in a fixed order (single block)
 void launch_reduce_add(const double* src, int n, int stride, double* dst, cudaStream_t st);
 
@@ -137,6 +142,7 @@ struct EvalArgs {
     int transform, loglik;
     const double* Rdisp; int Rn, Rm, Rt;   // NB dispersion (EVAL_NB_MEAN)
     const Scalars* scal;                   // nu2 of the current sample (Gaussian log-likelihood / predictive cdf)
+    const double* nu2c;                    // [nloc][P] known per-cell variances used instead of scal->nu2, or nullptr
     double count;                          // samples seen including this one
     double *mean, *below, *above, *cdf;    // per-cell state, all nullptr when not kept (cdf optional)
     unsigned *c_lt, *c_le;

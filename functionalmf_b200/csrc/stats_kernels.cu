@@ -83,6 +83,40 @@ void launch_prereduce_binomial(const double* Y, const double* Nt, int rows, int 
     prereduce_binomial_kernel<<<nb, 256, 0, st>>>(Y, Nt, rows, P, obs, kappa, ntr, ld);
 }
 
+// Known per-cell noise variances (the reference's heteroskedastic Gaussian branch, factor.py:345-346 and 390-391
+// with an [N, M, T] nu2): weight w = cnt / nu2 and right-hand side S / nu2 of the statistics, both 0 where nothing is
+// observed or nu2 = +inf (such a cell counts as missing).  Observed cells whose variance is NaN or <= 0 are counted.
+__global__ void nu2_weights_kernel(const double* __restrict__ nu2, long long lds, int rows, int P,
+                                   const uint8_t* __restrict__ cnt, const double* __restrict__ S, long long ld,
+                                   double* __restrict__ keep, double* __restrict__ w, double* __restrict__ s,
+                                   unsigned long long* __restrict__ nbad) {
+    unsigned bad = 0;
+    long long total = (long long)rows * P;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total;
+         e += (long long)gridDim.x * blockDim.x) {
+        int i = (int)(e / P), p = (int)(e - (long long)i * P);
+        const double v = nu2[(long long)i * lds + p];
+        const long long o = (long long)i * ld + p;
+        const double c = (double)cnt[o];
+        const bool on = c > 0.0 && v < INFINITY;
+        bad += (c > 0.0 && !(v > 0.0)) ? 1u : 0u;
+        w[o] = on ? c / v : 0.0;
+        s[o] = on ? S[o] / v : 0.0;
+        if (keep) keep[o] = v;
+    }
+    for (int d = 16; d > 0; d >>= 1) bad += __shfl_down_sync(0xffffffffu, bad, d);
+    if ((threadIdx.x & 31) == 0 && bad) atomicAdd(nbad, (unsigned long long)bad);
+}
+
+void launch_nu2_weights(const double* nu2, long long lds, int rows, int P, const uint8_t* cnt, const double* S,
+                        long long ld, double* keep, double* w, double* s, unsigned long long* nbad, cudaStream_t st) {
+    long long total = (long long)rows * P;
+    int nb = (int)((total + 255) / 256);
+    if (nb > 148 * 16) nb = 148 * 16;
+    if (nb < 1) nb = 1;
+    nu2_weights_kernel<<<nb, 256, 0, st>>>(nu2, lds, rows, P, cnt, S, ld, keep, w, s, nbad);
+}
+
 __global__ void reduce_add_kernel(const double* __restrict__ src, int n, int stride, double* dst) {
     __shared__ double sh[32];
     double v = 0.0;

@@ -121,6 +121,15 @@ class Engine(object):
         Y = _f64(Y)
         L.check(self.lib.btf_set_data_negbin(self._h, _ptr(Y), Y.shape[3]))
 
+    def set_nu2_cells(self, nu2):
+        """Known per-cell noise variances [Nloc, M, T] of a Gaussian engine (``None``: back to the scalar nu2)."""
+        a = None
+        if nu2 is not None:
+            a = _f64(nu2)
+            if a.shape != (self.nloc, self.M, self.T):
+                raise ValueError('nu2 must be a [%d,%d,%d] tensor, got %s' % (self.nloc, self.M, self.T, a.shape))
+        L.check(self.lib.btf_set_nu2_cells(self._h, _ptr(a)))
+
     # ---- state
     def set(self, name, value):
         a = _f64(np.asarray(value, dtype=np.float64).reshape(-1))
@@ -185,6 +194,15 @@ class Engine(object):
                 raise ValueError('classes must have the local shape %r, got %r' % (shape, c.shape))
         L.check(self.lib.btf_eval_set(self._h, int(slot), _ptr(t), _ptr(c), int(nclasses), int(transform),
                                       int(loglik), int(cell_state), 1 if auto_update else 0, int(max_samples)))
+
+    def eval_set_nu2(self, slot, nu2):
+        """Per-cell variances [Nloc, M, T] for the Gaussian scores of an evaluator slot (``None``: the scalar nu2)."""
+        a = None
+        if nu2 is not None:
+            a = _f64(nu2)
+            if a.shape != (self.nloc, self.M, self.T):
+                raise ValueError('nu2 must have the local shape %r, got %r' % ((self.nloc, self.M, self.T), a.shape))
+        L.check(self.lib.btf_eval_set_nu2(self._h, int(slot), _ptr(a)))
 
     def eval_clear(self, slot):
         L.check(self.lib.btf_eval_clear(self._h, int(slot)))

@@ -13,7 +13,11 @@ Differences, all deliberate (SURVEY.md appendix D):
 * Cholesky retries are bounded and raise ``NotPositiveDefiniteError`` (Q4/Q5);
 * ``Tau2_init`` / ``Tau2_true`` still initialise ``Tau2_a/b/c`` from the prior (Q6);
 * ``lam2`` follows the reference as written (last column only, Q1) unless
-  ``ref_compat=False``.
+  ``ref_compat=False``;
+* with known per-cell noise variances (Gaussian ``nu2`` an [N, M, T] array held
+  fixed), ``run_gibbs`` returns ``results['nu2']`` as a read-only
+  ``np.broadcast_to`` view [nsamples, N, M, T] of that one array, not nsamples
+  copies.
 """
 import warnings
 import numpy as np
@@ -235,6 +239,10 @@ class BayesianTensorFiltering(_BayesianModel):
     def _scalar_names(self):
         return ['sigma2', 'lam2', 'lam2_a']
 
+    def _nu2_per_cell(self):
+        """The known per-cell noise variances [N, M, T] the next sweep uses, or None (GaussianBayesianTensorFiltering)."""
+        return None
+
     # ---- host <-> device coherence: the host attributes are authoritative between
     # calls (callers assign model.W[:] = ...), the device during a call
     def _push_state(self):
@@ -418,13 +426,23 @@ class BayesianTensorFiltering(_BayesianModel):
 
 
 class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
-    """factor.py:286-423."""
+    """factor.py:286-423.
+
+    ``nu2`` is a scalar, or an [N, M, T] array of known per-cell noise variances (the reference's heteroskedastic
+    branch, e.g. per-cell standard errors squared): when ``model.nu2`` has that shape and ``sample_nu2`` is False
+    (``nu2_true=array``), the W and V steps weight every cell by cnt / nu2[n, m, t].  A variance of +inf makes an
+    observed cell count as missing; NaN or <= 0 at an observed cell is refused.  With ``sample_nu2`` True the nu2
+    step draws a scalar from the residual like the reference's ``_resample_nu2``.  Single GPU only."""
     _likelihood = L.GAUSSIAN
 
     def __init__(self, nrows, ncols, ndepth, nu2_init=None, nu2_true=None, nu2_a=0.1, nu2_b=0.1, **kwargs):
         self.nu2_a, self.nu2_b = nu2_a, nu2_b
         self._nu2_args = (nu2_init, nu2_true)
+        self._nu2_key = None          # fingerprint of the per-cell variances on the device, None in scalar mode
         super().__init__(nrows, ncols, ndepth, **kwargs)
+        fixed = nu2_true if nu2_true is not None else nu2_init
+        if self._likelihood == L.GAUSSIAN and fixed is not None and np.size(fixed) != 1:
+            self.nu2 = np.asarray(fixed, dtype=np.float64)     # uploaded by the first sweep that uses it
 
     def _likelihood_options(self):
         return dict(nu2_a=self.nu2_a, nu2_b=self.nu2_b)
@@ -436,13 +454,37 @@ class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
 
     def _after_base_init(self):
         nu2_init, nu2_true = self._nu2_args
-        if nu2_true is not None:
-            self._engine.set('nu2', [nu2_true])
-        elif nu2_init is not None:
-            self._engine.set('nu2', [nu2_init])
+        fixed = nu2_true if nu2_true is not None else nu2_init
+        if fixed is None or (self._likelihood == L.GAUSSIAN and np.size(fixed) != 1):
+            return
+        self._engine.set('nu2', [fixed])
 
     def _scalar_names(self):
-        return ['sigma2', 'lam2', 'lam2_a', 'nu2']
+        names = ['sigma2', 'lam2', 'lam2_a']
+        return names if self._nu2_per_cell() is not None else names + ['nu2']
+
+    def _nu2_per_cell(self):
+        if self._likelihood != L.GAUSSIAN:
+            return None               # (the PG models' nu2 is the per-cell 1/omega they redraw every sweep)
+        nu2 = getattr(self, 'nu2', None)
+        if np.size(nu2) == 1:
+            return None
+        nu2 = np.asarray(nu2, dtype=np.float64)
+        shape = (self.nrows, self.ncols, self.ndepth)
+        if nu2.shape != shape:
+            raise ValueError('nu2 must be a scalar or an array of per-cell variances of shape %r, got %r'
+                             % (shape, nu2.shape))
+        return None if self.sample_nu2 else nu2
+
+    def _push_state(self):
+        super()._push_state()
+        cells = self._nu2_per_cell()
+        # re-uploaded only when the variances changed (same rule as the data, see _fingerprint)
+        key = None if cells is None else self._fingerprint(cells, getattr(self, '_full_check', False))
+        if key != self._nu2_key:
+            self._nu2_key = None      # the engine is in scalar mode after a refused upload
+            self._engine.set_nu2_cells(None if cells is None else self._local_rows(cells))
+            self._nu2_key = key
 
     def _upload(self, data):
         Y = np.asarray(data)
@@ -459,7 +501,11 @@ class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
 
     def _finish_results(self, results):
         results = super()._finish_results(results)
-        results['nu2'] = results.pop('_nu2_scalar')
+        nu2 = results.pop('_nu2_scalar')
+        cells = self._nu2_per_cell()
+        if cells is not None:
+            nu2 = np.broadcast_to(cells, (nu2.shape[0],) + cells.shape)
+        results['nu2'] = nu2
         return results
 
     def _inferred_variables(self, var_map):

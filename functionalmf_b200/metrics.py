@@ -86,6 +86,9 @@ class HeldOutEvaluator(object):
         self.model._engine.eval_set(self.slot, self._target, self._classes, self.nclasses,
                                     TRANSFORMS[self.transform], LOGLIKS[self.loglik_kind], self._cell_state,
                                     auto_update=True, max_samples=max(int(nsamples), 1))
+        cells = self.model._nu2_per_cell()
+        if cells is not None:        # known per-cell variances: the Gaussian scores use them, not the scalar nu2
+            self.model._engine.eval_set_nu2(self.slot, self.model._local_rows(cells))
         self._armed = True
 
     def update(self):

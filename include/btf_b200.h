@@ -87,6 +87,17 @@ int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int
                                int32_t reset);
 int btf_set_data_binomial(btf_engine* e, const double* Ysucc, const double* Ntrials);
 int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps);
+/* Known per-cell noise variances of a Gaussian model: the reference's heteroskedastic branch, nu2 an
+ * [N, M, T] array (factor.py:345-346, 390-391; SURVEY.md 3.2).  `nu2` holds the LOCAL rows [Nloc, M, T] in
+ * C order, host or device memory; NULL returns to the scalar nu2.  The W and V conditionals then weight
+ * cell (i,j,t) by cnt / nu2[i,j,t] with right-hand side S / nu2[i,j,t]; nu2 = +inf makes an observed cell
+ * count as missing, and at missing cells any value is accepted.  The weights are formed again after every
+ * btf_set_data_gaussian*; the variances are kept on the device (24 B per cell with the two weight buffers).
+ * BTF_ESTATE on a non-Gaussian engine, BTF_EINVAL on a sharded one (world_size > 1) and when observed
+ * cells have a variance that is NaN or <= 0 (the message gives their number; the engine stays in scalar
+ * mode).  While the variances are set, btf_sweep / btf_run* refuse BTF_SAMPLE_NU2 with BTF_ESTATE: the
+ * reference holds an array nu2 fixed. */
+int btf_set_nu2_cells(btf_engine* e, const double* nu2);
 
 /* ---- state: names "W" [N,K] (global), "V" [M,T,K], "Tau2","Tau2_a","Tau2_b",
  * "Tau2_c" [M,R_D], "lam2","lam2_a","sigma2","nu2" [1], "omega" [Nloc,M,T]
@@ -133,6 +144,11 @@ int btf_mu_stats_get(btf_engine* e, double* mean_out, double* var_out, int64_t* 
  * Up to 4 evaluators (slots 0..3) per engine.  Sums are over the LOCAL rows; ranks add them up. */
 int btf_eval_set(btf_engine* e, int32_t slot, const double* target, const uint8_t* cls, int32_t nclasses,
                  int32_t transform, int32_t loglik, int32_t cell_state, int32_t auto_update, int64_t max_samples);
+/* Per-cell variances [Nloc, M, T] of the slot's cells (host or device memory; NULL: back to the sample's
+ * scalar nu2): the Gaussian log-likelihood per sample and of the posterior mean, and the predictive band,
+ * then use nu2[cell], as the reference's heteroskedastic branch scores a model fitted with known
+ * variances (see btf_set_nu2_cells).  Call after btf_eval_set, which clears them. */
+int btf_eval_set_nu2(btf_engine* e, int32_t slot, const double* nu2);
 int btf_eval_clear(btf_engine* e, int32_t slot);
 int btf_eval_update(btf_engine* e, int32_t slot);
 /* out [count, nclasses, 4] = {n, sum (y-mu)^2, sum |y-mu|, sum loglik} per scored sample */
