@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('BTF_B200_LIB') or os.path.join(_HERE, 'libbtf_b200.so')
 
 BTF_OK, BTF_EINVAL, BTF_ECUDA, BTF_ENOTPD, BTF_ESTATE, BTF_ENCCL = 0, -1, -2, -3, -4, -5
-GAUSSIAN, BINOMIAL, NEGBINOMIAL = 0, 1, 2
+GAUSSIAN, BINOMIAL, NEGBINOMIAL, POISSON = 0, 1, 2, 3
 SAMPLE_NU2, SAMPLE_SIGMA2, SAMPLE_TAU2, SAMPLE_LAM2, SAMPLE_W, SAMPLE_V, SAMPLE_R = 1, 2, 4, 8, 16, 32, 64
 SAMPLE_ALL = 127
 I8_ROUTE_FUSED, I8_ROUTE_SPLITK = 2, 3     # btf_get_diag("i8_route")
@@ -69,6 +69,9 @@ SIGNATURES = {
     'btf_set_data_binomial': (C.c_int, [_P, _P, _P]),
     'btf_set_data_negbin': (C.c_int, [_P, _P, C.c_int32]),
     'btf_set_nu2_cells': (C.c_int, [_P, _P]),
+    'btf_set_data_poisson': (C.c_int, [_P, _P, C.c_int32]),
+    'btf_set_gass': (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, C.c_int32, _P, C.c_int32]),
+    'btf_set_ep': (C.c_int, [_P, _P, _P]),
     'btf_set_state': (C.c_int, [_P, C.c_char_p, _P, C.c_size_t]),
     'btf_get_state': (C.c_int, [_P, C.c_char_p, _P, C.c_size_t]),
     'btf_delta_rows': (C.c_int, [_P]),

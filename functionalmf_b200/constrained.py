@@ -14,16 +14,24 @@ engine in ONE batched launch per step instead of per-row / per-column Python + C
   v_j = L_j^-T z_j for all columns at once;
 * sigma2 / Tau2 / lam2 steps (factor.py:130-153) run on the device as for the conjugate models.
 
+``loglikelihood='poisson'`` selects the built-in Poisson likelihood of examples/poisson_tensor_filtering.py
+(``nansum(poisson.logpmf(Y, W V^T))`` over the replicates).  Then the whole sweep -- sigma2, Tau2, lam2, the W and V
+centres and proposals, and one GASS transition per row and per column -- runs inside the engine (gass_kernels.cu), so
+``run_gibbs`` runs in ``btf_run_segment`` pieces (or a CUDA graph) and ``HeldOutEvaluator``, ``track_mu``,
+``results_dir`` and checkpoints work as for the conjugate models.  Its random choices are Philox draws of the engine,
+not ``np.random``.  Single GPU.
+
 ``nthreads``, ``multiprocessing``, ``sharedprefix`` are accepted and ignored (there is no worker
 pool to manage: rows and columns are batched on the GPU); ``shutdown()`` is a no-op kept for
 drop-in compatibility.
 """
+import warnings
 import numpy as np
-from scipy.stats import norm
+from scipy.stats import norm, poisson
 
 from . import _lib as L
-from .factor import BayesianTensorFiltering
-from .gass import gass
+from .factor import BayesianTensorFiltering, _BayesianModel
+from .gass import gass, FINE_GRID
 
 
 class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
@@ -33,6 +41,11 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
     def __init__(self, nrows, ncols, ndepth, loglikelihood, Constraints, ep_approx=None, nthreads=3,
                  gass_ngrid=100, Row_constraints=None, multiprocessing=True, sharedprefix=None,
                  worker_init=None, **kwargs):
+        self._poisson = isinstance(loglikelihood, str)
+        if self._poisson:
+            if loglikelihood != 'poisson':
+                raise ValueError("loglikelihood must be a callable or 'poisson', got %r" % (loglikelihood,))
+            self._likelihood = L.POISSON
         self.loglikelihood = loglikelihood
         Constraints = np.asarray(Constraints, dtype=float)
         self.Constraints_A, self.Constraints_C = Constraints[:, :-1], Constraints[:, -1:]
@@ -45,6 +58,7 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
         else:
             self.Mu_ep, self.Sigma_ep = ep_approx
         self._ep_key = None
+        self._gass_key = None
         self._rng = np.random            # slice heights / grid choices: the reference's global stream
         super().__init__(nrows, ncols, ndepth, **kwargs)
         if worker_init is not None:
@@ -62,6 +76,15 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
     def _sync_ep(self):
         N, M, T = self.nrows, self.ncols, self.ndepth
         key = None if self.Mu_ep is None else (self._fingerprint(self.Mu_ep), self._fingerprint(self.Sigma_ep))
+        if self._poisson:
+            if key != self._ep_key:
+                self._ep_key = None
+                if self.Mu_ep is None:
+                    self._engine.set_ep(None, None)
+                else:
+                    self._engine.set_ep(np.asarray(self.Mu_ep, dtype=float), np.asarray(self.Sigma_ep, dtype=float))
+                self._ep_key = key
+            return
         if key == self._ep_key and self._omega is not None:
             return
         if self.Mu_ep is None:
@@ -79,7 +102,29 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     _omega = None
 
+    def _sync_gass(self):
+        """Constraints, row constraints and the angle grids of the device GASS steps (re-sent when they change)."""
+        R = self.Row_constraints
+        key = (int(self.gass_ngrid), self._fingerprint(self.Constraints_A), self._fingerprint(self.Constraints_C),
+               None if R is None else self._fingerprint(R))
+        if key == self._gass_key:
+            return
+        self._gass_key = None
+        self._engine.set_gass(self.Constraints_A, self.Constraints_C[:, 0], np.linspace(-np.pi, np.pi, FINE_GRID),
+                              np.linspace(-np.pi, np.pi, int(self.gass_ngrid)), rowcons=R)
+        self._gass_key = key
+
     def _upload(self, data):
+        if self._poisson:
+            Y = np.asarray(data)
+            assert Y.ndim in (3, 4), 'Observations must be a 3- or 4-tensor.'
+            key = self._fingerprint(data, getattr(self, '_full_check', False))
+            self._data_nbytes = int(Y.nbytes)
+            if key != self._data_key:
+                self._data_key = None
+                self._engine.set_data_poisson(Y)
+                self._data_key = key
+            self._sync_gass()
         self._sync_ep()
 
     def _scalar_names(self):
@@ -112,6 +157,8 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     def resample(self, data, **kwargs):
         '''One sweep: sigma2, Tau2, lam2 (device), then GASS for W and V (factor.py:112-128).'''
+        if self._poisson:
+            return BayesianTensorFiltering.resample(self, data, **kwargs)
         self._sync_ep()
         self._device_hyper_step()
         if self.sample_W:
@@ -121,6 +168,9 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     def run_gibbs(self, data, nburn=1000, nthin=1, nsamples=1000, verbose=True, print_freq=100,
                   callback=None, **kwargs):
+        if self._poisson:
+            return _BayesianModel.run_gibbs(self, data, nburn=nburn, nthin=nthin, nsamples=nsamples, verbose=verbose,
+                                            print_freq=print_freq, callback=callback, **kwargs)
         # the likelihood is a Python callback: always the per-sweep path of genlasso.py:37-66
         cb = callback if callback is not None else (lambda *a, **k: None)
         return self._run_gibbs_callback(data, nburn, nthin, nsamples, verbose, print_freq, cb, **kwargs)
@@ -202,8 +252,20 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
                          ngrid=self.gass_ngrid, rng=self._rng)
             self.V[j] = xn.reshape((self.nembeds, self.ndepth)).T
 
+    def _finish_results(self, results):
+        results = super()._finish_results(results)
+        results.pop('_nu2_scalar')
+        return results
+
     def logprob(self, data, **kwargs):
         tau = (self.W[:, None, None] * self.V[None]).sum(axis=-1)
+        if self._poisson:
+            Y = np.asarray(data)
+            if Y.ndim > tau.ndim:
+                tau = tau[..., None]
+            with warnings.catch_warnings():
+                warnings.simplefilter('ignore', category=RuntimeWarning)
+                return np.nansum(poisson.logpmf(Y, tau))
         return self.loglikelihood(data, tau, self.W, self.V)
 
 
@@ -215,6 +277,8 @@ class NonconjugateBayesianTensorFiltering(ConstrainedNonconjugateBayesianTensorF
     the slice sampling itself and the likelihood callback stay on the host as in the reference."""
 
     def __init__(self, nrows, ncols, ndepth, loglikelihood, **kwargs):
+        if isinstance(loglikelihood, str):
+            raise ValueError('NonconjugateBayesianTensorFiltering takes a callable loglikelihood(W, V, data)')
         no_constraints = np.zeros((0, ndepth + 1))
         super().__init__(nrows, ncols, ndepth, loglikelihood, no_constraints, **kwargs)
 

@@ -6,7 +6,7 @@ OUT="$HERE/../libbtf_b200.so"
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-std=c++17 -O3 -lineinfo -gencode arch=compute_100a,code=sm_100a -Xcompiler -fPIC -Xptxas -v"
 mkdir -p "$HERE/_obj"
-SRCS="engine stats_kernels stats_zpre solve_kernels band_lookahead hyper_kernels pg_kernels eval_kernels i8gemm2 stats_i8 nccl_shard peaks"
+SRCS="engine stats_kernels stats_zpre solve_kernels band_lookahead hyper_kernels pg_kernels gass_kernels eval_kernels i8gemm2 stats_i8 nccl_shard peaks"
 pids=()
 for f in $SRCS; do
   ( $NVCC $FLAGS -c "$HERE/$f.cu" -o "$HERE/_obj/$f.o" > "$HERE/_obj/$f.log" 2>&1 || { cat "$HERE/_obj/$f.log"; exit 1; } ) &

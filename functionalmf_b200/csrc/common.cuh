@@ -30,7 +30,7 @@ struct Scalars {
 // RNG stream identifiers (mixed into the Philox key)
 enum Stream : uint32_t {
     STREAM_W = 1, STREAM_V = 2, STREAM_TAU = 3, STREAM_LAM = 4, STREAM_SIGMA = 5,
-    STREAM_NU = 6, STREAM_PG = 7, STREAM_R = 8
+    STREAM_NU = 6, STREAM_PG = 7, STREAM_R = 8, STREAM_GASS_W = 9, STREAM_GASS_V = 10
 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {

@@ -96,6 +96,15 @@ struct btf_engine {
     double *nu2c = nullptr, *wc = nullptr, *sc = nullptr;      // [nloc_pad][Ppad], allocated on first use
     unsigned long long* nu2_nbad = nullptr;
     StatsPlan plan_row_w{}, plan_col_w{};                      // statistics plans for those f64 weights
+    // Poisson model (constrained GASS steps, gass_kernels.cu; single GPU).  With an EP approximation the W / V centres
+    // come from the f64-weight statistics of wc = 1 / sigma^2 and sc = mu / sigma^2 (the buffers of the per-cell nu2 mode)
+    bool gass_set = false, ep_on = false;
+    int gJ = 0, gnrc = 0, gnfine = 0, gngrid = 0;
+    double *gA = nullptr, *gC = nullptr, *growc = nullptr, *ggrid_f = nullptr, *ggrid_c = nullptr;
+    double *Wold = nullptr, *Vold = nullptr, *gmeanW = nullptr, *gmeanV = nullptr;   // the state before the step, the centres
+    double *ep_mu = nullptr, *ep_sig = nullptr;                // [nloc_pad][Ppad]
+    double* lgy = nullptr;                                     // [nloc_pad][Ppad] sum of lgamma(y + 1) over the observed replicates
+    int* gass_nbad = nullptr;                                  // [2] rows / columns whose starting point violates a constraint
     int nreps = 1;
     bool has_data = false, data_reduced = false;
     double* staging[2] = {nullptr, nullptr};   // upload staging (kept for the engine's lifetime: no malloc/free per call, no leak on error paths)
@@ -262,6 +271,8 @@ int btf_create(const btf_config* c, btf_engine** out) {
     if (c->nembeds < 1 || c->nembeds > 32) return set_err(BTF_EINVAL, "nembeds must be in [1, 32]");
     if (c->tf_order < 0 || c->tf_order > 3) return set_err(BTF_EINVAL, "tf_order must be in [0, 3]");
     if (c->ndepth < c->tf_order + 2) return set_err(BTF_EINVAL, "ndepth must be >= tf_order + 2");
+    if (c->likelihood < BTF_GAUSSIAN || c->likelihood > BTF_POISSON) return set_err(BTF_EINVAL, "unknown likelihood %d", c->likelihood);
+    if (c->likelihood == BTF_POISSON && c->world_size > 1) return set_err(BTF_EINVAL, "the Poisson model is single-GPU");
     btf_engine* e = new btf_engine();
     // every early return below releases what has been created so far (streams, events, device buffers)
     struct Guard { btf_engine* e; ~Guard() { if (e) btf_destroy(e); } } guard{e};
@@ -366,8 +377,8 @@ int btf_create(const btf_config* c, btf_engine** out) {
     const size_t cells = (size_t)e->nloc_pad * e->Ppad;
     CK(dev_alloc(&e->cnt, cells));
     CK(dev_alloc(&e->S, cells));
-    const bool pg = c->likelihood != BTF_GAUSSIAN;
-    if (pg) { CK(dev_alloc(&e->ntr, cells)); CK(dev_alloc(&e->omega, cells)); }
+    const bool pg = c->likelihood != BTF_GAUSSIAN;      // f64 weights in the statistics (Poisson: the EP weights)
+    if (c->likelihood == BTF_BINOMIAL || c->likelihood == BTF_NEGBINOMIAL) { CK(dev_alloc(&e->ntr, cells)); CK(dev_alloc(&e->omega, cells)); }
     if (c->likelihood == BTF_NEGBINOMIAL) {
         e->Rn = (c->rdims_mask & 1) ? 1 : e->N;
         e->Rm = (c->rdims_mask & 2) ? 1 : e->M;
@@ -445,7 +456,9 @@ void btf_destroy(btf_engine* e) {
     void* ptrs[] = {e->W, e->V, e->Tau2, e->Tau2_a, e->Tau2_b, e->Tau2_c, e->scal, e->cnt, e->S, e->ntr, e->omega,
                     e->Yraw, e->Rdisp, e->nb_work, e->nb_hist, e->d_start, e->d_width, e->d_coef, e->pm_ptr, e->pm_row, e->pm_coef,
                     e->row_stats, e->col_stats, e->zbuf, e->mu_mean, e->mu_m2, e->work_L, e->work_y, e->partials, e->lam_partials, e->resid_partials,
-                    e->snapW, e->snapV, e->snapTau2, e->snapScal, e->snapR, e->diag_retries, e->nu2c, e->wc, e->sc, e->nu2_nbad};
+                    e->snapW, e->snapV, e->snapTau2, e->snapScal, e->snapR, e->diag_retries, e->nu2c, e->wc, e->sc, e->nu2_nbad,
+                    e->gA, e->gC, e->growc, e->ggrid_f, e->ggrid_c, e->Wold, e->Vold, e->gmeanW, e->gmeanV, e->ep_mu, e->ep_sig,
+                    e->gass_nbad, e->lgy};
     for (void* p : ptrs) if (p) cudaFree(p);
     {
         void* i8p[] = {e->i8.planes, e->i8.colmax, e->i8.expo, e->i8.D, e->i8.bpart, e->cntT, e->cnt_rowsum, e->cnt_colsum, e->guard_n, e->guard_flags, e->Scol};
@@ -525,10 +538,17 @@ static void parallel_memcpy(void* dst, const void* src, size_t bytes, int thread
 
 // Pre-reduce `nrows` local rows starting at local row `row0` (streaming form for shards that
 // are generated or loaded piecewise; reset != 0 clears the running totals first).
+static int set_data_compact(btf_engine* e, const double* Y, int32_t row0, int32_t nrows, int32_t nreps, int32_t reset);
+
 int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int32_t nrows, int32_t nreps,
                                int32_t reset) {
     if (!e || !Y || nreps < 1 || nreps > 255) return set_err(BTF_EINVAL, "bad arguments (1 <= nreps <= 255)");
     if (e->cfg.likelihood != BTF_GAUSSIAN) return set_err(BTF_ESTATE, "engine is not Gaussian");
+    return set_data_compact(e, Y, row0, nrows, nreps, reset);
+}
+
+// the compact form of replicated observations (K0): # observed replicates (u8) and their sum per cell
+static int set_data_compact(btf_engine* e, const double* Y, int32_t row0, int32_t nrows, int32_t nreps, int32_t reset) {
     if (row0 < 0 || nrows < 0 || row0 + nrows > e->nloc) return set_err(BTF_EINVAL, "row range outside the shard");
     if (!reset && e->shard && e->data_reduced)
         return set_err(BTF_ESTATE, "a sharded engine that has already run holds all-reduced totals: restart the upload with reset = 1");
@@ -602,6 +622,39 @@ int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int
 int btf_set_data_gaussian(btf_engine* e, const double* Y, int32_t nreps) {
     if (!e) return set_err(BTF_EINVAL, "null engine");
     return btf_set_data_gaussian_rows(e, Y, 0, e->nloc, nreps, 1);
+}
+
+static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host);
+
+// Poisson counts [Nloc, M, T, nreps] in the compact form of the Gaussian data, plus sum_r lgamma(y_r + 1) per cell
+// (scipy's logpmf keeps it, and a cell whose rate is negative drops out of the log-likelihood together with it).
+// Every observed value must be a non-negative integer.
+int btf_set_data_poisson(btf_engine* e, const double* Y, int32_t nreps) {
+    if (!e || !Y || nreps < 1 || nreps > 255) return set_err(BTF_EINVAL, "bad arguments (1 <= nreps <= 255)");
+    if (e->cfg.likelihood != BTF_POISSON) return set_err(BTF_ESTATE, "engine is not Poisson");
+    CK(cudaSetDevice(e->cfg.device));
+    const size_t cells = (size_t)e->nloc * e->P, total = cells * nreps;
+    std::vector<double> hcopy;
+    const double* hy = Y;
+    if (is_device_ptr(Y)) {
+        hcopy.resize(total);
+        CK(cudaMemcpy(hcopy.data(), Y, total * sizeof(double), cudaMemcpyDeviceToHost));
+        hy = hcopy.data();
+    }
+    unsigned long long nbad = 0;
+    std::vector<double> lg(cells, 0.0);
+    for (size_t c = 0; c < cells; ++c)
+        for (int r = 0; r < nreps; ++r) {
+            const double y = hy[c * nreps + r];
+            if (std::isnan(y)) continue;
+            if (!(y >= 0.0 && std::isfinite(y) && y == std::floor(y))) ++nbad;
+            else lg[c] += std::lgamma(y + 1.0);
+        }
+    if (nbad) return set_err(BTF_EINVAL, "%llu observed value(s) are not non-negative integer counts", nbad);
+    if (!e->lgy) CK(dev_alloc(&e->lgy, (size_t)e->nloc_pad * e->Ppad));
+    CK(cudaStreamSynchronize(e->stream));
+    { int rc = copy_pitched(e, e->lgy, lg.data(), false); if (rc) return rc; }
+    return set_data_compact(e, Y, 0, e->nloc, nreps, 1);
 }
 
 int btf_set_data_binomial(btf_engine* e, const double* Ys, const double* Nt) {
@@ -770,6 +823,101 @@ int btf_set_nu2_cells(btf_engine* e, const double* nu2) {
     return BTF_OK;
 }
 
+// pitched [nloc][P] <-> dense copies for omega / Ntrials / the EP approximation
+static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host) {
+    if (to_host)
+        CK(cudaMemcpy2D(host, (size_t)e->P * 8, dev, (size_t)e->Ppad * 8, (size_t)e->P * 8, e->nloc, cudaMemcpyDeviceToHost));
+    else
+        CK(cudaMemcpy2D(dev, (size_t)e->Ppad * 8, host, (size_t)e->P * 8, (size_t)e->P * 8, e->nloc, cudaMemcpyHostToDevice));
+    return BTF_OK;
+}
+
+// ------------------------------------------------------------------ constrained Poisson model (GASS steps)
+static cudaError_t upload_copy(double** dst, const double* src, size_t n) {
+    if (*dst) { cudaFree(*dst); *dst = nullptr; }
+    cudaError_t ce = dev_alloc(dst, std::max<size_t>(n, 1), false);
+    if (ce == cudaSuccess && n) ce = h2d(*dst, src, n * sizeof(double));
+    return ce;
+}
+
+int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, const double* rowcons, int32_t nrowcons,
+                 const double* grid_fine, int32_t ngrid_fine, const double* grid_coarse, int32_t ngrid) {
+    if (!e) return set_err(BTF_EINVAL, "null engine");
+    if (e->cfg.likelihood != BTF_POISSON) return set_err(BTF_ESTATE, "GASS steps need a Poisson engine");
+    if (J < 0 || nrowcons < 0 || (J > 0 && (!A || !C)) || (nrowcons > 0 && !rowcons))
+        return set_err(BTF_EINVAL, "constraints: J >= 0 rows of A [J, T] and C [J], nrowcons >= 0 rows of [K + 1]");
+    if (!grid_fine || !grid_coarse || ngrid < 1 || ngrid > ngrid_fine || ngrid_fine > 65535)
+        return set_err(BTF_EINVAL, "grids: 1 <= ngrid <= ngrid_fine <= 65535 (got ngrid = %d, ngrid_fine = %d)", ngrid, ngrid_fine);
+    size_t nonfinite = 0;
+    for (size_t i = 0; i < (size_t)J * e->T; ++i) nonfinite += !std::isfinite(A[i]);
+    for (int i = 0; i < J; ++i) nonfinite += !std::isfinite(C[i]);
+    for (size_t i = 0; i < (size_t)nrowcons * (e->K + 1); ++i) nonfinite += !std::isfinite(rowcons[i]);
+    if (nonfinite) return set_err(BTF_EINVAL, "%zu constraint coefficient(s) are not finite", nonfinite);
+    for (int i = 0; i < ngrid_fine; ++i)
+        if (!std::isfinite(grid_fine[i]) || (i && !(grid_fine[i] >= grid_fine[i - 1]))) return set_err(BTF_EINVAL, "the fine grid must be finite and ascending");
+    for (int i = 0; i < ngrid; ++i)
+        if (!std::isfinite(grid_coarse[i])) return set_err(BTF_EINVAL, "the coarse grid must be finite");
+    cudaDeviceProp prop;
+    CK(cudaGetDeviceProperties(&prop, e->cfg.device));
+    const size_t smem = gass_smem_bytes(e->T * e->K, ngrid_fine, ngrid) + 1024;
+    if (smem > (size_t)prop.sharedMemPerBlockOptin)
+        return set_err(BTF_EINVAL, "GASS steps at T K = %d with %d grid points need %zu bytes of shared memory per block, the device offers %zu",
+                       e->T * e->K, ngrid_fine, smem, (size_t)prop.sharedMemPerBlockOptin);
+    CK(cudaSetDevice(e->cfg.device));
+    CK(cudaStreamSynchronize(e->stream));
+    free_graph(e);
+    e->gass_set = false;
+    CK(upload_copy(&e->gA, A, (size_t)J * e->T));
+    CK(upload_copy(&e->gC, C, (size_t)J));
+    CK(upload_copy(&e->growc, rowcons, (size_t)nrowcons * (e->K + 1)));
+    CK(upload_copy(&e->ggrid_f, grid_fine, (size_t)ngrid_fine));
+    CK(upload_copy(&e->ggrid_c, grid_coarse, (size_t)ngrid));
+    if (!e->Wold) {
+        CK(dev_alloc(&e->Wold, (size_t)e->N * e->K));
+        CK(dev_alloc(&e->Vold, (size_t)e->P * e->K));
+        CK(dev_alloc(&e->gmeanW, (size_t)e->N * e->K));
+        CK(dev_alloc(&e->gmeanV, (size_t)e->P * e->K));
+        CK(dev_alloc(&e->gass_nbad, 2));
+    }
+    e->gJ = J; e->gnrc = nrowcons; e->gnfine = ngrid_fine; e->gngrid = ngrid;
+    e->gass_set = true;
+    return BTF_OK;
+}
+
+// EP approximation N(mu, sigma^2) per cell (host memory, [Nloc, M, T]); NULL: none
+int btf_set_ep(btf_engine* e, const double* mu, const double* sigma) {
+    if (!e) return set_err(BTF_EINVAL, "null engine");
+    if (e->cfg.likelihood != BTF_POISSON) return set_err(BTF_ESTATE, "an EP approximation needs a Poisson engine");
+    CK(cudaSetDevice(e->cfg.device));
+    CK(cudaStreamSynchronize(e->stream));
+    if (!mu || !sigma) {
+        if (e->ep_on) free_graph(e);
+        e->ep_on = false;
+        return BTF_OK;
+    }
+    const size_t n = (size_t)e->nloc * e->P;
+    size_t nbad = 0;
+    for (size_t i = 0; i < n; ++i) nbad += !(std::isfinite(mu[i]) && std::isfinite(sigma[i]) && sigma[i] > 0.0);
+    if (nbad) return set_err(BTF_EINVAL, "%zu cell(s) of the EP approximation have a mean that is not finite or a scale that is not finite and > 0", nbad);
+    free_graph(e);
+    e->ep_on = false;
+    const size_t cells = (size_t)e->nloc_pad * e->Ppad;
+    if (!e->ep_mu) {
+        CK(dev_alloc(&e->ep_mu, cells)); CK(dev_alloc(&e->ep_sig, cells));
+        CK(dev_alloc(&e->wc, cells)); CK(dev_alloc(&e->sc, cells));
+    }
+    // the statistics' weights as numpy forms them: w = 1 / sigma**2, s = mu * w
+    std::vector<double> w(n), s(n);
+    for (size_t i = 0; i < n; ++i) { w[i] = 1.0 / (sigma[i] * sigma[i]); s[i] = mu[i] * w[i]; }
+    { int rc = copy_pitched(e, e->ep_mu, const_cast<double*>(mu), false); if (rc) return rc; }
+    { int rc = copy_pitched(e, e->ep_sig, const_cast<double*>(sigma), false); if (rc) return rc; }
+    { int rc = copy_pitched(e, e->wc, w.data(), false); if (rc) return rc; }
+    { int rc = copy_pitched(e, e->sc, s.data(), false); if (rc) return rc; }
+    CK(cudaStreamSynchronize(cudaStreamLegacy));
+    e->ep_on = true;
+    return BTF_OK;
+}
+
 // ------------------------------------------------------------------ state
 struct StateRef { double* p; size_t n; bool scalar_field; };
 
@@ -792,15 +940,6 @@ static bool state_ref(btf_engine* e, const std::string& nm, StateRef* r) {
     if (nm == "ss_total") { r->p = &e->scal->ss_total; return true; }
     if (nm == "n_obs") { r->p = &e->scal->n_obs; return true; }
     return false;
-}
-
-// pitched [nloc][P] <-> dense copies for omega / Ntrials
-static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host) {
-    if (to_host)
-        CK(cudaMemcpy2D(host, (size_t)e->P * 8, dev, (size_t)e->Ppad * 8, (size_t)e->P * 8, e->nloc, cudaMemcpyDeviceToHost));
-    else
-        CK(cudaMemcpy2D(dev, (size_t)e->Ppad * 8, host, (size_t)e->P * 8, (size_t)e->P * 8, e->nloc, cudaMemcpyHostToDevice));
-    return BTF_OK;
 }
 
 int btf_set_state(btf_engine* e, const char* name, const double* host, size_t n) {
@@ -874,6 +1013,10 @@ int btf_inject_noise(btf_engine* e, const char* name, const double* host, size_t
     else if (nm == "g_sigma2" || nm == "g_nu2") want = 1;
     else if (nm == "omega") want = (size_t)e->nloc * e->P;
     else if (nm == "z_R" || nm == "u_R") want = (size_t)e->cfg.nmetropolis * rsize;
+    else if (nm == "gass_u_W" || nm == "gass_u_V") {
+        if (!e->gass_set) return set_err(BTF_ESTATE, "%s: call btf_set_gass first", name);
+        want = (size_t)(nm == "gass_u_W" ? e->N : e->M) * (e->gngrid + 2);
+    }
     else return set_err(BTF_EINVAL, "unknown noise '%s'", name);
     if (n != want) return set_err(BTF_EINVAL, "%s: expected %zu values, got %zu", name, want, n);
     DevBuf& b = e->inject[nm];
@@ -1215,6 +1358,47 @@ static int ensure_data_reduced(btf_engine* e) {
     return BTF_OK;
 }
 
+// The GASS step of the W rows (col = false) or V columns after their Gaussian draw (the old state is in Wold / Vold)
+static GassArgs gass_args(btf_engine* e, bool col) {
+    GassArgs g;
+    memset(&g, 0, sizeof(g));
+    g.col = col;
+    g.N = e->N; g.M = e->M; g.T = e->T; g.K = e->K; g.P = e->P; g.ld = e->Ppad;
+    g.cnt = e->cnt; g.S = e->S; g.lgy = e->lgy;
+    g.ep_mu = e->ep_on ? e->ep_mu : nullptr; g.ep_sig = e->ep_on ? e->ep_sig : nullptr;
+    g.A = e->gA; g.C = e->gC; g.J = e->gJ; g.rowcons = e->growc; g.nrc = e->gnrc;
+    g.grid_fine = e->ggrid_f; g.nfine = e->gnfine; g.grid_coarse = e->ggrid_c; g.ngrid = e->gngrid;
+    g.Wold = e->Wold; g.Vold = e->Vold; g.Wnew = e->W; g.Vnew = e->V;
+    g.Wcur = e->W; g.Vcur = e->V;
+    g.u_inject = inj(e, col ? "gass_u_V" : "gass_u_W");
+    g.scal = e->scal; g.seed = e->cfg.seed;
+    g.diag = diag_get(e, col ? "gass_V" : "gass_W", (size_t)(col ? e->M : e->N) * 3);
+    return g;
+}
+
+// The reference asserts that every GASS step starts from a feasible point ('Invalid starting point!'): count the rows and
+// columns whose current state violates a constraint before a sweep changes anything
+static int gass_check_start(btf_engine* e) {
+    const int mask = e->cfg.sample_mask;
+    if (!(mask & (BTF_SAMPLE_W | BTF_SAMPLE_V))) return BTF_OK;
+    cudaStream_t st = e->stream;
+    CK(cudaMemsetAsync(e->gass_nbad, 0, 2 * sizeof(int), st));
+    for (int col = 0; col < 2; ++col) {
+        if (!(mask & (col ? BTF_SAMPLE_V : BTF_SAMPLE_W))) continue;
+        GassArgs g = gass_args(e, col != 0);
+        g.Wold = e->W; g.Vold = e->V; g.u_inject = nullptr; g.diag = nullptr;
+        g.check_only = 1; g.nbad = e->gass_nbad + col;
+        launch_gass(g, st); e->launches++;
+    }
+    int h[2] = {0, 0};
+    CK(cudaMemcpyAsync(h, e->gass_nbad, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    if (h[0] || h[1])
+        return set_err(BTF_ESTATE, "invalid starting point: the state violates a constraint in %d row(s) and %d column(s)", h[0], h[1]);
+    return BTF_OK;
+}
+
 // Enqueue one resample(data) on e->stream.  Order: factor.py:306-311 (nu2 / omega),
 // then 112-128 (sigma2, Tau2, lam2, W, V); NB adds the R update first (494-511).
 static int enqueue_sweep(btf_engine* e) {
@@ -1262,7 +1446,7 @@ static int enqueue_sweep(btf_engine* e) {
             ScalarStepArgs sa{e->scal, c.seed, c.nu2_a, c.nu2_b, inj(e, "g_nu2")};
             launch_nu2(sa, st); e->launches++;
         }
-    } else if ((mask & BTF_SAMPLE_NU2) || inj(e, "omega")) {
+    } else if (e->omega && ((mask & BTF_SAMPLE_NU2) || inj(e, "omega"))) {
         const double* om = inj(e, "omega");
         if (om) {
             cudaMemcpy2DAsync(e->omega, (size_t)e->Ppad * 8, om, (size_t)e->P * 8, (size_t)e->P * 8, e->nloc,
@@ -1317,8 +1501,11 @@ static int enqueue_sweep(btf_engine* e) {
     }
     // ---- W | rest
     phase_mark(e, PH_ROW_STATS);
-    const void* wt = percell ? (const void*)e->wc : gauss ? (const void*)e->cnt : (const void*)e->omega;
-    const double* sv = percell ? e->sc : e->S;
+    // Poisson: the statistics of the EP approximation (weights 1 / sigma^2, right-hand side mu / sigma^2), none without it
+    const bool poisson = c.likelihood == BTF_POISSON;
+    const bool no_stats = poisson && !e->ep_on;
+    const void* wt = (percell || poisson) ? (const void*)e->wc : gauss ? (const void*)e->cnt : (const void*)e->omega;
+    const double* sv = (percell || poisson) ? e->sc : e->S;
     const bool wf64 = !homo;
     const StatsPlan& prow = stats_plan(e, false);
     const StatsPlan& pcol = stats_plan(e, true);
@@ -1326,13 +1513,13 @@ static int enqueue_sweep(btf_engine* e) {
         if (e->i8_on) {
             if (!fork) { int rc = begin_row_stats_i8(e, false, 0, &pend_row); if (rc) return rc; }
             { int rc = finish_row_stats_i8(e, fork, pend_row); if (rc) return rc; }
-        } else {
+        } else if (!no_stats) {
             launch_stats(prow, false, wf64, wt, sv, e->V, e->Ppad, e->Ppad, e->nloc, e->row_stats, e->zbuf, st);
             e->launches += prow.zpre ? 2 : 1;
         }
         phase_mark(e, PH_ROW_SOLVE);
         RowSolveArgs ra;
-        ra.stats = e->row_stats; ra.nsplit = e->i8_on ? 1 : prow.nsplit; ra.split_stride = prow.out_elems_per_split;
+        ra.stats = e->row_stats; ra.nsplit = no_stats ? 0 : e->i8_on ? 1 : prow.nsplit; ra.split_stride = prow.out_elems_per_split;
         ra.nloc = e->nloc; ra.row_begin = c.row_begin; ra.K = e->K;
         ra.scale_from_nu2 = homo ? &e->scal->nu2 : nullptr; ra.scal = e->scal; ra.W = e->W;
         ra.z_inject = inj(e, "z_W"); ra.seed = c.seed;
@@ -1340,7 +1527,17 @@ static int enqueue_sweep(btf_engine* e) {
         ra.diag_L = diag_get(e, "W_L", (size_t)e->N * e->K * e->K);
         ra.diag_mean = diag_get(e, "W_mean", (size_t)e->N * e->K);
         ra.diag_b = diag_get(e, "W_b", (size_t)e->N * e->K);
+        if (poisson) {
+            // GASS needs the old state and, with EP, the centre of the ellipse
+            CK(cudaMemcpyAsync(e->Wold, e->W, (size_t)e->N * e->K * 8, cudaMemcpyDeviceToDevice, st));
+            if (e->ep_on && !ra.diag_mean) ra.diag_mean = e->gmeanW;
+        }
         launch_row_solve(ra, nullptr, st); e->launches++;
+        if (poisson) {
+            GassArgs ga = gass_args(e, false);
+            ga.Wmean = e->ep_on ? ra.diag_mean : nullptr;
+            launch_gass(ga, st); e->launches++;
+        }
         e->resid_valid = false;
     } else {
         phase_mark(e, PH_ROW_SOLVE);
@@ -1366,18 +1563,33 @@ static int enqueue_sweep(btf_engine* e) {
         ba.diag_band = diag_get(e, "V_band", bn);
         ba.diag_chol = diag_get(e, "V_chol", bn);
         ba.diag_mean = diag_get(e, "V_mean", (size_t)e->P * e->K);
+        if (poisson && e->ep_on && !ba.diag_mean) ba.diag_mean = e->gmeanV;
         ba.diag_retries = e->diag_retries;
         ba.resid_partials = homo ? e->resid_partials + c.col_begin : nullptr;
-        auto band = [&]() { launch_band_solve(ba, st); e->launches++; };
+        auto band = [&]() {
+            if (poisson) CK(cudaMemcpyAsync(e->Vold, e->V, (size_t)e->P * e->K * 8, cudaMemcpyDeviceToDevice, st));
+            launch_band_solve(ba, st); e->launches++;
+            if (poisson) {
+                GassArgs ga = gass_args(e, true);
+                ga.Vmean = e->ep_on ? ba.diag_mean : nullptr;
+                launch_gass(ga, st); e->launches++;
+            }
+            return BTF_OK;
+        };
         if (e->i8_on) {
             e->col_collapsed = false;
             int rc = col_step_i8(e, fork, 1, band);
             if (rc) return rc;
         } else {
             int nsplit = pcol.nsplit;
-            launch_stats(pcol, true, wf64, wt, sv, e->W + (size_t)c.row_begin * e->K, e->nloc_pad, e->Ppad, e->P,
-                         e->col_stats, e->zbuf, st);
-            e->launches += pcol.zpre ? 2 : 1;
+            if (no_stats) {
+                ba.stats = nullptr;           // prior-only system
+                nsplit = 0;
+            } else {
+                launch_stats(pcol, true, wf64, wt, sv, e->W + (size_t)c.row_begin * e->K, e->nloc_pad, e->Ppad, e->P,
+                             e->col_stats, e->zbuf, st);
+                e->launches += pcol.zpre ? 2 : 1;
+            }
             if (e->shard) {
                 // FP64 statistics path across GPUs: partial statistics over the local rows for all columns, collapsed
                 // over the splits, then reduce-scattered by column block
@@ -1397,7 +1609,7 @@ static int enqueue_sweep(btf_engine* e) {
             }
             ba.nsplit = nsplit;
             phase_mark(e, PH_BAND_SOLVE);
-            if (e->Mloc > 0) band();
+            if (e->Mloc > 0) { int rc = band(); if (rc) return rc; }
         }
         phase_mark(e, PH_COMM);
         if (e->shard) {
@@ -1504,6 +1716,11 @@ static int pre_run(btf_engine* e) {
             e->nu2_dirty = false;
         }
         if (e->nu2_bad) return nu2_bad_error(e);
+    }
+    if (e->cfg.likelihood == BTF_POISSON) {
+        if (!e->gass_set) return set_err(BTF_ESTATE, "no constraints: call btf_set_gass first");
+        int rc = gass_check_start(e);
+        if (rc) return rc;
     }
     int rc = ensure_data_reduced(e);
     if (rc) return rc;

@@ -266,4 +266,27 @@ void launch_nb_hist(const NbArgs& a, int vstride, cudaStream_t st);
 // (factor.py:513-554, 494-511)
 void launch_nb_update(const NbArgs& a, cudaStream_t st);
 
+// ---------------------------------------------------------------- GASS steps of the constrained Poisson model (gass_kernels.cu)
+struct GassArgs {
+    bool col;                                   // false: one CTA per W row (gass_row_kernel), true: per V column (gass_col_kernel)
+    int N, M, T, K, P; long long ld;
+    const uint8_t* cnt; const double* S;        // observed replicates and their sum, [N][ld]
+    const double* lgy;                          // sum of lgamma(y + 1) over the observed replicates, [N][ld]
+    const double *ep_mu, *ep_sig;               // EP approximation [N][ld], or nullptr
+    const double* A; const double* C; int J;    // constraints A[c] . Mu[i, j, :] >= C[c], A [J][T]
+    const double* rowcons; int nrc;             // row constraints [nrc][K + 1] (W rows only)
+    const double* grid_fine; int nfine;         // ascending angle grids of the feasible set
+    const double* grid_coarse; int ngrid;
+    const double *Wold, *Vold;                  // the state x before the step
+    double *Wnew, *Vnew;                        // in: the Gaussian draw mu + v; out: the new state
+    const double *Wmean, *Vmean;                // the centre mu (nullptr: 0)
+    const double *Wcur, *Vcur;                  // the other factor (column step: W, row step: V)
+    const double* u_inject;                     // [rows or cols][ngrid + 2] uniforms, or nullptr (Philox)
+    const Scalars* scal; uint64_t seed;
+    double* diag;                               // [rows or cols][3] = (F, G, theta), or nullptr
+    int check_only; int* nbad;                  // 1: only count the rows / columns whose state violates a constraint
+};
+size_t gass_smem_bytes(int D, int nfine, int ngrid);
+void launch_gass(const GassArgs& a, cudaStream_t st);
+
 }  // namespace btf

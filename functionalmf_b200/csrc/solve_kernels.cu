@@ -91,10 +91,9 @@ __global__ void __launch_bounds__(128) row_solve_kernel(RowSolveArgs a) {
     }
     if (lane < d) {
         a.W[(size_t)i * K + lane] = xd;
-        if (a.diag_L) {
+        if (a.diag_L)
             for (int c = 0; c <= lane; ++c) a.diag_L[((size_t)i * K + lane) * K + c] = Lm[lane * KS + c];
-            a.diag_mean[(size_t)i * K + lane] = xm;
-        }
+        if (a.diag_mean) a.diag_mean[(size_t)i * K + lane] = xm;
     }
 }
 

@@ -130,6 +130,41 @@ class Engine(object):
                 raise ValueError('nu2 must be a [%d,%d,%d] tensor, got %s' % (self.nloc, self.M, self.T, a.shape))
         L.check(self.lib.btf_set_nu2_cells(self._h, _ptr(a)))
 
+    def set_data_poisson(self, Y):
+        """Counts [Nloc, M, T(, R)] of a Poisson engine (NaN = missing)."""
+        Y = np.asarray(Y)
+        if Y.ndim == 3:
+            Y = Y[..., None]
+        if Y.ndim != 4 or Y.shape[:3] != (self.nloc, self.M, self.T):
+            raise ValueError('Counts must be a [%d,%d,%d(,R)] tensor, got %s' % (self.nloc, self.M, self.T, Y.shape))
+        Y = _f64(Y)
+        L.check(self.lib.btf_set_data_poisson(self._h, _ptr(Y), Y.shape[3]))
+
+    def set_gass(self, A, C, grid_fine, grid_coarse, rowcons=None):
+        """Constraints A [J, T] tau >= C [J] on every cell's depth profile, optional row constraints [nrc, K + 1] on W,
+        and the fine / coarse angle grids of the GASS steps (len(grid_coarse) = ngrid candidates)."""
+        A = _f64(np.asarray(A, dtype=np.float64).reshape(-1, self.T))
+        C = _f64(np.asarray(C, dtype=np.float64).reshape(-1))
+        if C.shape[0] != A.shape[0]:
+            raise ValueError('A has %d rows, C has %d entries' % (A.shape[0], C.shape[0]))
+        R = None
+        if rowcons is not None:
+            R = _f64(np.asarray(rowcons, dtype=np.float64).reshape(-1, self.K + 1))
+        gf, gc = _f64(grid_fine), _f64(grid_coarse)
+        L.check(self.lib.btf_set_gass(self._h, _ptr(A), _ptr(C), A.shape[0], _ptr(R), 0 if R is None else R.shape[0],
+                                      _ptr(gf), gf.size, _ptr(gc), gc.size))
+
+    def set_ep(self, mu, sigma):
+        """EP approximation N(mu, sigma^2) per cell [Nloc, M, T] of a Poisson engine (``None``: none)."""
+        if mu is None:
+            L.check(self.lib.btf_set_ep(self._h, C.c_void_p(0), C.c_void_p(0)))
+            return
+        shape = (self.nloc, self.M, self.T)
+        m, s = _f64(mu), _f64(sigma)
+        if m.shape != shape or s.shape != shape:
+            raise ValueError('the EP approximation must be two %r tensors, got %r and %r' % (shape, m.shape, s.shape))
+        L.check(self.lib.btf_set_ep(self._h, _ptr(m), _ptr(s)))
+
     # ---- state
     def set(self, name, value):
         a = _f64(np.asarray(value, dtype=np.float64).reshape(-1))
@@ -243,7 +278,7 @@ class Engine(object):
             'W_Q': (N, K, K), 'W_L': (N, K, K), 'W_mean': (N, K), 'W_b': (N, K), 'V_mean': (M, T, K),
             'V_band': (self.Mloc, T * K, kd + 1), 'V_chol': (self.Mloc, T * K, kd + 1),
             'V_retries': (self.Mloc,), 'row_stats': (self.nloc, Lp + K), 'col_stats': (M * T, Lp + K),
-            'nu2_rate': (3,), 'lam2_rate': (2,), 'info': (3,), 'i8_guard': (2,), 'i8_route': (2,),
+            'gass_W': (N, 3), 'gass_V': (M, 3), 'nu2_rate': (3,), 'lam2_rate': (2,), 'info': (3,), 'i8_guard': (2,), 'i8_route': (2,),
         }
         a = np.empty(shapes[name], dtype=np.float64)
         L.check(self.lib.btf_get_diag(self._h, name.encode(), _ptr(a), a.size))

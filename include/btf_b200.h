@@ -30,7 +30,7 @@ extern "C" {
 #define BTF_ESTATE       -4   /* call order / missing data */
 #define BTF_ENCCL        -5   /* NCCL error */
 
-enum { BTF_GAUSSIAN = 0, BTF_BINOMIAL = 1, BTF_NEGBINOMIAL = 2 };
+enum { BTF_GAUSSIAN = 0, BTF_BINOMIAL = 1, BTF_NEGBINOMIAL = 2, BTF_POISSON = 3 };
 
 /* sample_mask bits: which variables resample() updates (factor.py:112-128, 306-311) */
 enum {
@@ -45,7 +45,7 @@ typedef struct btf_engine btf_engine;
 typedef struct btf_config {
     int32_t nrows, ncols, ndepth;      /* global N, M, T */
     int32_t nembeds, tf_order;         /* K, p */
-    int32_t likelihood;                /* BTF_GAUSSIAN / BINOMIAL / NEGBINOMIAL */
+    int32_t likelihood;                /* BTF_GAUSSIAN / BINOMIAL / NEGBINOMIAL / POISSON */
     double  sigma2_a, sigma2_b;        /* factor.py:27 */
     double  nu2_a, nu2_b;              /* factor.py:289 */
     double  stability;                 /* factor.py:32 */
@@ -98,6 +98,33 @@ int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps);
  * mode).  While the variances are set, btf_sweep / btf_run* refuse BTF_SAMPLE_NU2 with BTF_ESTATE: the
  * reference holds an array nu2 fixed. */
 int btf_set_nu2_cells(btf_engine* e, const double* nu2);
+
+/* ---- the constrained Poisson model (ConstrainedNonconjugateBayesianTensorFiltering with the Poisson likelihood of
+ * examples/poisson_tensor_filtering.py, factor.py:894-1017).  A BTF_POISSON engine runs the whole sweep on the device:
+ * sigma2, Tau2, lam2, then for W and for V the Gaussian centre and proposal (the f64-weight statistics of an EP
+ * approximation, or the prior alone) followed by one GASS transition per row / column (gass.py:13-130) under
+ * ll = nansum of scipy.stats.poisson.logpmf(y, lambda) over the observed replicates, lambda = W V^T (a cell with
+ * lambda < 0 is NaN there and drops out, lambda = 0 with y > 0 gives -inf), minus sum_cells norm.logpdf(lambda; mu_ep,
+ * sigma_ep) with EP.
+ * Single GPU: btf_create refuses world_size > 1 for this likelihood.
+ *
+ * Counts Y [Nloc, M, T, nreps] (NaN = missing, host or device memory), kept in the Gaussian data's compact form
+ * plus sum_r lgamma(y_r + 1) per cell (17 B / cell).  BTF_EINVAL when observed values are negative or not integers (the message gives their number). */
+int btf_set_data_poisson(btf_engine* e, const double* Y, int32_t nreps);
+/* Constraints and angle grids (host memory).  A [J, T], C [J]: every cell's depth profile tau = Mu[i, j, :] must satisfy
+ * A tau >= C (the Kronecker form of factor.py:711-721, 847-853 is never built); rowcons [nrowcons, K + 1] (may be NULL when
+ * nrowcons = 0): row i of W satisfies rowcons[:, :nd] w >= rowcons[:, K], nd = min(K, i + 1).  grid_fine (ascending,
+ * ngrid_fine <= 65535 points; gass.py uses linspace(-pi, pi, 10000)) is the grid the feasible angles are taken from;
+ * grid_coarse (ngrid points) is used instead when no constraint is active.  ngrid candidates at most are evaluated:
+ * 1 <= ngrid <= ngrid_fine.  Every btf_sweep / btf_run* first checks that the state satisfies the constraints
+ * ('Invalid starting point!' in the reference) and fails with BTF_ESTATE, giving the number of rows and columns in
+ * violation, before anything changes. */
+int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, const double* rowcons, int32_t nrowcons,
+                 const double* grid_fine, int32_t ngrid_fine, const double* grid_coarse, int32_t ngrid);
+/* EP approximation (host memory, [Nloc, M, T] each; NULL: none).  The W / V centres come from the weights 1 / sigma^2 and
+ * the right-hand side mu / sigma^2; every candidate's ll subtracts sum norm.logpdf(lambda; mu, sigma) over ALL cells of the
+ * row / column.  BTF_EINVAL when a mean is not finite or a scale is not finite and > 0 (with their number). 32 B / cell. */
+int btf_set_ep(btf_engine* e, const double* mu, const double* sigma);
 
 /* ---- state: names "W" [N,K] (global), "V" [M,T,K], "Tau2","Tau2_a","Tau2_b",
  * "Tau2_c" [M,R_D], "lam2","lam2_a","sigma2","nu2" [1], "omega" [Nloc,M,T]
@@ -172,7 +199,10 @@ int btf_sweep_timed(btf_engine* e, int32_t nsweeps, double* ms_out);
 /* ---- parity hooks.  Inject the noise the NEXT sweep consumes instead of the
  * Philox stream (cleared after that sweep): "z_W" [N,K], "z_V" [M,T,K] t-major,
  * "g_tau" [M,4,R_D], "g_lam" [2], "g_sigma2" [1], "g_nu2" [1] (standard gammas),
- * "omega" [Nloc,M,T], "z_R"/"u_R" [nmetropolis,*R.shape]. */
+ * "omega" [Nloc,M,T], "z_R"/"u_R" [nmetropolis,*R.shape],
+ * "gass_u_W" [N, ngrid+2], "gass_u_V" [M, ngrid+2] (Poisson: per row / column the slice uniform, ngrid thinning
+ * uniforms -- candidate k swaps position k with k + floor(u_k (F - k)) of the ascending feasible list when F > ngrid --
+ * and the pick uniform: candidate floor(u G) of the G at or above the slice). */
 int btf_inject_noise(btf_engine* e, const char* name, const double* host, size_t n);
 /* Diagnostics of the LAST sweep (enable with btf_enable_diag before it):
  * "W_Q","W_L" [N,K,K], "W_mean" [N,K], "W_b" [N,K], "V_mean" [M,T,K],
@@ -181,7 +211,9 @@ int btf_inject_noise(btf_engine* e, const char* name, const double* host, size_t
  * "nu2_rate" [3] = (a_post,b_post,n_obs), "lam2_rate" [2],
  * "i8_route" [2] = route of the last row / column product block of the integer
  * statistics path: 0 none yet, 2 2-CTA kernel with the fused epilogue, 3 2-CTA
- * kernel in split-K mode (recorded without btf_enable_diag). */
+ * kernel in split-K mode (recorded without btf_enable_diag),
+ * "gass_W" [N,3], "gass_V" [M,3] = (# feasible grid angles F, # candidates at or above the slice G, chosen angle;
+ * 0 when the state is kept). */
 int btf_enable_diag(btf_engine* e, int32_t on);
 int btf_get_diag(btf_engine* e, const char* name, double* host, size_t n);
 
