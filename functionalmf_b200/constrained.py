@@ -15,8 +15,11 @@ engine in ONE batched launch per step instead of per-row / per-column Python + C
 * sigma2 / Tau2 / lam2 steps (factor.py:130-153) run on the device as for the conjugate models.
 
 ``loglikelihood='poisson'`` selects the built-in Poisson likelihood of examples/poisson_tensor_filtering.py
-(``nansum(poisson.logpmf(Y, W V^T))`` over the replicates).  Then the whole sweep -- sigma2, Tau2, lam2, the W and V
-centres and proposals, and one GASS transition per row and per column -- runs inside the engine (gass_kernels.cu), so
+(``nansum(poisson.logpmf(Y, W V^T))`` over the replicates).  ``loglikelihood='binomial'`` selects the built-in Binomial
+likelihood of successes out of trials, ``data = (Y, Ntrials)``, whose success probability is the surface p = W V^T
+itself (``nansum(binom.logpmf(Y, Ntrials, W V^T))``; the constraints keep p in [0, 1] and give it its shape).  With
+either, the whole sweep -- sigma2, Tau2, lam2, the W and V centres and proposals, and one GASS transition per row and
+per column -- runs inside the engine (gass_kernels.cu), so
 ``run_gibbs`` runs in ``btf_run_segment`` pieces (or a CUDA graph) and ``HeldOutEvaluator``, ``track_mu``,
 ``results_dir`` and checkpoints work as for the conjugate models.  Its random choices are Philox draws of the engine,
 not ``np.random``.  Single GPU.
@@ -27,7 +30,7 @@ drop-in compatibility.
 """
 import warnings
 import numpy as np
-from scipy.stats import norm, poisson
+from scipy.stats import binom, norm, poisson
 
 from . import _lib as L
 from .factor import BayesianTensorFiltering, _BayesianModel
@@ -37,15 +40,17 @@ from .gass import gass, FINE_GRID
 class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
     # the engine runs in its f64-weight mode: weights = 1/Sigma_ep^2 are injected as "omega"
     _likelihood = L.BINOMIAL
+    # the built-in likelihoods, whose GASS steps run on the device
+    _BUILTIN = {'poisson': L.POISSON, 'binomial': L.CBINOMIAL}
 
     def __init__(self, nrows, ncols, ndepth, loglikelihood, Constraints, ep_approx=None, nthreads=3,
                  gass_ngrid=100, Row_constraints=None, multiprocessing=True, sharedprefix=None,
                  worker_init=None, **kwargs):
-        self._poisson = isinstance(loglikelihood, str)
-        if self._poisson:
-            if loglikelihood != 'poisson':
-                raise ValueError("loglikelihood must be a callable or 'poisson', got %r" % (loglikelihood,))
-            self._likelihood = L.POISSON
+        self._builtin = loglikelihood if isinstance(loglikelihood, str) else None
+        if self._builtin is not None:
+            if loglikelihood not in self._BUILTIN:
+                raise ValueError("loglikelihood must be a callable, 'poisson' or 'binomial', got %r" % (loglikelihood,))
+            self._likelihood = self._BUILTIN[loglikelihood]
         self.loglikelihood = loglikelihood
         Constraints = np.asarray(Constraints, dtype=float)
         self.Constraints_A, self.Constraints_C = Constraints[:, :-1], Constraints[:, -1:]
@@ -76,7 +81,7 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
     def _sync_ep(self):
         N, M, T = self.nrows, self.ncols, self.ndepth
         key = None if self.Mu_ep is None else (self._fingerprint(self.Mu_ep), self._fingerprint(self.Sigma_ep))
-        if self._poisson:
+        if self._builtin:
             if key != self._ep_key:
                 self._ep_key = None
                 if self.Mu_ep is None:
@@ -114,8 +119,27 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
                               np.linspace(-np.pi, np.pi, int(self.gass_ngrid)), rowcons=R)
         self._gass_key = key
 
+    def _binomial_data(self, data):
+        """(Y, Ntrials) of the built-in Binomial likelihood as two float arrays of the model's [N, M, T] shape."""
+        shape = (self.nrows, self.ncols, self.ndepth)
+        if isinstance(data, (tuple, list)) and len(data) == 2:
+            Y, Nt = np.asarray(data[0], dtype=float), np.asarray(data[1], dtype=float)
+            if Y.shape == shape and Nt.shape == shape:
+                return Y, Nt
+        raise ValueError("loglikelihood='binomial' takes the data as a tuple (Y, Ntrials) of two %r arrays" % (shape,))
+
     def _upload(self, data):
-        if self._poisson:
+        if self._builtin == 'binomial':
+            Y, Nt = self._binomial_data(data)
+            full = getattr(self, '_full_check', False)
+            key = (self._fingerprint(Y, full), self._fingerprint(Nt, full))
+            self._data_nbytes = int(Y.nbytes + Nt.nbytes)
+            if key != self._data_key:
+                self._data_key = None
+                self._engine.set_data_binomial(Y, Nt)
+                self._data_key = key
+            self._sync_gass()
+        elif self._builtin == 'poisson':
             Y = np.asarray(data)
             assert Y.ndim in (3, 4), 'Observations must be a 3- or 4-tensor.'
             key = self._fingerprint(data, getattr(self, '_full_check', False))
@@ -157,7 +181,7 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     def resample(self, data, **kwargs):
         '''One sweep: sigma2, Tau2, lam2 (device), then GASS for W and V (factor.py:112-128).'''
-        if self._poisson:
+        if self._builtin:
             return BayesianTensorFiltering.resample(self, data, **kwargs)
         self._sync_ep()
         self._device_hyper_step()
@@ -168,7 +192,7 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     def run_gibbs(self, data, nburn=1000, nthin=1, nsamples=1000, verbose=True, print_freq=100,
                   callback=None, **kwargs):
-        if self._poisson:
+        if self._builtin:
             return _BayesianModel.run_gibbs(self, data, nburn=nburn, nthin=nthin, nsamples=nsamples, verbose=verbose,
                                             print_freq=print_freq, callback=callback, **kwargs)
         # the likelihood is a Python callback: always the per-sweep path of genlasso.py:37-66
@@ -259,12 +283,15 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     def logprob(self, data, **kwargs):
         tau = (self.W[:, None, None] * self.V[None]).sum(axis=-1)
-        if self._poisson:
-            Y = np.asarray(data)
-            if Y.ndim > tau.ndim:
-                tau = tau[..., None]
+        if self._builtin:
             with warnings.catch_warnings():
                 warnings.simplefilter('ignore', category=RuntimeWarning)
+                if self._builtin == 'binomial':
+                    Y, Nt = self._binomial_data(data)
+                    return np.nansum(binom.logpmf(Y, Nt, tau))
+                Y = np.asarray(data)
+                if Y.ndim > tau.ndim:
+                    tau = tau[..., None]
                 return np.nansum(poisson.logpmf(Y, tau))
         return self.loglikelihood(data, tau, self.W, self.V)
 

@@ -96,14 +96,16 @@ struct btf_engine {
     double *nu2c = nullptr, *wc = nullptr, *sc = nullptr;      // [nloc_pad][Ppad], allocated on first use
     unsigned long long* nu2_nbad = nullptr;
     StatsPlan plan_row_w{}, plan_col_w{};                      // statistics plans for those f64 weights
-    // Poisson model (constrained GASS steps, gass_kernels.cu; single GPU).  With an EP approximation the W / V centres
-    // come from the f64-weight statistics of wc = 1 / sigma^2 and sc = mu / sigma^2 (the buffers of the per-cell nu2 mode)
+    // Constrained Poisson and Binomial models (GASS steps, gass_kernels.cu; single GPU).  With an EP approximation the
+    // W / V centres come from the f64-weight statistics of wc = 1 / sigma^2 and sc = mu / sigma^2 (the buffers of the
+    // per-cell nu2 mode)
     bool gass_set = false, ep_on = false;
     int gJ = 0, gnrc = 0, gnfine = 0, gngrid = 0;
     double *gA = nullptr, *gC = nullptr, *growc = nullptr, *ggrid_f = nullptr, *ggrid_c = nullptr;
     double *Wold = nullptr, *Vold = nullptr, *gmeanW = nullptr, *gmeanV = nullptr;   // the state before the step, the centres
     double *ep_mu = nullptr, *ep_sig = nullptr;                // [nloc_pad][Ppad]
-    double* lgy = nullptr;                                     // [nloc_pad][Ppad] sum of lgamma(y + 1) over the observed replicates
+    double* lgy = nullptr;                                     // [nloc_pad][Ppad] Poisson: sum of lgamma(y + 1) over the observed
+                                                               // replicates; Binomial: the log binomial coefficient
     int* gass_nbad = nullptr;                                  // [2] rows / columns whose starting point violates a constraint
     int nreps = 1;
     bool has_data = false, data_reduced = false;
@@ -167,6 +169,9 @@ struct btf_engine {
 };
 
 static int round_up(int x, int m) { return (x + m - 1) / m * m; }
+
+// the likelihoods whose W and V steps are GASS transitions (gass_kernels.cu)
+static bool gass_likelihood(int lik) { return lik == BTF_POISSON || lik == BTF_CBINOMIAL; }
 
 void btf_config_default(btf_config* c) {
     memset(c, 0, sizeof(*c));
@@ -271,8 +276,9 @@ int btf_create(const btf_config* c, btf_engine** out) {
     if (c->nembeds < 1 || c->nembeds > 32) return set_err(BTF_EINVAL, "nembeds must be in [1, 32]");
     if (c->tf_order < 0 || c->tf_order > 3) return set_err(BTF_EINVAL, "tf_order must be in [0, 3]");
     if (c->ndepth < c->tf_order + 2) return set_err(BTF_EINVAL, "ndepth must be >= tf_order + 2");
-    if (c->likelihood < BTF_GAUSSIAN || c->likelihood > BTF_POISSON) return set_err(BTF_EINVAL, "unknown likelihood %d", c->likelihood);
-    if (c->likelihood == BTF_POISSON && c->world_size > 1) return set_err(BTF_EINVAL, "the Poisson model is single-GPU");
+    if (c->likelihood < BTF_GAUSSIAN || c->likelihood > BTF_CBINOMIAL) return set_err(BTF_EINVAL, "unknown likelihood %d", c->likelihood);
+    if (gass_likelihood(c->likelihood) && c->world_size > 1)
+        return set_err(BTF_EINVAL, "the constrained %s model is single-GPU", c->likelihood == BTF_POISSON ? "Poisson" : "Binomial");
     btf_engine* e = new btf_engine();
     // every early return below releases what has been created so far (streams, events, device buffers)
     struct Guard { btf_engine* e; ~Guard() { if (e) btf_destroy(e); } } guard{e};
@@ -377,8 +383,9 @@ int btf_create(const btf_config* c, btf_engine** out) {
     const size_t cells = (size_t)e->nloc_pad * e->Ppad;
     CK(dev_alloc(&e->cnt, cells));
     CK(dev_alloc(&e->S, cells));
-    const bool pg = c->likelihood != BTF_GAUSSIAN;      // f64 weights in the statistics (Poisson: the EP weights)
+    const bool pg = c->likelihood != BTF_GAUSSIAN;      // f64 weights in the statistics (GASS models: the EP weights)
     if (c->likelihood == BTF_BINOMIAL || c->likelihood == BTF_NEGBINOMIAL) { CK(dev_alloc(&e->ntr, cells)); CK(dev_alloc(&e->omega, cells)); }
+    if (c->likelihood == BTF_CBINOMIAL) CK(dev_alloc(&e->ntr, cells));
     if (c->likelihood == BTF_NEGBINOMIAL) {
         e->Rn = (c->rdims_mask & 1) ? 1 : e->N;
         e->Rm = (c->rdims_mask & 2) ? 1 : e->M;
@@ -657,10 +664,39 @@ int btf_set_data_poisson(btf_engine* e, const double* Y, int32_t nreps) {
     return set_data_compact(e, Y, 0, e->nloc, nreps, 1);
 }
 
+// The constrained Binomial model: every observed cell (y and n not NaN) must hold non-negative integers with y <= n.
+// The log binomial coefficient lgamma(n + 1) - (lgamma(y + 1) + lgamma(n - y + 1)) of each observed cell goes to `lc`:
+// scipy's logpmf keeps it, and a cell whose probability leaves [0, 1] drops out of the log-likelihood together with it.
+static int binomial_coefficients(btf_engine* e, const double* Ys, const double* Nt, std::vector<double>* lc) {
+    const size_t cells = (size_t)e->nloc * e->P;
+    std::vector<double> hy, hn;
+    if (is_device_ptr(Ys)) { hy.resize(cells); CK(cudaMemcpy(hy.data(), Ys, cells * sizeof(double), cudaMemcpyDeviceToHost)); Ys = hy.data(); }
+    if (is_device_ptr(Nt)) { hn.resize(cells); CK(cudaMemcpy(hn.data(), Nt, cells * sizeof(double), cudaMemcpyDeviceToHost)); Nt = hn.data(); }
+    lc->assign(cells, 0.0);
+    unsigned long long nbad = 0;
+    for (size_t c = 0; c < cells; ++c) {
+        const double y = Ys[c], n = Nt[c];
+        if (std::isnan(y) || std::isnan(n)) continue;
+        const bool count_y = y >= 0.0 && std::isfinite(y) && y == std::floor(y);
+        const bool count_n = n >= 0.0 && std::isfinite(n) && n == std::floor(n);
+        if (!(count_y && count_n && y <= n)) { ++nbad; continue; }
+        (*lc)[c] = std::lgamma(n + 1.0) - (std::lgamma(y + 1.0) + std::lgamma(n - y + 1.0));
+    }
+    if (nbad)
+        return set_err(BTF_EINVAL, "%llu observed cell(s) do not hold non-negative integer counts y <= n (successes, trials)", nbad);
+    return BTF_OK;
+}
+
 int btf_set_data_binomial(btf_engine* e, const double* Ys, const double* Nt) {
     if (!e || !Ys || !Nt) return set_err(BTF_EINVAL, "null argument");
-    if (e->cfg.likelihood != BTF_BINOMIAL) return set_err(BTF_ESTATE, "engine is not Binomial");
+    if (e->cfg.likelihood != BTF_BINOMIAL && e->cfg.likelihood != BTF_CBINOMIAL) return set_err(BTF_ESTATE, "engine is not Binomial");
     CK(cudaSetDevice(e->cfg.device));
+    std::vector<double> lc;
+    if (e->cfg.likelihood == BTF_CBINOMIAL) {
+        int rc = binomial_coefficients(e, Ys, Nt, &lc);
+        if (rc) return rc;
+        if (!e->lgy) CK(dev_alloc(&e->lgy, (size_t)e->nloc_pad * e->Ppad));
+    }
     free_graph(e);
     const size_t row_elems = (size_t)e->P;
     const bool on_dev = is_device_ptr(Ys) && is_device_ptr(Nt);
@@ -691,6 +727,7 @@ int btf_set_data_binomial(btf_engine* e, const double* Ys, const double* Nt) {
     }
     CK(cudaStreamSynchronize(e->stream));
     CK(cudaGetLastError());
+    if (!lc.empty()) { int rc = copy_pitched(e, e->lgy, lc.data(), false); if (rc) return rc; }
     e->has_data = true; e->data_reduced = true; e->i8_decided = false;
     return BTF_OK;
 }
@@ -832,7 +869,7 @@ static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host) 
     return BTF_OK;
 }
 
-// ------------------------------------------------------------------ constrained Poisson model (GASS steps)
+// ------------------------------------------------------------------ constrained Poisson and Binomial models (GASS steps)
 static cudaError_t upload_copy(double** dst, const double* src, size_t n) {
     if (*dst) { cudaFree(*dst); *dst = nullptr; }
     cudaError_t ce = dev_alloc(dst, std::max<size_t>(n, 1), false);
@@ -843,7 +880,7 @@ static cudaError_t upload_copy(double** dst, const double* src, size_t n) {
 int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, const double* rowcons, int32_t nrowcons,
                  const double* grid_fine, int32_t ngrid_fine, const double* grid_coarse, int32_t ngrid) {
     if (!e) return set_err(BTF_EINVAL, "null engine");
-    if (e->cfg.likelihood != BTF_POISSON) return set_err(BTF_ESTATE, "GASS steps need a Poisson engine");
+    if (!gass_likelihood(e->cfg.likelihood)) return set_err(BTF_ESTATE, "GASS steps need a constrained Poisson or Binomial engine");
     if (J < 0 || nrowcons < 0 || (J > 0 && (!A || !C)) || (nrowcons > 0 && !rowcons))
         return set_err(BTF_EINVAL, "constraints: J >= 0 rows of A [J, T] and C [J], nrowcons >= 0 rows of [K + 1]");
     if (!grid_fine || !grid_coarse || ngrid < 1 || ngrid > ngrid_fine || ngrid_fine > 65535)
@@ -887,7 +924,7 @@ int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, con
 // EP approximation N(mu, sigma^2) per cell (host memory, [Nloc, M, T]); NULL: none
 int btf_set_ep(btf_engine* e, const double* mu, const double* sigma) {
     if (!e) return set_err(BTF_EINVAL, "null engine");
-    if (e->cfg.likelihood != BTF_POISSON) return set_err(BTF_ESTATE, "an EP approximation needs a Poisson engine");
+    if (!gass_likelihood(e->cfg.likelihood)) return set_err(BTF_ESTATE, "an EP approximation needs a constrained Poisson or Binomial engine");
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaStreamSynchronize(e->stream));
     if (!mu || !sigma) {
@@ -956,6 +993,8 @@ int btf_set_state(btf_engine* e, const char* name, const double* host, size_t n)
         e->resid_valid = false;
         return BTF_OK;
     }
+    if (nm == "Ntrials" && e->cfg.likelihood == BTF_CBINOMIAL)
+        return set_err(BTF_ESTATE, "the trials of a constrained Binomial engine come with its data: use btf_set_data_binomial");
     if ((nm == "omega" && e->omega) || (nm == "Ntrials" && e->ntr)) {
         if (n != (size_t)e->nloc * e->P) return set_err(BTF_EINVAL, "%s: expected %zu values", name, (size_t)e->nloc * e->P);
         return copy_pitched(e, nm == "omega" ? e->omega : e->ntr, const_cast<double*>(host), false);
@@ -1364,7 +1403,8 @@ static GassArgs gass_args(btf_engine* e, bool col) {
     memset(&g, 0, sizeof(g));
     g.col = col;
     g.N = e->N; g.M = e->M; g.T = e->T; g.K = e->K; g.P = e->P; g.ld = e->Ppad;
-    g.cnt = e->cnt; g.S = e->S; g.lgy = e->lgy;
+    g.cnt = e->cnt; g.S = e->S; g.lgy = e->lgy; g.ntr = e->ntr;
+    g.binomial = e->cfg.likelihood == BTF_CBINOMIAL;
     g.ep_mu = e->ep_on ? e->ep_mu : nullptr; g.ep_sig = e->ep_on ? e->ep_sig : nullptr;
     g.A = e->gA; g.C = e->gC; g.J = e->gJ; g.rowcons = e->growc; g.nrc = e->gnrc;
     g.grid_fine = e->ggrid_f; g.nfine = e->gnfine; g.grid_coarse = e->ggrid_c; g.ngrid = e->gngrid;
@@ -1501,11 +1541,11 @@ static int enqueue_sweep(btf_engine* e) {
     }
     // ---- W | rest
     phase_mark(e, PH_ROW_STATS);
-    // Poisson: the statistics of the EP approximation (weights 1 / sigma^2, right-hand side mu / sigma^2), none without it
-    const bool poisson = c.likelihood == BTF_POISSON;
-    const bool no_stats = poisson && !e->ep_on;
-    const void* wt = (percell || poisson) ? (const void*)e->wc : gauss ? (const void*)e->cnt : (const void*)e->omega;
-    const double* sv = (percell || poisson) ? e->sc : e->S;
+    // GASS models: the statistics of the EP approximation (weights 1 / sigma^2, right-hand side mu / sigma^2), none without it
+    const bool gass = gass_likelihood(c.likelihood);
+    const bool no_stats = gass && !e->ep_on;
+    const void* wt = (percell || gass) ? (const void*)e->wc : gauss ? (const void*)e->cnt : (const void*)e->omega;
+    const double* sv = (percell || gass) ? e->sc : e->S;
     const bool wf64 = !homo;
     const StatsPlan& prow = stats_plan(e, false);
     const StatsPlan& pcol = stats_plan(e, true);
@@ -1527,13 +1567,13 @@ static int enqueue_sweep(btf_engine* e) {
         ra.diag_L = diag_get(e, "W_L", (size_t)e->N * e->K * e->K);
         ra.diag_mean = diag_get(e, "W_mean", (size_t)e->N * e->K);
         ra.diag_b = diag_get(e, "W_b", (size_t)e->N * e->K);
-        if (poisson) {
+        if (gass) {
             // GASS needs the old state and, with EP, the centre of the ellipse
             CK(cudaMemcpyAsync(e->Wold, e->W, (size_t)e->N * e->K * 8, cudaMemcpyDeviceToDevice, st));
             if (e->ep_on && !ra.diag_mean) ra.diag_mean = e->gmeanW;
         }
         launch_row_solve(ra, nullptr, st); e->launches++;
-        if (poisson) {
+        if (gass) {
             GassArgs ga = gass_args(e, false);
             ga.Wmean = e->ep_on ? ra.diag_mean : nullptr;
             launch_gass(ga, st); e->launches++;
@@ -1563,13 +1603,13 @@ static int enqueue_sweep(btf_engine* e) {
         ba.diag_band = diag_get(e, "V_band", bn);
         ba.diag_chol = diag_get(e, "V_chol", bn);
         ba.diag_mean = diag_get(e, "V_mean", (size_t)e->P * e->K);
-        if (poisson && e->ep_on && !ba.diag_mean) ba.diag_mean = e->gmeanV;
+        if (gass && e->ep_on && !ba.diag_mean) ba.diag_mean = e->gmeanV;
         ba.diag_retries = e->diag_retries;
         ba.resid_partials = homo ? e->resid_partials + c.col_begin : nullptr;
         auto band = [&]() {
-            if (poisson) CK(cudaMemcpyAsync(e->Vold, e->V, (size_t)e->P * e->K * 8, cudaMemcpyDeviceToDevice, st));
+            if (gass) CK(cudaMemcpyAsync(e->Vold, e->V, (size_t)e->P * e->K * 8, cudaMemcpyDeviceToDevice, st));
             launch_band_solve(ba, st); e->launches++;
-            if (poisson) {
+            if (gass) {
                 GassArgs ga = gass_args(e, true);
                 ga.Vmean = e->ep_on ? ba.diag_mean : nullptr;
                 launch_gass(ga, st); e->launches++;
@@ -1717,7 +1757,7 @@ static int pre_run(btf_engine* e) {
         }
         if (e->nu2_bad) return nu2_bad_error(e);
     }
-    if (e->cfg.likelihood == BTF_POISSON) {
+    if (gass_likelihood(e->cfg.likelihood)) {
         if (!e->gass_set) return set_err(BTF_ESTATE, "no constraints: call btf_set_gass first");
         int rc = gass_check_start(e);
         if (rc) return rc;

@@ -1,12 +1,13 @@
-// GASS: generalized analytic slice sampling of the constrained model's W rows and V columns under the built-in
-// Poisson likelihood (functionalmf_b200/gass.py, factor.py:665-892).  One CTA per row or column:
+// GASS: generalized analytic slice sampling of the constrained model's W rows and V columns under a built-in
+// likelihood, Poisson or Binomial (functionalmf_b200/gass.py, factor.py:665-892).  One CTA per row or column:
 //   1. the constraint products a = A(x - mu), b = A v, c = C - A mu of every constraint row, without the Kronecker
 //      matrix (rows: coefficients sum_t A[c,t] V[j,t,:]; columns: A[c,t] W[i,:]);
 //   2. the feasible grid of gass.feasible_angles: "outside" intervals are removed as index ranges through a difference
 //      array, the "inside" ones intersected into [lo, hi]; no active constraint selects the coarse grid;
 //   3. thinning by a partial Fisher-Yates over the ascending feasible index list;
 //   4. the log-likelihood of every candidate (FP64, fixed-order block reductions) and the uniform pick among those
-//      at or above the slice height.
+//      at or above the slice height.  The kernels are instantiated per likelihood: a cell type loads what a cell of
+//      the data holds and evaluates its log-likelihood at a candidate's rate or probability.
 // Every random choice is a function of ngrid + 2 uniforms per row / column (slice, thinning, pick): Philox keyed by
 // (seed, sweep, stream, row or column), or injected.
 #include "kernels.h"
@@ -90,6 +91,48 @@ __device__ __forceinline__ double poisson_cell(double lam, int n, double s, doub
     if (lam == 0.0) return s > 0.0 ? -INFINITY : 0.0;
     return 0.0;
 }
+// scipy.stats.binom.logpmf(y, n, p) of one observed cell, dropped by nansum where it is NaN (scipy 1.18's _logpmf:
+// combiln + xlogy(y, p) + xlog1py(n - y, -p), combiln = lgamma(n + 1) - (lgamma(y + 1) + lgamma(n - y + 1)) = lc):
+// 0 < p < 1 -> lc + y log p + (n - y) log1p(-p), a zero count contributing exactly 0; p = 0 -> 0 if y = 0, else -inf;
+// p = 1 -> 0 if y = n, else -inf; p outside [0, 1] (NaN in scipy) -> 0, with lc; n = 0 -> 0.  Evaluated without fused
+// operations, in scipy's order.
+__device__ __forceinline__ double binomial_cell(double p, double y, double n, double lc) {
+    if (n == 0.0) return 0.0;
+    if (p > 0.0 && p < 1.0) {
+        const double ty = y > 0.0 ? mul(y, log(p)) : 0.0;
+        const double tn = n > y ? mul(n - y, log1p(-p)) : 0.0;
+        return add(add(lc, ty), tn);
+    }
+    if (p == 0.0) return y > 0.0 ? -INFINITY : 0.0;
+    if (p == 1.0) return y < n ? -INFINITY : 0.0;
+    return 0.0;
+}
+
+// The cell likelihoods gass_body is instantiated for: load() reads what the data keep for a cell, ll() is its
+// log-likelihood at the rate / probability lam of a candidate.
+struct PoissonLik {
+    struct Cell { int n; double s, lg; };
+    static __device__ __forceinline__ Cell load(const GassArgs& a, size_t cell) {
+        Cell c;
+        c.n = a.cnt[cell];
+        c.s = a.S[cell]; c.lg = a.lgy[cell];
+        return c;
+    }
+    static __device__ __forceinline__ double ll(double lam, const Cell& c) { return poisson_cell(lam, c.n, c.s, c.lg); }
+};
+struct BinomialLik {
+    struct Cell { bool obs; double y, n, lc; };
+    static __device__ __forceinline__ Cell load(const GassArgs& a, size_t cell) {
+        Cell c;
+        c.obs = a.cnt[cell] != 0;
+        c.n = a.ntr[cell];
+        c.y = a.S[cell] + 0.5 * c.n;       // kappa = y - n/2: exact for integer counts
+        c.lc = a.lgy[cell];
+        return c;
+    }
+    static __device__ __forceinline__ double ll(double p, const Cell& c) { return c.obs ? binomial_cell(p, c.y, c.n, c.lc) : 0.0; }
+};
+
 // scipy.stats.norm.logpdf(lam, mu, sigma)
 __device__ __forceinline__ double norm_logpdf(double lam, double mu, double sg) {
     const double z = (lam - mu) / sg;
@@ -113,6 +156,7 @@ size_t gass_smem_bytes(int D, int nfine, int ngrid) {
 }
 
 // One row (col = false: W row i, D = min(K, i + 1) entries) or one column (col = true: V[j], D = T K, t-major).
+template <class Lik>
 __device__ void gass_body(const GassArgs& a, bool col) {
     extern __shared__ __align__(16) unsigned char gsm[];
     __shared__ double shd[32];
@@ -276,15 +320,14 @@ __device__ void gass_body(const GassArgs& a, bool col) {
                     const double fk = f[k], xk = x[t * K + k], mk = mu[t * K + k];
                     tx += fk * xk; t0 += fk * (xk - mk); tv += fk * v[t * K + k]; tm += fk * mk;
                 }
-                const int n = a.cnt[cell];
-                const double s = a.S[cell], lg = a.lgy[cell];
+                const typename Lik::Cell cd = Lik::load(a, cell);
                 const bool ep = a.ep_mu != nullptr;
                 const double em = ep ? a.ep_mu[cell] : 0.0, es = ep ? a.ep_sig[cell] : 1.0;
 #pragma unroll
                 for (int q = 0; q < GASS_CHUNK; ++q) {
                     if (q >= nc) continue;
                     const double lam = c0 < 0 ? tx : t0 * cs[q] + tv * sn[q] + tm;
-                    acc[q] += poisson_cell(lam, n, s, lg);
+                    acc[q] += Lik::ll(lam, cd);
                     if (ep) acc[q] -= norm_logpdf(lam, em, es);
                 }
             } else {
@@ -295,15 +338,14 @@ __device__ void gass_body(const GassArgs& a, bool col) {
                     const double fk = f[k];
                     tx += fk * x[k]; t0 += fk * (x[k] - mu[k]); tv += fk * v[k]; tm += fk * mu[k];
                 }
-                const int n = a.cnt[cell];
-                const double s = a.S[cell], lg = a.lgy[cell];
+                const typename Lik::Cell cd = Lik::load(a, cell);
                 const bool ep = a.ep_mu != nullptr;
                 const double em = ep ? a.ep_mu[cell] : 0.0, es = ep ? a.ep_sig[cell] : 1.0;
 #pragma unroll
                 for (int q = 0; q < GASS_CHUNK; ++q) {
                     if (q >= nc) continue;
                     const double lam = c0 < 0 ? tx : t0 * cs[q] + tv * sn[q] + tm;
-                    acc[q] += poisson_cell(lam, n, s, lg);
+                    acc[q] += Lik::ll(lam, cd);
                     if (ep) acc[q] -= norm_logpdf(lam, em, es);
                 }
             }
@@ -352,20 +394,28 @@ __device__ void gass_body(const GassArgs& a, bool col) {
     }
 }
 
-__global__ void __launch_bounds__(GASS_THREADS) gass_row_kernel(GassArgs a) { gass_body(a, false); }
-__global__ void __launch_bounds__(GASS_THREADS) gass_col_kernel(GassArgs a) { gass_body(a, true); }
+template <class Lik>
+__global__ void __launch_bounds__(GASS_THREADS) gass_row_kernel(GassArgs a) { gass_body<Lik>(a, false); }
+template <class Lik>
+__global__ void __launch_bounds__(GASS_THREADS) gass_col_kernel(GassArgs a) { gass_body<Lik>(a, true); }
 
-void launch_gass(const GassArgs& a, cudaStream_t st) {
+template <class Lik>
+static void launch_gass_lik(const GassArgs& a, cudaStream_t st) {
     static PerDeviceMax attr_row, attr_col;
     const int D = a.col ? a.T * a.K : a.K;
     const size_t smem = gass_smem_bytes(D, a.nfine, a.ngrid);
     if (a.col) {
-        if (attr_col.raise(smem)) cudaFuncSetAttribute(gass_col_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        gass_col_kernel<<<a.M, GASS_THREADS, smem, st>>>(a);
+        if (attr_col.raise(smem)) cudaFuncSetAttribute(gass_col_kernel<Lik>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        gass_col_kernel<Lik><<<a.M, GASS_THREADS, smem, st>>>(a);
     } else {
-        if (attr_row.raise(smem)) cudaFuncSetAttribute(gass_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        gass_row_kernel<<<a.N, GASS_THREADS, smem, st>>>(a);
+        if (attr_row.raise(smem)) cudaFuncSetAttribute(gass_row_kernel<Lik>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        gass_row_kernel<Lik><<<a.N, GASS_THREADS, smem, st>>>(a);
     }
+}
+
+void launch_gass(const GassArgs& a, cudaStream_t st) {
+    if (a.binomial) launch_gass_lik<BinomialLik>(a, st);
+    else launch_gass_lik<PoissonLik>(a, st);
 }
 
 }  // namespace btf

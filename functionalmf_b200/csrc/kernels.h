@@ -266,12 +266,15 @@ void launch_nb_hist(const NbArgs& a, int vstride, cudaStream_t st);
 // (factor.py:513-554, 494-511)
 void launch_nb_update(const NbArgs& a, cudaStream_t st);
 
-// ---------------------------------------------------------------- GASS steps of the constrained Poisson model (gass_kernels.cu)
+// ---------------------------------------------------------------- GASS steps of the constrained Poisson and Binomial
+// models (gass_kernels.cu)
 struct GassArgs {
     bool col;                                   // false: one CTA per W row (gass_row_kernel), true: per V column (gass_col_kernel)
     int N, M, T, K, P; long long ld;
-    const uint8_t* cnt; const double* S;        // observed replicates and their sum, [N][ld]
-    const double* lgy;                          // sum of lgamma(y + 1) over the observed replicates, [N][ld]
+    const uint8_t* cnt; const double* S;        // Poisson: observed replicates and their sum; Binomial: observed flag and
+                                                // kappa = y - n/2, [N][ld]
+    const double* lgy;                          // Poisson: sum of lgamma(y + 1) over the observed replicates; Binomial: the
+                                                // log binomial coefficient lgamma(n + 1) - (lgamma(y + 1) + lgamma(n - y + 1)), [N][ld]
     const double *ep_mu, *ep_sig;               // EP approximation [N][ld], or nullptr
     const double* A; const double* C; int J;    // constraints A[c] . Mu[i, j, :] >= C[c], A [J][T]
     const double* rowcons; int nrc;             // row constraints [nrc][K + 1] (W rows only)
@@ -285,6 +288,9 @@ struct GassArgs {
     const Scalars* scal; uint64_t seed;
     double* diag;                               // [rows or cols][3] = (F, G, theta), or nullptr
     int check_only; int* nbad;                  // 1: only count the rows / columns whose state violates a constraint
+    // (appended, so that the Poisson kernels read every field above at the offsets they always had)
+    const double* ntr;                          // Binomial: trials n, [N][ld]
+    bool binomial;                              // the cell likelihood: false Poisson, true Binomial
 };
 size_t gass_smem_bytes(int D, int nfine, int ngrid);
 void launch_gass(const GassArgs& a, cudaStream_t st);

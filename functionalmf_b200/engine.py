@@ -107,6 +107,7 @@ class Engine(object):
                                                     int(nreps), 1 if reset else 0))
 
     def set_data_binomial(self, Y, Nt):
+        """Successes and trials [Nloc, M, T] of a Binomial or constrained Binomial engine (NaN = missing)."""
         Y, Nt = _f64(Y), _f64(Nt)
         if Y.shape != (self.nloc, self.M, self.T) or Nt.shape != Y.shape:
             raise ValueError('Binomial data must be two [%d,%d,%d] tensors' % (self.nloc, self.M, self.T))
@@ -155,7 +156,8 @@ class Engine(object):
                                       _ptr(gf), gf.size, _ptr(gc), gc.size))
 
     def set_ep(self, mu, sigma):
-        """EP approximation N(mu, sigma^2) per cell [Nloc, M, T] of a Poisson engine (``None``: none)."""
+        """EP approximation N(mu, sigma^2) per cell [Nloc, M, T] of a constrained Poisson or Binomial engine
+        (``None``: none)."""
         if mu is None:
             L.check(self.lib.btf_set_ep(self._h, C.c_void_p(0), C.c_void_p(0)))
             return

@@ -30,7 +30,9 @@ extern "C" {
 #define BTF_ESTATE       -4   /* call order / missing data */
 #define BTF_ENCCL        -5   /* NCCL error */
 
-enum { BTF_GAUSSIAN = 0, BTF_BINOMIAL = 1, BTF_NEGBINOMIAL = 2, BTF_POISSON = 3 };
+/* BTF_POISSON and BTF_CBINOMIAL: the constrained model's built-in likelihoods, whose W and V steps are GASS transitions
+ * (Poisson counts; Binomial successes out of trials with the identity link p = W V^T) */
+enum { BTF_GAUSSIAN = 0, BTF_BINOMIAL = 1, BTF_NEGBINOMIAL = 2, BTF_POISSON = 3, BTF_CBINOMIAL = 4 };
 
 /* sample_mask bits: which variables resample() updates (factor.py:112-128, 306-311) */
 enum {
@@ -45,7 +47,7 @@ typedef struct btf_engine btf_engine;
 typedef struct btf_config {
     int32_t nrows, ncols, ndepth;      /* global N, M, T */
     int32_t nembeds, tf_order;         /* K, p */
-    int32_t likelihood;                /* BTF_GAUSSIAN / BINOMIAL / NEGBINOMIAL / POISSON */
+    int32_t likelihood;                /* BTF_GAUSSIAN / BINOMIAL / NEGBINOMIAL / POISSON / CBINOMIAL */
     double  sigma2_a, sigma2_b;        /* factor.py:27 */
     double  nu2_a, nu2_b;              /* factor.py:289 */
     double  stability;                 /* factor.py:32 */
@@ -85,6 +87,9 @@ int btf_set_data_gaussian(btf_engine* e, const double* Y, int32_t nreps);
 /* streaming form: rows [row0, row0+nrows) of the local shard; reset != 0 on the first piece */
 int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int32_t nrows, int32_t nreps,
                                int32_t reset);
+/* Successes and trials [Nloc, M, T] each (a cell is missing where either is NaN).  BTF_BINOMIAL (Polya-Gamma) or
+ * BTF_CBINOMIAL (see the constrained models below; there every observed cell must hold non-negative integers y <= n,
+ * else BTF_EINVAL giving the number of such cells, and nothing changes). */
 int btf_set_data_binomial(btf_engine* e, const double* Ysucc, const double* Ntrials);
 int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps);
 /* Known per-cell noise variances of a Gaussian model: the reference's heteroskedastic branch, nu2 an
@@ -99,14 +104,19 @@ int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps);
  * reference holds an array nu2 fixed. */
 int btf_set_nu2_cells(btf_engine* e, const double* nu2);
 
-/* ---- the constrained Poisson model (ConstrainedNonconjugateBayesianTensorFiltering with the Poisson likelihood of
- * examples/poisson_tensor_filtering.py, factor.py:894-1017).  A BTF_POISSON engine runs the whole sweep on the device:
- * sigma2, Tau2, lam2, then for W and for V the Gaussian centre and proposal (the f64-weight statistics of an EP
- * approximation, or the prior alone) followed by one GASS transition per row / column (gass.py:13-130) under
- * ll = nansum of scipy.stats.poisson.logpmf(y, lambda) over the observed replicates, lambda = W V^T (a cell with
- * lambda < 0 is NaN there and drops out, lambda = 0 with y > 0 gives -inf), minus sum_cells norm.logpdf(lambda; mu_ep,
- * sigma_ep) with EP.
- * Single GPU: btf_create refuses world_size > 1 for this likelihood.
+/* ---- the constrained Poisson and Binomial models (ConstrainedNonconjugateBayesianTensorFiltering with the Poisson
+ * likelihood of examples/poisson_tensor_filtering.py, or a Binomial one; factor.py:894-1017).  A BTF_POISSON or
+ * BTF_CBINOMIAL engine runs the whole sweep on the device: sigma2, Tau2, lam2, then for W and for V the Gaussian centre
+ * and proposal (the f64-weight statistics of an EP approximation, or the prior alone) followed by one GASS transition
+ * per row / column (gass.py:13-130) under ll = nansum of the cells' log-likelihoods at lambda = W V^T, minus
+ * sum_cells norm.logpdf(lambda; mu_ep, sigma_ep) with EP:
+ *   Poisson: scipy.stats.poisson.logpmf(y, lambda) over the observed replicates (a cell with lambda < 0 is NaN there and
+ *     drops out, lambda = 0 with y > 0 gives -inf);
+ *   Binomial: scipy.stats.binom.logpmf(y, n, p = lambda) (p outside [0, 1] is NaN there and drops out; p = 0 with y > 0
+ *     and p = 1 with y < n give -inf; n = 0 gives 0).  The data come through btf_set_data_binomial and take 25 B / cell
+ *     (observed flag, kappa = y - n/2, n and the log binomial coefficient); btf_set_data_poisson refuses this engine
+ *     with BTF_ESTATE, as btf_set_data_binomial refuses a Poisson one.
+ * Single GPU: btf_create refuses world_size > 1 for these likelihoods.
  *
  * Counts Y [Nloc, M, T, nreps] (NaN = missing, host or device memory), kept in the Gaussian data's compact form
  * plus sum_r lgamma(y_r + 1) per cell (17 B / cell).  BTF_EINVAL when observed values are negative or not integers (the message gives their number). */
@@ -121,14 +131,14 @@ int btf_set_data_poisson(btf_engine* e, const double* Y, int32_t nreps);
  * violation, before anything changes. */
 int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, const double* rowcons, int32_t nrowcons,
                  const double* grid_fine, int32_t ngrid_fine, const double* grid_coarse, int32_t ngrid);
-/* EP approximation (host memory, [Nloc, M, T] each; NULL: none).  The W / V centres come from the weights 1 / sigma^2 and
+/* EP approximation (host memory, [Nloc, M, T] each; NULL: none) of either model.  The W / V centres come from the weights 1 / sigma^2 and
  * the right-hand side mu / sigma^2; every candidate's ll subtracts sum norm.logpdf(lambda; mu, sigma) over ALL cells of the
  * row / column.  BTF_EINVAL when a mean is not finite or a scale is not finite and > 0 (with their number). 32 B / cell. */
 int btf_set_ep(btf_engine* e, const double* mu, const double* sigma);
 
 /* ---- state: names "W" [N,K] (global), "V" [M,T,K], "Tau2","Tau2_a","Tau2_b",
  * "Tau2_c" [M,R_D], "lam2","lam2_a","sigma2","nu2" [1], "omega" [Nloc,M,T]
- * (Binomial/NB: 1/nu2), "R" [R shape], "Ntrials" [Nloc,M,T], "Delta" [R_D,T]
+ * (Binomial/NB: 1/nu2), "R" [R shape], "Ntrials" [Nloc,M,T] (read-only on BTF_CBINOMIAL engines), "Delta" [R_D,T]
  * (read-only, utils.py:56-98).  `n` = number of doubles in `host`. */
 int btf_set_state(btf_engine* e, const char* name, const double* host, size_t n);
 int btf_get_state(btf_engine* e, const char* name, double* host, size_t n);
@@ -200,7 +210,7 @@ int btf_sweep_timed(btf_engine* e, int32_t nsweeps, double* ms_out);
  * Philox stream (cleared after that sweep): "z_W" [N,K], "z_V" [M,T,K] t-major,
  * "g_tau" [M,4,R_D], "g_lam" [2], "g_sigma2" [1], "g_nu2" [1] (standard gammas),
  * "omega" [Nloc,M,T], "z_R"/"u_R" [nmetropolis,*R.shape],
- * "gass_u_W" [N, ngrid+2], "gass_u_V" [M, ngrid+2] (Poisson: per row / column the slice uniform, ngrid thinning
+ * "gass_u_W" [N, ngrid+2], "gass_u_V" [M, ngrid+2] (GASS models: per row / column the slice uniform, ngrid thinning
  * uniforms -- candidate k swaps position k with k + floor(u_k (F - k)) of the ascending feasible list when F > ngrid --
  * and the pick uniform: candidate floor(u G) of the G at or above the slice). */
 int btf_inject_noise(btf_engine* e, const char* name, const double* host, size_t n);

@@ -1,10 +1,12 @@
-"""Sweeps/s of the constrained Poisson model (ConstrainedNonconjugateBayesianTensorFiltering):
-  politics   19 x 19 x 228, K = 5, p = 2, positivity constraints Mu >= 0, ngrid = 100 (the shape of politics/benchmark.py):
-             the device path (loglikelihood='poisson', every step in the engine) and the host path (the same likelihood
+"""Sweeps/s of the constrained Poisson or Binomial model (ConstrainedNonconjugateBayesianTensorFiltering):
+  politics   19 x 19 x 228, K = 5, p = 2, ngrid = 100 (the shape of politics/benchmark.py): the device path
+             (loglikelihood='poisson' or 'binomial', every step in the engine) and the host path (the same likelihood
              as a Python callable, GASS on the host), timed alternately in one process;
   large      1024 x 256 x 64, K = 8, device path only.
-Synthetic counts from a positive low-rank rate.  Prints the card name and power limit beside the numbers.
-usage: python tools/constrained_bench.py [--rounds 2] [--steps 20] [--host-steps 20]"""
+Poisson: synthetic counts from a positive low-rank rate, constraints Mu >= 0.  Binomial: 20 trials per cell, successes
+from a low-rank probability in (0, 0.9], constraints 0 <= Mu <= 1.  Prints the card name and power limit beside the
+numbers.
+usage: python tools/constrained_bench.py [--likelihood poisson] [--rounds 2] [--steps 20] [--host-steps 20]"""
 import argparse
 import json
 import os
@@ -25,12 +27,21 @@ def card():
     return q.stdout.strip()
 
 
-def problem(N, M, T, K, seed):
+def problem(N, M, T, K, seed, likelihood='poisson'):
     rs = np.random.RandomState(seed)
     W = np.abs(rs.normal(size=(N, K))) + 0.1
     W[np.triu_indices(K, k=1)] = 0
     V = (np.abs(rs.normal(size=(M, T, K))) * 0.2).cumsum(axis=1) / np.sqrt(T) + 0.05
-    Y = rs.poisson(np.einsum('nk,mtk->nmt', W, V)).astype(float)
+    lam = np.einsum('nk,mtk->nmt', W, V)
+    if likelihood == 'binomial':
+        V *= 0.9 / lam.max()                   # p = W V^T in (0, 0.9]
+        Nt = np.full(lam.shape, 20.0)
+        Y = rs.binomial(20, np.einsum('nk,mtk->nmt', W, V)).astype(float)
+        Y[rs.random_sample(Y.shape) < 0.1] = np.nan
+        cons = np.concatenate([np.concatenate([np.eye(T), -np.eye(T)]),
+                               np.concatenate([np.zeros(T), -np.ones(T)])[:, None]], axis=1)
+        return W, V, (Y, Nt), cons
+    Y = rs.poisson(lam).astype(float)
     Y[rs.random_sample(Y.shape) < 0.1] = np.nan
     cons = np.concatenate([np.eye(T), np.zeros((T, 1))], axis=1)
     return W, V, Y, cons
@@ -52,17 +63,24 @@ def timed(m, Y, steps):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument('--likelihood', choices=('poisson', 'binomial'), default='poisson')
     ap.add_argument('--rounds', type=int, default=2)
     ap.add_argument('--steps', type=int, default=20)
     ap.add_argument('--host-steps', type=int, default=20)
     args = ap.parse_args()
     warnings.simplefilter('ignore')
-    from constrained_ll import rowcol_loglikelihood
+    lik = args.likelihood
+    if lik == 'binomial':
+        from test_gpu_constrained_binomial import binomial_rowcol_loglikelihood as host_ll
+    else:
+        from constrained_ll import rowcol_loglikelihood as host_ll
     out = {'card': card()}
+    if lik != 'poisson':
+        out['likelihood'] = lik
     N, M, T, K = 19, 19, 228, 5
-    W, V, Y, cons = problem(N, M, T, K, 1)
-    dev = model('poisson', N, M, T, K, W, V, cons, 100)
-    host = model(rowcol_loglikelihood, N, M, T, K, W, V, cons, 100)
+    W, V, Y, cons = problem(N, M, T, K, 1, lik)
+    dev = model(lik, N, M, T, K, W, V, cons, 100)
+    host = model(host_ll, N, M, T, K, W, V, cons, 100)
     dev.run_gibbs(Y, nburn=3, nsamples=0, verbose=False)
     host.resample(Y)
     sec = {'device': [], 'host': []}
@@ -78,8 +96,8 @@ def main():
                        'host_sweeps_per_s': [round(1.0 / s, 3) for s in sec['host']],
                        'device_resample_sweeps_per_s': round(1.0 / timed(dev, Y, args.steps), 2)}
     N, M, T, K = 1024, 256, 64, 8
-    W, V, Y, cons = problem(N, M, T, K, 2)
-    big = model('poisson', N, M, T, K, W, V, cons, 100)
+    W, V, Y, cons = problem(N, M, T, K, 2, lik)
+    big = model(lik, N, M, T, K, W, V, cons, 100)
     big.run_gibbs(Y, nburn=2, nsamples=0, verbose=False)
     s = []
     for _ in range(args.rounds):
