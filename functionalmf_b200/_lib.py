@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('BTF_B200_LIB') or os.path.join(_HERE, 'libbtf_b200.so')
 
 BTF_OK, BTF_EINVAL, BTF_ECUDA, BTF_ENOTPD, BTF_ESTATE, BTF_ENCCL = 0, -1, -2, -3, -4, -5
-GAUSSIAN, BINOMIAL, NEGBINOMIAL, POISSON, CBINOMIAL = 0, 1, 2, 3, 4     # CBINOMIAL: constrained Binomial (GASS)
+GAUSSIAN, BINOMIAL, NEGBINOMIAL, POISSON, CBINOMIAL, CGAUSSIAN = 0, 1, 2, 3, 4, 5   # C*: constrained Binomial / Gaussian (GASS)
 SAMPLE_NU2, SAMPLE_SIGMA2, SAMPLE_TAU2, SAMPLE_LAM2, SAMPLE_W, SAMPLE_V, SAMPLE_R = 1, 2, 4, 8, 16, 32, 64
 SAMPLE_ALL = 127
 I8_ROUTE_FUSED, I8_ROUTE_SPLITK = 2, 3     # btf_get_diag("i8_route")

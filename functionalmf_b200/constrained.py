@@ -17,9 +17,15 @@ engine in ONE batched launch per step instead of per-row / per-column Python + C
 ``loglikelihood='poisson'`` selects the built-in Poisson likelihood of examples/poisson_tensor_filtering.py
 (``nansum(poisson.logpmf(Y, W V^T))`` over the replicates).  ``loglikelihood='binomial'`` selects the built-in Binomial
 likelihood of successes out of trials, ``data = (Y, Ntrials)``, whose success probability is the surface p = W V^T
-itself (``nansum(binom.logpmf(Y, Ntrials, W V^T))``; the constraints keep p in [0, 1] and give it its shape).  With
-either, the whole sweep -- sigma2, Tau2, lam2, the W and V centres and proposals, and one GASS transition per row and
-per column -- runs inside the engine (gass_kernels.cu), so
+itself (``nansum(binom.logpmf(Y, Ntrials, W V^T))``; the constraints keep p in [0, 1] and give it its shape).
+``loglikelihood='gaussian'`` selects the Gaussian likelihood ``nansum(norm.logpdf(Y, W V^T, sqrt(nu2)))`` over the
+replicates, for continuous responses with a shape-constrained mean; its noise variance ``nu2`` takes the arguments
+and rules of GaussianBayesianTensorFiltering (``nu2_init``, ``nu2_true``, ``nu2_a``, ``nu2_b``): a scalar sampled from
+its conjugate conditional at the start of every sweep, a fixed scalar, or fixed known per-cell variances [N, M, T].
+It needs at least one constraint (on the tensor or on the rows of W): without any, W and V have Gaussian conditionals,
+which GaussianBayesianTensorFiltering draws exactly, so the slice sampler would only mix more slowly; that
+combination raises ValueError.  With any of the three built-in likelihoods, the whole sweep -- (nu2,) sigma2, Tau2, lam2, the W and V centres and proposals, and one GASS
+transition per row and per column -- runs inside the engine (gass_kernels.cu), so
 ``run_gibbs`` runs in ``btf_run_segment`` pieces (or a CUDA graph) and ``HeldOutEvaluator``, ``track_mu``,
 ``results_dir`` and checkpoints work as for the conjugate models.  Its random choices are Philox draws of the engine,
 not ``np.random``.  Single GPU.
@@ -33,15 +39,15 @@ import numpy as np
 from scipy.stats import binom, norm, poisson
 
 from . import _lib as L
-from .factor import BayesianTensorFiltering, _BayesianModel
+from .factor import BayesianTensorFiltering, _BayesianModel, _GaussianNoise
 from .gass import gass, FINE_GRID
 
 
-class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
+class ConstrainedNonconjugateBayesianTensorFiltering(_GaussianNoise, BayesianTensorFiltering):
     # the engine runs in its f64-weight mode: weights = 1/Sigma_ep^2 are injected as "omega"
     _likelihood = L.BINOMIAL
     # the built-in likelihoods, whose GASS steps run on the device
-    _BUILTIN = {'poisson': L.POISSON, 'binomial': L.CBINOMIAL}
+    _BUILTIN = {'poisson': L.POISSON, 'binomial': L.CBINOMIAL, 'gaussian': L.CGAUSSIAN}
 
     def __init__(self, nrows, ncols, ndepth, loglikelihood, Constraints, ep_approx=None, nthreads=3,
                  gass_ngrid=100, Row_constraints=None, multiprocessing=True, sharedprefix=None,
@@ -49,12 +55,17 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
         self._builtin = loglikelihood if isinstance(loglikelihood, str) else None
         if self._builtin is not None:
             if loglikelihood not in self._BUILTIN:
-                raise ValueError("loglikelihood must be a callable, 'poisson' or 'binomial', got %r" % (loglikelihood,))
+                raise ValueError("loglikelihood must be a callable, 'poisson', 'binomial' or 'gaussian', got %r"
+                                 % (loglikelihood,))
             self._likelihood = self._BUILTIN[loglikelihood]
         self.loglikelihood = loglikelihood
         Constraints = np.asarray(Constraints, dtype=float)
         self.Constraints_A, self.Constraints_C = Constraints[:, :-1], Constraints[:, -1:]
         self.nconstraints = self.Constraints_A.shape[0]
+        if self._builtin == 'gaussian' and self.nconstraints == 0 and (
+                Row_constraints is None or np.size(Row_constraints) == 0):
+            raise ValueError("loglikelihood='gaussian' without any constraint is the conjugate Gaussian model: use "
+                             "GaussianBayesianTensorFiltering, which draws W and V from their exact conditionals")
         self.nthreads, self.gass_ngrid = nthreads, gass_ngrid
         self.Row_constraints = Row_constraints
         self.multiprocessing, self.sharedprefix = multiprocessing, sharedprefix
@@ -70,8 +81,13 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
             worker_init(self)
 
     # ---- engine configuration
+    def _gaussian_noise(self):
+        return self._builtin == 'gaussian'      # nu2 (_GaussianNoise) exists for the built-in Gaussian likelihood only
+
     def _likelihood_options(self):
-        return dict(clip_prior_precision=1)
+        opts = super()._likelihood_options()
+        opts.update(clip_prior_precision=1)
+        return opts
 
     def shutdown(self):
         """Nothing to release: the reference tears down its worker pool and shared memory here
@@ -139,20 +155,20 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
                 self._engine.set_data_binomial(Y, Nt)
                 self._data_key = key
             self._sync_gass()
-        elif self._builtin == 'poisson':
+        elif self._builtin in ('poisson', 'gaussian'):
             Y = np.asarray(data)
             assert Y.ndim in (3, 4), 'Observations must be a 3- or 4-tensor.'
             key = self._fingerprint(data, getattr(self, '_full_check', False))
             self._data_nbytes = int(Y.nbytes)
             if key != self._data_key:
                 self._data_key = None
-                self._engine.set_data_poisson(Y)
+                if self._builtin == 'poisson':
+                    self._engine.set_data_poisson(Y)
+                else:
+                    self._engine.set_data_gaussian(Y)
                 self._data_key = key
             self._sync_gass()
         self._sync_ep()
-
-    def _scalar_names(self):
-        return ['sigma2', 'lam2', 'lam2_a']
 
     # ---- batched Gaussian centres / proposals from the engine
     def _engine_step(self, mask, z_name=None, z=None):
@@ -278,7 +294,7 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
 
     def _finish_results(self, results):
         results = super()._finish_results(results)
-        results.pop('_nu2_scalar')
+        results.pop('_nu2_scalar', None)         # (the built-in Gaussian likelihood has made it results['nu2'])
         return results
 
     def logprob(self, data, **kwargs):
@@ -292,6 +308,12 @@ class ConstrainedNonconjugateBayesianTensorFiltering(BayesianTensorFiltering):
                 Y = np.asarray(data)
                 if Y.ndim > tau.ndim:
                     tau = tau[..., None]
+                if self._builtin == 'gaussian':
+                    nu2 = np.asarray(self.nu2, dtype=float)
+                    if nu2.ndim and Y.ndim > nu2.ndim:
+                        nu2 = nu2[..., None]
+                    Y = np.where(np.isinf(nu2), np.nan, Y)          # a known variance of +inf: the cell is missing
+                    return np.nansum(norm.logpdf(Y, tau, np.sqrt(nu2)))
                 return np.nansum(poisson.logpmf(Y, tau))
         return self.loglikelihood(data, tau, self.W, self.V)
 

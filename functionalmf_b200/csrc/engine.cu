@@ -96,16 +96,17 @@ struct btf_engine {
     double *nu2c = nullptr, *wc = nullptr, *sc = nullptr;      // [nloc_pad][Ppad], allocated on first use
     unsigned long long* nu2_nbad = nullptr;
     StatsPlan plan_row_w{}, plan_col_w{};                      // statistics plans for those f64 weights
-    // Constrained Poisson and Binomial models (GASS steps, gass_kernels.cu; single GPU).  With an EP approximation the
-    // W / V centres come from the f64-weight statistics of wc = 1 / sigma^2 and sc = mu / sigma^2 (the buffers of the
-    // per-cell nu2 mode)
+    // Constrained Poisson, Binomial and Gaussian models (GASS steps, gass_kernels.cu; single GPU).  With an EP
+    // approximation the W / V centres come from the f64-weight statistics of wc = 1 / sigma^2 and sc = mu / sigma^2 (the
+    // buffers of the per-cell nu2 mode; a constrained Gaussian engine keeps its known variances in nu2c alone)
     bool gass_set = false, ep_on = false;
     int gJ = 0, gnrc = 0, gnfine = 0, gngrid = 0;
     double *gA = nullptr, *gC = nullptr, *growc = nullptr, *ggrid_f = nullptr, *ggrid_c = nullptr;
     double *Wold = nullptr, *Vold = nullptr, *gmeanW = nullptr, *gmeanV = nullptr;   // the state before the step, the centres
     double *ep_mu = nullptr, *ep_sig = nullptr;                // [nloc_pad][Ppad]
     double* lgy = nullptr;                                     // [nloc_pad][Ppad] Poisson: sum of lgamma(y + 1) over the observed
-                                                               // replicates; Binomial: the log binomial coefficient
+                                                               // replicates; Binomial: the log binomial coefficient;
+                                                               // Gaussian: sum (y - ybar)^2 over the observed replicates
     int* gass_nbad = nullptr;                                  // [2] rows / columns whose starting point violates a constraint
     int nreps = 1;
     bool has_data = false, data_reduced = false;
@@ -171,7 +172,8 @@ struct btf_engine {
 static int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 // the likelihoods whose W and V steps are GASS transitions (gass_kernels.cu)
-static bool gass_likelihood(int lik) { return lik == BTF_POISSON || lik == BTF_CBINOMIAL; }
+static bool gass_likelihood(int lik) { return lik == BTF_POISSON || lik == BTF_CBINOMIAL || lik == BTF_CGAUSSIAN; }
+static const char* gass_name(int lik) { return lik == BTF_POISSON ? "Poisson" : lik == BTF_CBINOMIAL ? "Binomial" : "Gaussian"; }
 
 void btf_config_default(btf_config* c) {
     memset(c, 0, sizeof(*c));
@@ -276,9 +278,9 @@ int btf_create(const btf_config* c, btf_engine** out) {
     if (c->nembeds < 1 || c->nembeds > 32) return set_err(BTF_EINVAL, "nembeds must be in [1, 32]");
     if (c->tf_order < 0 || c->tf_order > 3) return set_err(BTF_EINVAL, "tf_order must be in [0, 3]");
     if (c->ndepth < c->tf_order + 2) return set_err(BTF_EINVAL, "ndepth must be >= tf_order + 2");
-    if (c->likelihood < BTF_GAUSSIAN || c->likelihood > BTF_CBINOMIAL) return set_err(BTF_EINVAL, "unknown likelihood %d", c->likelihood);
+    if (c->likelihood < BTF_GAUSSIAN || c->likelihood > BTF_CGAUSSIAN) return set_err(BTF_EINVAL, "unknown likelihood %d", c->likelihood);
     if (gass_likelihood(c->likelihood) && c->world_size > 1)
-        return set_err(BTF_EINVAL, "the constrained %s model is single-GPU", c->likelihood == BTF_POISSON ? "Poisson" : "Binomial");
+        return set_err(BTF_EINVAL, "the constrained %s model is single-GPU", gass_name(c->likelihood));
     btf_engine* e = new btf_engine();
     // every early return below releases what has been created so far (streams, events, device buffers)
     struct Guard { btf_engine* e; ~Guard() { if (e) btf_destroy(e); } } guard{e};
@@ -440,7 +442,8 @@ int btf_create(const btf_config* c, btf_engine** out) {
 
 // the statistics plan of the rows (col = false) or columns: count weights, or f64 weights with per-cell variances
 static const StatsPlan& stats_plan(const btf_engine* e, bool col) {
-    if (e->nu2_cells) return col ? e->plan_col_w : e->plan_row_w;
+    // (a constrained Gaussian engine's variances do not enter the statistics: its f64 weights are the EP approximation's)
+    if (e->nu2_cells && e->cfg.likelihood == BTF_GAUSSIAN) return col ? e->plan_col_w : e->plan_row_w;
     return col ? e->plan_col : e->plan_row;
 }
 
@@ -550,6 +553,8 @@ static int set_data_compact(btf_engine* e, const double* Y, int32_t row0, int32_
 int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int32_t nrows, int32_t nreps,
                                int32_t reset) {
     if (!e || !Y || nreps < 1 || nreps > 255) return set_err(BTF_EINVAL, "bad arguments (1 <= nreps <= 255)");
+    if (e->cfg.likelihood == BTF_CGAUSSIAN)
+        return set_err(BTF_ESTATE, "a constrained Gaussian engine takes its data whole: use btf_set_data_gaussian");
     if (e->cfg.likelihood != BTF_GAUSSIAN) return set_err(BTF_ESTATE, "engine is not Gaussian");
     return set_data_compact(e, Y, row0, nrows, nreps, reset);
 }
@@ -626,12 +631,52 @@ static int set_data_compact(btf_engine* e, const double* Y, int32_t row0, int32_
     return BTF_OK;
 }
 
-int btf_set_data_gaussian(btf_engine* e, const double* Y, int32_t nreps) {
-    if (!e) return set_err(BTF_EINVAL, "null engine");
-    return btf_set_data_gaussian_rows(e, Y, 0, e->nloc, nreps, 1);
+static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host);
+
+// The constrained Gaussian model: observations [Nloc, M, T, nreps] in the compact form, plus the within-cell sum of
+// squared deviations ss = sum_r (y_r - ybar)^2 per cell, so that the GASS steps evaluate the log-likelihood in its
+// centred form.  Every observed value must be finite.
+static int set_data_cgaussian(btf_engine* e, const double* Y, int32_t nreps) {
+    if (!Y || nreps < 1 || nreps > 255) return set_err(BTF_EINVAL, "bad arguments (1 <= nreps <= 255)");
+    CK(cudaSetDevice(e->cfg.device));
+    const size_t cells = (size_t)e->nloc * e->P, total = cells * nreps;
+    std::vector<double> hcopy;
+    const double* hy = Y;
+    if (is_device_ptr(Y)) {
+        hcopy.resize(total);
+        CK(cudaMemcpy(hcopy.data(), Y, total * sizeof(double), cudaMemcpyDeviceToHost));
+        hy = hcopy.data();
+    }
+    unsigned long long nbad = 0;
+    std::vector<double> ss(cells, 0.0);
+    for (size_t c = 0; c < cells; ++c) {
+        const double* y = hy + c * nreps;
+        int n = 0;
+        double sum = 0.0;
+        for (int r = 0; r < nreps; ++r) {
+            if (std::isnan(y[r])) continue;
+            if (!std::isfinite(y[r])) { ++nbad; continue; }
+            ++n; sum += y[r];
+        }
+        if (n < 2) continue;
+        const double ybar = sum / n;
+        double q = 0.0;
+        for (int r = 0; r < nreps; ++r)
+            if (std::isfinite(y[r])) q += (y[r] - ybar) * (y[r] - ybar);
+        ss[c] = q;
+    }
+    if (nbad) return set_err(BTF_EINVAL, "%llu observed value(s) are not finite", nbad);
+    if (!e->lgy) CK(dev_alloc(&e->lgy, (size_t)e->nloc_pad * e->Ppad));
+    CK(cudaStreamSynchronize(e->stream));
+    { int rc = copy_pitched(e, e->lgy, ss.data(), false); if (rc) return rc; }
+    return set_data_compact(e, Y, 0, e->nloc, nreps, 1);
 }
 
-static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host);
+int btf_set_data_gaussian(btf_engine* e, const double* Y, int32_t nreps) {
+    if (!e) return set_err(BTF_EINVAL, "null engine");
+    if (e->cfg.likelihood == BTF_CGAUSSIAN) return set_data_cgaussian(e, Y, nreps);
+    return btf_set_data_gaussian_rows(e, Y, 0, e->nloc, nreps, 1);
+}
 
 // Poisson counts [Nloc, M, T, nreps] in the compact form of the Gaussian data, plus sum_r lgamma(y_r + 1) per cell
 // (scipy's logpmf keeps it, and a cell whose rate is negative drops out of the log-likelihood together with it).
@@ -778,6 +823,11 @@ int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps) {
 // Known per-cell noise variances (the reference's heteroskedastic Gaussian branch: nu2 an [N, M, T] array).
 // First use: the statistics plans for f64 weights (their split buffers may be larger) and the cell buffers.
 static int ensure_nu2_buffers(btf_engine* e) {
+    if (e->cfg.likelihood == BTF_CGAUSSIAN) {
+        // the GASS steps read the variances themselves; wc / sc belong to the EP approximation
+        if (!e->nu2c) { CK(dev_alloc(&e->nu2_nbad, 1)); CK(dev_alloc(&e->nu2c, (size_t)e->nloc_pad * e->Ppad)); }
+        return BTF_OK;
+    }
     if (e->wc) return BTF_OK;
     if (!plan_stats(&e->plan_row_w, e->K, false, true, e->nloc_pad, e->Ppad, e->nloc, e->cfg.stats_splits_row, e->sm_count) ||
         !plan_stats(&e->plan_col_w, e->K, true, true, e->Ppad, e->nloc_pad, e->P, e->cfg.stats_splits_col, e->sm_count))
@@ -799,10 +849,12 @@ static int ensure_nu2_buffers(btf_engine* e) {
 }
 
 // Weights from `rows` rows of variances at pitch lds (starting at local row row0); keep != 0: store the variances too.
+// A constrained Gaussian engine forms no weights (its wc / sc hold the EP approximation's): it only checks and keeps.
 static void enqueue_nu2_weights(btf_engine* e, const double* nu2, long long lds, int row0, int rows, bool keep) {
     const size_t o = (size_t)row0 * e->Ppad;
-    launch_nu2_weights(nu2, lds, rows, e->P, e->cnt + o, e->S + o, e->Ppad, keep ? e->nu2c + o : nullptr, e->wc + o,
-                       e->sc + o, e->nu2_nbad, e->stream);
+    const bool weights = e->cfg.likelihood == BTF_GAUSSIAN;
+    launch_nu2_weights(nu2, lds, rows, e->P, e->cnt + o, e->S + o, e->Ppad, keep ? e->nu2c + o : nullptr,
+                       weights ? e->wc + o : nullptr, weights ? e->sc + o : nullptr, e->nu2_nbad, e->stream);
     e->launches++;
 }
 
@@ -821,7 +873,8 @@ static int nu2_bad_error(btf_engine* e) {
 
 int btf_set_nu2_cells(btf_engine* e, const double* nu2) {
     if (!e) return set_err(BTF_EINVAL, "null engine");
-    if (e->cfg.likelihood != BTF_GAUSSIAN) return set_err(BTF_ESTATE, "per-cell noise variances need a Gaussian engine");
+    if (e->cfg.likelihood != BTF_GAUSSIAN && e->cfg.likelihood != BTF_CGAUSSIAN)
+        return set_err(BTF_ESTATE, "per-cell noise variances need a Gaussian or constrained Gaussian engine");
     if (e->cfg.world_size > 1) return set_err(BTF_EINVAL, "per-cell noise variances are single-GPU");
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaStreamSynchronize(e->stream));
@@ -869,7 +922,7 @@ static int copy_pitched(btf_engine* e, double* dev, double* host, bool to_host) 
     return BTF_OK;
 }
 
-// ------------------------------------------------------------------ constrained Poisson and Binomial models (GASS steps)
+// ------------------------------------------------------------------ constrained Poisson, Binomial and Gaussian models (GASS steps)
 static cudaError_t upload_copy(double** dst, const double* src, size_t n) {
     if (*dst) { cudaFree(*dst); *dst = nullptr; }
     cudaError_t ce = dev_alloc(dst, std::max<size_t>(n, 1), false);
@@ -880,7 +933,7 @@ static cudaError_t upload_copy(double** dst, const double* src, size_t n) {
 int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, const double* rowcons, int32_t nrowcons,
                  const double* grid_fine, int32_t ngrid_fine, const double* grid_coarse, int32_t ngrid) {
     if (!e) return set_err(BTF_EINVAL, "null engine");
-    if (!gass_likelihood(e->cfg.likelihood)) return set_err(BTF_ESTATE, "GASS steps need a constrained Poisson or Binomial engine");
+    if (!gass_likelihood(e->cfg.likelihood)) return set_err(BTF_ESTATE, "GASS steps need a constrained Poisson, Binomial or Gaussian engine");
     if (J < 0 || nrowcons < 0 || (J > 0 && (!A || !C)) || (nrowcons > 0 && !rowcons))
         return set_err(BTF_EINVAL, "constraints: J >= 0 rows of A [J, T] and C [J], nrowcons >= 0 rows of [K + 1]");
     if (!grid_fine || !grid_coarse || ngrid < 1 || ngrid > ngrid_fine || ngrid_fine > 65535)
@@ -924,7 +977,7 @@ int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, con
 // EP approximation N(mu, sigma^2) per cell (host memory, [Nloc, M, T]); NULL: none
 int btf_set_ep(btf_engine* e, const double* mu, const double* sigma) {
     if (!e) return set_err(BTF_EINVAL, "null engine");
-    if (!gass_likelihood(e->cfg.likelihood)) return set_err(BTF_ESTATE, "an EP approximation needs a constrained Poisson or Binomial engine");
+    if (!gass_likelihood(e->cfg.likelihood)) return set_err(BTF_ESTATE, "an EP approximation needs a constrained Poisson, Binomial or Gaussian engine");
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaStreamSynchronize(e->stream));
     if (!mu || !sigma) {
@@ -1405,6 +1458,8 @@ static GassArgs gass_args(btf_engine* e, bool col) {
     g.N = e->N; g.M = e->M; g.T = e->T; g.K = e->K; g.P = e->P; g.ld = e->Ppad;
     g.cnt = e->cnt; g.S = e->S; g.lgy = e->lgy; g.ntr = e->ntr;
     g.binomial = e->cfg.likelihood == BTF_CBINOMIAL;
+    g.gaussian = e->cfg.likelihood == BTF_CGAUSSIAN;
+    g.nu2c = e->nu2_cells ? e->nu2c : nullptr;
     g.ep_mu = e->ep_on ? e->ep_mu : nullptr; g.ep_sig = e->ep_on ? e->ep_sig : nullptr;
     g.A = e->gA; g.C = e->gC; g.J = e->gJ; g.rowcons = e->growc; g.nrc = e->gnrc;
     g.grid_fine = e->ggrid_f; g.nfine = e->gnfine; g.grid_coarse = e->ggrid_c; g.ngrid = e->gngrid;
@@ -1445,6 +1500,7 @@ static int enqueue_sweep(btf_engine* e) {
     const btf_config& c = e->cfg;
     cudaStream_t st = e->stream;
     const bool gauss = c.likelihood == BTF_GAUSSIAN;
+    const bool cgauss = c.likelihood == BTF_CGAUSSIAN;
     // known per-cell variances: the PG models' f64-weight route, with weights cnt / nu2 and right-hand side S / nu2
     const bool percell = gauss && e->nu2_cells;
     const bool homo = gauss && !percell;      // one scalar nu2 scales the statistics
@@ -1470,9 +1526,10 @@ static int enqueue_sweep(btf_engine* e) {
         nb.hist = e->nb_hist; nb.hist_stride = e->nb_hist_stride;
         launch_nb_update(nb, st); e->launches += nb.nmh > 0 ? (nb.hist ? 4 : 2 * nb.nmh + 4) : 1;
     }
-    if (gauss) {
+    if (gauss || cgauss) {
         if (mask & BTF_SAMPLE_NU2) {
-            if (!e->resid_valid || c.resid_direct) {
+            // constrained Gaussian: the GASS steps leave no residual by-product, so the direct pass runs every sweep
+            if (!e->resid_valid || c.resid_direct || cgauss) {
                 int nb = 0;
                 launch_residual(e->cnt, e->S, e->Ppad, e->W + (size_t)c.row_begin * e->K, e->V, e->nloc_pad, e->Ppad,
                                 e->K, e->partials, &nb, st);

@@ -1,5 +1,5 @@
 // GASS: generalized analytic slice sampling of the constrained model's W rows and V columns under a built-in
-// likelihood, Poisson or Binomial (functionalmf_b200/gass.py, factor.py:665-892).  One CTA per row or column:
+// likelihood, Poisson, Binomial or Gaussian (functionalmf_b200/gass.py, factor.py:665-892).  One CTA per row or column:
 //   1. the constraint products a = A(x - mu), b = A v, c = C - A mu of every constraint row, without the Kronecker
 //      matrix (rows: coefficients sum_t A[c,t] V[j,t,:]; columns: A[c,t] W[i,:]);
 //   2. the feasible grid of gass.feasible_angles: "outside" intervals are removed as index ranges through a difference
@@ -131,6 +131,30 @@ struct BinomialLik {
         return c;
     }
     static __device__ __forceinline__ double ll(double p, const Cell& c) { return c.obs ? binomial_cell(p, c.y, c.n, c.lc) : 0.0; }
+};
+// scipy.stats.norm.logpdf(y, tau, sigma) summed over the n observed replicates of a cell, in the centred form
+// -n log sigma - n log sqrt(2 pi) - (ss + n (ybar - tau)^2) / (2 sigma^2) with ss = sum (y - ybar)^2: expanding the
+// square instead (sum y^2 - 2 tau sum y + n tau^2) cancels badly when |y| is large against the noise, and which
+// candidates clear the slice depends on the value.  The variance is the scalar nu2 or the cell's known variance; a cell
+// with n = 0 or an infinite variance (missing) contributes 0.  Evaluated without fused operations.
+struct GaussianLik {
+    struct Cell { double n, ybar, ss, c0, tv; };    // n = 0: not observed; c0 = -n (log sigma + log sqrt(2 pi)), tv = 2 sigma^2
+    static __device__ __forceinline__ Cell load(const GassArgs& a, size_t cell) {
+        Cell c;
+        const int n = a.cnt[cell];
+        const double var = a.nu2c ? a.nu2c[cell] : a.scal->nu2;
+        c.n = n > 0 && var < INFINITY ? (double)n : 0.0;
+        c.ybar = n > 0 ? a.S[cell] / n : 0.0;
+        c.ss = a.lgy[cell];
+        c.c0 = -mul(c.n, add(0.5 * log(var), LOG_SQRT_2PI));
+        c.tv = 2.0 * var;
+        return c;
+    }
+    static __device__ __forceinline__ double ll(double tau, const Cell& c) {
+        if (c.n == 0.0) return 0.0;
+        const double d = add(c.ybar, -tau);
+        return add(c.c0, -(add(c.ss, mul(c.n, mul(d, d))) / c.tv));
+    }
 };
 
 // scipy.stats.norm.logpdf(lam, mu, sigma)
@@ -414,7 +438,8 @@ static void launch_gass_lik(const GassArgs& a, cudaStream_t st) {
 }
 
 void launch_gass(const GassArgs& a, cudaStream_t st) {
-    if (a.binomial) launch_gass_lik<BinomialLik>(a, st);
+    if (a.gaussian) launch_gass_lik<GaussianLik>(a, st);
+    else if (a.binomial) launch_gass_lik<BinomialLik>(a, st);
     else launch_gass_lik<PoissonLik>(a, st);
 }
 

@@ -266,15 +266,16 @@ void launch_nb_hist(const NbArgs& a, int vstride, cudaStream_t st);
 // (factor.py:513-554, 494-511)
 void launch_nb_update(const NbArgs& a, cudaStream_t st);
 
-// ---------------------------------------------------------------- GASS steps of the constrained Poisson and Binomial
-// models (gass_kernels.cu)
+// ---------------------------------------------------------------- GASS steps of the constrained Poisson, Binomial and
+// Gaussian models (gass_kernels.cu)
 struct GassArgs {
     bool col;                                   // false: one CTA per W row (gass_row_kernel), true: per V column (gass_col_kernel)
     int N, M, T, K, P; long long ld;
-    const uint8_t* cnt; const double* S;        // Poisson: observed replicates and their sum; Binomial: observed flag and
-                                                // kappa = y - n/2, [N][ld]
+    const uint8_t* cnt; const double* S;        // Poisson, Gaussian: observed replicates and their sum; Binomial: observed
+                                                // flag and kappa = y - n/2, [N][ld]
     const double* lgy;                          // Poisson: sum of lgamma(y + 1) over the observed replicates; Binomial: the
-                                                // log binomial coefficient lgamma(n + 1) - (lgamma(y + 1) + lgamma(n - y + 1)), [N][ld]
+                                                // log binomial coefficient lgamma(n + 1) - (lgamma(y + 1) + lgamma(n - y + 1));
+                                                // Gaussian: sum (y - ybar)^2 over the observed replicates, [N][ld]
     const double *ep_mu, *ep_sig;               // EP approximation [N][ld], or nullptr
     const double* A; const double* C; int J;    // constraints A[c] . Mu[i, j, :] >= C[c], A [J][T]
     const double* rowcons; int nrc;             // row constraints [nrc][K + 1] (W rows only)
@@ -291,6 +292,8 @@ struct GassArgs {
     // (appended, so that the Poisson kernels read every field above at the offsets they always had)
     const double* ntr;                          // Binomial: trials n, [N][ld]
     bool binomial;                              // the cell likelihood: false Poisson, true Binomial
+    const double* nu2c;                         // Gaussian: known per-cell variances [N][ld], or nullptr (the scalar nu2)
+    bool gaussian;                              // the cell likelihood is Gaussian (then binomial is false)
 };
 size_t gass_smem_bytes(int D, int nfine, int ngrid);
 void launch_gass(const GassArgs& a, cudaStream_t st);

@@ -85,7 +85,8 @@ void launch_prereduce_binomial(const double* Y, const double* Nt, int rows, int 
 
 // Known per-cell noise variances (the reference's heteroskedastic Gaussian branch, factor.py:345-346 and 390-391
 // with an [N, M, T] nu2): weight w = cnt / nu2 and right-hand side S / nu2 of the statistics, both 0 where nothing is
-// observed or nu2 = +inf (such a cell counts as missing).  Observed cells whose variance is NaN or <= 0 are counted.
+// observed or nu2 = +inf (such a cell counts as missing); w = s = nullptr: no weights (the constrained Gaussian model,
+// whose GASS steps read the variances).  Observed cells whose variance is NaN or <= 0 are counted.
 __global__ void nu2_weights_kernel(const double* __restrict__ nu2, long long lds, int rows, int P,
                                    const uint8_t* __restrict__ cnt, const double* __restrict__ S, long long ld,
                                    double* __restrict__ keep, double* __restrict__ w, double* __restrict__ s,
@@ -100,8 +101,10 @@ __global__ void nu2_weights_kernel(const double* __restrict__ nu2, long long lds
         const double c = (double)cnt[o];
         const bool on = c > 0.0 && v < INFINITY;
         bad += (c > 0.0 && !(v > 0.0)) ? 1u : 0u;
-        w[o] = on ? c / v : 0.0;
-        s[o] = on ? S[o] / v : 0.0;
+        if (w) {
+            w[o] = on ? c / v : 0.0;
+            s[o] = on ? S[o] / v : 0.0;
+        }
         if (keep) keep[o] = v;
     }
     for (int d = 16; d > 0; d >>= 1) bad += __shfl_down_sync(0xffffffffu, bad, d);

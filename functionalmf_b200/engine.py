@@ -123,7 +123,8 @@ class Engine(object):
         L.check(self.lib.btf_set_data_negbin(self._h, _ptr(Y), Y.shape[3]))
 
     def set_nu2_cells(self, nu2):
-        """Known per-cell noise variances [Nloc, M, T] of a Gaussian engine (``None``: back to the scalar nu2)."""
+        """Known per-cell noise variances [Nloc, M, T] of a Gaussian or constrained Gaussian engine (``None``: back to
+        the scalar nu2)."""
         a = None
         if nu2 is not None:
             a = _f64(nu2)
@@ -156,7 +157,7 @@ class Engine(object):
                                       _ptr(gf), gf.size, _ptr(gc), gc.size))
 
     def set_ep(self, mu, sigma):
-        """EP approximation N(mu, sigma^2) per cell [Nloc, M, T] of a constrained Poisson or Binomial engine
+        """EP approximation N(mu, sigma^2) per cell [Nloc, M, T] of a constrained Poisson, Binomial or Gaussian engine
         (``None``: none)."""
         if mu is None:
             L.check(self.lib.btf_set_ep(self._h, C.c_void_p(0), C.c_void_p(0)))

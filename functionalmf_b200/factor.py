@@ -15,7 +15,7 @@ Differences, all deliberate (SURVEY.md appendix D):
 * ``lam2`` follows the reference as written (last column only, Q1) unless
   ``ref_compat=False``;
 * with known per-cell noise variances (Gaussian ``nu2`` an [N, M, T] array held
-  fixed), ``run_gibbs`` returns ``results['nu2']`` as a read-only
+  fixed, also for the constrained model's ``'gaussian'`` likelihood), ``run_gibbs`` returns ``results['nu2']`` as a read-only
   ``np.broadcast_to`` view [nsamples, N, M, T] of that one array, not nsamples
   copies.
 """
@@ -425,15 +425,18 @@ class BayesianTensorFiltering(_BayesianModel):
         return self._engine.kernel_launches
 
 
-class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
-    """factor.py:286-423.
+class _GaussianNoise(object):
+    """The noise variance ``nu2`` of a Gaussian likelihood (factor.py:286-423), shared by
+    GaussianBayesianTensorFiltering and the constrained model's built-in ``'gaussian'`` likelihood.
 
     ``nu2`` is a scalar, or an [N, M, T] array of known per-cell noise variances (the reference's heteroskedastic
     branch, e.g. per-cell standard errors squared): when ``model.nu2`` has that shape and ``sample_nu2`` is False
-    (``nu2_true=array``), the W and V steps weight every cell by cnt / nu2[n, m, t].  A variance of +inf makes an
-    observed cell count as missing; NaN or <= 0 at an observed cell is refused.  With ``sample_nu2`` True the nu2
-    step draws a scalar from the residual like the reference's ``_resample_nu2``.  Single GPU only."""
-    _likelihood = L.GAUSSIAN
+    (``nu2_true=array``), every cell is weighted by its own variance.  A variance of +inf makes an observed cell count
+    as missing; NaN or <= 0 at an observed cell is refused.  With ``sample_nu2`` True the nu2 step draws a scalar from
+    the residual like the reference's ``_resample_nu2``.  Single GPU only.
+
+    A class that mixes this in and has other likelihoods too answers ``_gaussian_noise()`` with False for them: every
+    hook below then defers to the next class in the MRO."""
 
     def __init__(self, nrows, ncols, ndepth, nu2_init=None, nu2_true=None, nu2_a=0.1, nu2_b=0.1, **kwargs):
         self.nu2_a, self.nu2_b = nu2_a, nu2_b
@@ -441,31 +444,48 @@ class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
         self._nu2_key = None          # fingerprint of the per-cell variances on the device, None in scalar mode
         super().__init__(nrows, ncols, ndepth, **kwargs)
         fixed = nu2_true if nu2_true is not None else nu2_init
-        if self._likelihood == L.GAUSSIAN and fixed is not None and np.size(fixed) != 1:
+        if self._nu2_cells_model() and fixed is not None and np.size(fixed) != 1:
             self.nu2 = np.asarray(fixed, dtype=np.float64)     # uploaded by the first sweep that uses it
 
+    def _gaussian_noise(self):
+        return True
+
+    def _nu2_cells_model(self):
+        """May nu2 be an array of known per-cell variances?  (The PG models' nu2 is the per-cell 1/omega they redraw
+        every sweep.)"""
+        return self._likelihood in (L.GAUSSIAN, L.CGAUSSIAN)
+
     def _likelihood_options(self):
-        return dict(nu2_a=self.nu2_a, nu2_b=self.nu2_b)
+        opts = super()._likelihood_options()
+        if self._gaussian_noise():
+            opts.update(nu2_a=self.nu2_a, nu2_b=self.nu2_b)
+        return opts
 
     def _extra_init_mask(self):
+        if not self._gaussian_noise():
+            return super()._extra_init_mask()
         nu2_init, nu2_true = self._nu2_args
         self.sample_nu2 = nu2_true is None
         return L.INIT_NU2 if (nu2_init is None and nu2_true is None) else 0
 
     def _after_base_init(self):
+        if not self._gaussian_noise():
+            return super()._after_base_init()
         nu2_init, nu2_true = self._nu2_args
         fixed = nu2_true if nu2_true is not None else nu2_init
-        if fixed is None or (self._likelihood == L.GAUSSIAN and np.size(fixed) != 1):
+        if fixed is None or (self._nu2_cells_model() and np.size(fixed) != 1):
             return
         self._engine.set('nu2', [fixed])
 
     def _scalar_names(self):
-        names = ['sigma2', 'lam2', 'lam2_a']
+        names = super()._scalar_names()
+        if not self._gaussian_noise():
+            return names
         return names if self._nu2_per_cell() is not None else names + ['nu2']
 
     def _nu2_per_cell(self):
-        if self._likelihood != L.GAUSSIAN:
-            return None               # (the PG models' nu2 is the per-cell 1/omega they redraw every sweep)
+        if not (self._gaussian_noise() and self._nu2_cells_model()):
+            return super()._nu2_per_cell()
         nu2 = getattr(self, 'nu2', None)
         if np.size(nu2) == 1:
             return None
@@ -478,6 +498,8 @@ class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
 
     def _push_state(self):
         super()._push_state()
+        if not self._gaussian_noise():
+            return
         cells = self._nu2_per_cell()
         # re-uploaded only when the variances changed (same rule as the data, see _fingerprint)
         key = None if cells is None else self._fingerprint(cells, getattr(self, '_full_check', False))
@@ -486,21 +508,14 @@ class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
             self._engine.set_nu2_cells(None if cells is None else self._local_rows(cells))
             self._nu2_key = key
 
-    def _upload(self, data):
-        Y = np.asarray(data)
-        assert len(Y.shape) == 3 or len(Y.shape) == 4, 'Observations must be 3- or 4-tensor.'
-        key = self._fingerprint(data, getattr(self, '_full_check', False))
-        self._data_nbytes = int(np.asarray(data).nbytes)
-        if key != self._data_key:
-            self._engine.set_data_gaussian(self._local_rows(Y))
-            self._data_key = key
-
     def _init_nu2(self):
         self._engine.init_state(L.INIT_NU2)
         self.nu2 = self._engine.get_scalar('nu2')
 
     def _finish_results(self, results):
         results = super()._finish_results(results)
+        if not self._gaussian_noise():
+            return results
         nu2 = results.pop('_nu2_scalar')
         cells = self._nu2_per_cell()
         if cells is not None:
@@ -510,7 +525,23 @@ class GaussianBayesianTensorFiltering(BayesianTensorFiltering):
 
     def _inferred_variables(self, var_map):
         super()._inferred_variables(var_map)
-        var_map['nu2'] = self.nu2
+        if self._gaussian_noise():
+            var_map['nu2'] = self.nu2
+
+
+class GaussianBayesianTensorFiltering(_GaussianNoise, BayesianTensorFiltering):
+    """factor.py:286-423.  ``nu2`` is a scalar or an [N, M, T] array of known per-cell variances (see _GaussianNoise):
+    with the array the W and V steps weight every cell by cnt / nu2[n, m, t]."""
+    _likelihood = L.GAUSSIAN
+
+    def _upload(self, data):
+        Y = np.asarray(data)
+        assert len(Y.shape) == 3 or len(Y.shape) == 4, 'Observations must be 3- or 4-tensor.'
+        key = self._fingerprint(data, getattr(self, '_full_check', False))
+        self._data_nbytes = int(np.asarray(data).nbytes)
+        if key != self._data_key:
+            self._engine.set_data_gaussian(self._local_rows(Y))
+            self._data_key = key
 
 
 class BinomialBayesianTensorFiltering(GaussianBayesianTensorFiltering):

@@ -30,9 +30,10 @@ extern "C" {
 #define BTF_ESTATE       -4   /* call order / missing data */
 #define BTF_ENCCL        -5   /* NCCL error */
 
-/* BTF_POISSON and BTF_CBINOMIAL: the constrained model's built-in likelihoods, whose W and V steps are GASS transitions
- * (Poisson counts; Binomial successes out of trials with the identity link p = W V^T) */
-enum { BTF_GAUSSIAN = 0, BTF_BINOMIAL = 1, BTF_NEGBINOMIAL = 2, BTF_POISSON = 3, BTF_CBINOMIAL = 4 };
+/* BTF_POISSON, BTF_CBINOMIAL and BTF_CGAUSSIAN: the constrained model's built-in likelihoods, whose W and V steps are
+ * GASS transitions (Poisson counts; Binomial successes out of trials with the identity link p = W V^T; Gaussian
+ * observations with mean W V^T and a noise variance nu2 that is sampled, fixed, or known per cell) */
+enum { BTF_GAUSSIAN = 0, BTF_BINOMIAL = 1, BTF_NEGBINOMIAL = 2, BTF_POISSON = 3, BTF_CBINOMIAL = 4, BTF_CGAUSSIAN = 5 };
 
 /* sample_mask bits: which variables resample() updates (factor.py:112-128, 306-311) */
 enum {
@@ -47,7 +48,7 @@ typedef struct btf_engine btf_engine;
 typedef struct btf_config {
     int32_t nrows, ncols, ndepth;      /* global N, M, T */
     int32_t nembeds, tf_order;         /* K, p */
-    int32_t likelihood;                /* BTF_GAUSSIAN / BINOMIAL / NEGBINOMIAL / POISSON / CBINOMIAL */
+    int32_t likelihood;                /* BTF_GAUSSIAN / BINOMIAL / NEGBINOMIAL / POISSON / CBINOMIAL / CGAUSSIAN */
     double  sigma2_a, sigma2_b;        /* factor.py:27 */
     double  nu2_a, nu2_b;              /* factor.py:289 */
     double  stability;                 /* factor.py:32 */
@@ -84,7 +85,8 @@ const char* btf_last_error(void);
  * reference has no such limit; BTF_EINVAL otherwise).  Ordinary (pageable) host memory
  * is copied through pinned bounce buffers by several host threads (DESIGN.md section 2). */
 int btf_set_data_gaussian(btf_engine* e, const double* Y, int32_t nreps);
-/* streaming form: rows [row0, row0+nrows) of the local shard; reset != 0 on the first piece */
+/* streaming form: rows [row0, row0+nrows) of the local shard; reset != 0 on the first piece.  BTF_ESTATE on a
+ * BTF_CGAUSSIAN engine, which takes its data whole through btf_set_data_gaussian. */
 int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int32_t nrows, int32_t nreps,
                                int32_t reset);
 /* Successes and trials [Nloc, M, T] each (a cell is missing where either is NaN).  BTF_BINOMIAL (Polya-Gamma) or
@@ -92,21 +94,23 @@ int btf_set_data_gaussian_rows(btf_engine* e, const double* Y, int32_t row0, int
  * else BTF_EINVAL giving the number of such cells, and nothing changes). */
 int btf_set_data_binomial(btf_engine* e, const double* Ysucc, const double* Ntrials);
 int btf_set_data_negbin(btf_engine* e, const double* Y, int32_t nreps);
-/* Known per-cell noise variances of a Gaussian model: the reference's heteroskedastic branch, nu2 an
+/* Known per-cell noise variances of a Gaussian or constrained Gaussian model: the reference's heteroskedastic branch, nu2 an
  * [N, M, T] array (factor.py:345-346, 390-391; SURVEY.md 3.2).  `nu2` holds the LOCAL rows [Nloc, M, T] in
  * C order, host or device memory; NULL returns to the scalar nu2.  The W and V conditionals then weight
  * cell (i,j,t) by cnt / nu2[i,j,t] with right-hand side S / nu2[i,j,t]; nu2 = +inf makes an observed cell
  * count as missing, and at missing cells any value is accepted.  The weights are formed again after every
  * btf_set_data_gaussian*; the variances are kept on the device (24 B per cell with the two weight buffers).
- * BTF_ESTATE on a non-Gaussian engine, BTF_EINVAL on a sharded one (world_size > 1) and when observed
- * cells have a variance that is NaN or <= 0 (the message gives their number; the engine stays in scalar
- * mode).  While the variances are set, btf_sweep / btf_run* refuse BTF_SAMPLE_NU2 with BTF_ESTATE: the
- * reference holds an array nu2 fixed. */
+ * BTF_ESTATE on an engine that is neither BTF_GAUSSIAN nor BTF_CGAUSSIAN, BTF_EINVAL on a sharded one
+ * (world_size > 1) and when observed cells have a variance that is NaN or <= 0 (the message gives their
+ * number; the engine stays in scalar mode).  While the variances are set, btf_sweep / btf_run* refuse
+ * BTF_SAMPLE_NU2 with BTF_ESTATE: the reference holds an array nu2 fixed.  On a BTF_CGAUSSIAN engine no
+ * weights are formed (the GASS steps read the variances; its weight buffers hold the EP approximation's):
+ * the variances are checked and kept, 8 B per cell. */
 int btf_set_nu2_cells(btf_engine* e, const double* nu2);
 
-/* ---- the constrained Poisson and Binomial models (ConstrainedNonconjugateBayesianTensorFiltering with the Poisson
- * likelihood of examples/poisson_tensor_filtering.py, or a Binomial one; factor.py:894-1017).  A BTF_POISSON or
- * BTF_CBINOMIAL engine runs the whole sweep on the device: sigma2, Tau2, lam2, then for W and for V the Gaussian centre
+/* ---- the constrained Poisson, Binomial and Gaussian models (ConstrainedNonconjugateBayesianTensorFiltering with the
+ * Poisson likelihood of examples/poisson_tensor_filtering.py, a Binomial or a Gaussian one; factor.py:894-1017).  A
+ * BTF_POISSON, BTF_CBINOMIAL or BTF_CGAUSSIAN engine runs the whole sweep on the device: sigma2, Tau2, lam2, then for W and for V the Gaussian centre
  * and proposal (the f64-weight statistics of an EP approximation, or the prior alone) followed by one GASS transition
  * per row / column (gass.py:13-130) under ll = nansum of the cells' log-likelihoods at lambda = W V^T, minus
  * sum_cells norm.logpdf(lambda; mu_ep, sigma_ep) with EP:
@@ -116,6 +120,14 @@ int btf_set_nu2_cells(btf_engine* e, const double* nu2);
  *     and p = 1 with y < n give -inf; n = 0 gives 0).  The data come through btf_set_data_binomial and take 25 B / cell
  *     (observed flag, kappa = y - n/2, n and the log binomial coefficient); btf_set_data_poisson refuses this engine
  *     with BTF_ESTATE, as btf_set_data_binomial refuses a Poisson one.
+ *   Gaussian: scipy.stats.norm.logpdf(y, lambda, sqrt(nu2)) over the observed replicates, evaluated per cell in the
+ *     centred form -n log sqrt(2 pi nu2) - (ss + n (ybar - lambda)^2) / (2 nu2), ss = sum_r (y_r - ybar)^2.  nu2 is the
+ *     scalar state "nu2" or, after btf_set_nu2_cells, the cell's known variance (+inf: the cell is missing).  With
+ *     BTF_SAMPLE_NU2 every sweep starts with the Gaussian model's conjugate nu2 step on the residual of the current
+ *     (W, V), recomputed by a direct pass each sweep.  The data come through btf_set_data_gaussian (btf_set_data_gaussian_rows
+ *     refuses this engine) and take 17 B / cell (count, sum and ss); observed values that are +-inf give BTF_EINVAL with
+ *     their number, and nothing changes.  btf_set_data_poisson and btf_set_data_binomial refuse this engine with
+ *     BTF_ESTATE, as btf_set_data_gaussian refuses the other two.
  * Single GPU: btf_create refuses world_size > 1 for these likelihoods.
  *
  * Counts Y [Nloc, M, T, nreps] (NaN = missing, host or device memory), kept in the Gaussian data's compact form
@@ -131,7 +143,7 @@ int btf_set_data_poisson(btf_engine* e, const double* Y, int32_t nreps);
  * violation, before anything changes. */
 int btf_set_gass(btf_engine* e, const double* A, const double* C, int32_t J, const double* rowcons, int32_t nrowcons,
                  const double* grid_fine, int32_t ngrid_fine, const double* grid_coarse, int32_t ngrid);
-/* EP approximation (host memory, [Nloc, M, T] each; NULL: none) of either model.  The W / V centres come from the weights 1 / sigma^2 and
+/* EP approximation (host memory, [Nloc, M, T] each; NULL: none) of any of these models.  The W / V centres come from the weights 1 / sigma^2 and
  * the right-hand side mu / sigma^2; every candidate's ll subtracts sum norm.logpdf(lambda; mu, sigma) over ALL cells of the
  * row / column.  BTF_EINVAL when a mean is not finite or a scale is not finite and > 0 (with their number). 32 B / cell. */
 int btf_set_ep(btf_engine* e, const double* mu, const double* sigma);

@@ -1,12 +1,14 @@
-"""Sweeps/s of the constrained Poisson or Binomial model (ConstrainedNonconjugateBayesianTensorFiltering):
+"""Sweeps/s of the constrained Poisson, Binomial or Gaussian model (ConstrainedNonconjugateBayesianTensorFiltering):
   politics   19 x 19 x 228, K = 5, p = 2, ngrid = 100 (the shape of politics/benchmark.py): the device path
-             (loglikelihood='poisson' or 'binomial', every step in the engine) and the host path (the same likelihood
-             as a Python callable, GASS on the host), timed alternately in one process;
+             (loglikelihood='poisson', 'binomial' or 'gaussian', every step in the engine) and the host path (the same
+             likelihood as a Python callable, GASS on the host), timed alternately in one process;
   large      1024 x 256 x 64, K = 8, device path only.
 Poisson: synthetic counts from a positive low-rank rate, constraints Mu >= 0.  Binomial: 20 trials per cell, successes
-from a low-rank probability in (0, 0.9], constraints 0 <= Mu <= 1.  Prints the card name and power limit beside the
-numbers.
-usage: python tools/constrained_bench.py [--likelihood poisson] [--rounds 2] [--steps 20] [--host-steps 20]"""
+from a low-rank probability in (0, 0.9], constraints 0 <= Mu <= 1.  Gaussian: the low-rank surface plus noise of sd
+0.1, constraints Mu non-decreasing in t; the device samples nu2 every sweep, the host callable holds it at 0.01 (it
+has no nu2 step).  Prints the card name and power limit beside the numbers.
+usage: python tools/constrained_bench.py [--likelihood {poisson,binomial,gaussian}] [--rounds 2] [--steps 20]
+       [--host-steps 20]"""
 import argparse
 import json
 import os
@@ -41,6 +43,11 @@ def problem(N, M, T, K, seed, likelihood='poisson'):
         cons = np.concatenate([np.concatenate([np.eye(T), -np.eye(T)]),
                                np.concatenate([np.zeros(T), -np.ones(T)])[:, None]], axis=1)
         return W, V, (Y, Nt), cons
+    if likelihood == 'gaussian':
+        Y = lam + 0.1 * rs.normal(size=lam.shape)
+        Y[rs.random_sample(Y.shape) < 0.1] = np.nan
+        A = np.eye(T, k=1)[:-1] - np.eye(T)[:-1]      # Mu[t + 1] - Mu[t] >= 0
+        return W, V, Y, np.concatenate([A, np.zeros((T - 1, 1))], axis=1)
     Y = rs.poisson(lam).astype(float)
     Y[rs.random_sample(Y.shape) < 0.1] = np.nan
     cons = np.concatenate([np.eye(T), np.zeros((T, 1))], axis=1)
@@ -49,7 +56,8 @@ def problem(N, M, T, K, seed, likelihood='poisson'):
 
 def model(ll, N, M, T, K, W, V, cons, ngrid):
     from functionalmf_b200 import ConstrainedNonconjugateBayesianTensorFiltering as CM
-    return CM(N, M, T, ll, cons, nembeds=K, tf_order=2, gass_ngrid=ngrid, W_init=W, V_init=V, seed=7)
+    kw = dict(nu2_init=0.01) if ll == 'gaussian' else {}
+    return CM(N, M, T, ll, cons, nembeds=K, tf_order=2, gass_ngrid=ngrid, W_init=W, V_init=V, seed=7, **kw)
 
 
 def timed(m, Y, steps):
@@ -63,7 +71,7 @@ def timed(m, Y, steps):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument('--likelihood', choices=('poisson', 'binomial'), default='poisson')
+    ap.add_argument('--likelihood', choices=('poisson', 'binomial', 'gaussian'), default='poisson')
     ap.add_argument('--rounds', type=int, default=2)
     ap.add_argument('--steps', type=int, default=20)
     ap.add_argument('--host-steps', type=int, default=20)
@@ -72,6 +80,9 @@ def main():
     lik = args.likelihood
     if lik == 'binomial':
         from test_gpu_constrained_binomial import binomial_rowcol_loglikelihood as host_ll
+    elif lik == 'gaussian':
+        from test_gpu_constrained_gaussian import GaussianLL
+        host_ll = GaussianLL(0.01)
     else:
         from constrained_ll import rowcol_loglikelihood as host_ll
     out = {'card': card()}
